@@ -55,7 +55,12 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the config 3 (reward throughput) and config 5 (curriculum) objects")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 WORKLOAD = ("configs[3]: full A2C training step (rollout+reward+value+loss+backward+allreduce+Adam), "
@@ -132,11 +137,37 @@ def make_nets(seed, dev):
     return M.AdvantageActorCriticNetwork(V, P).to(dev), R.to(dev)
 
 
+DUMP_ROWS = 8192
+
+
+def dump_outputs(out_dir, per_row, stats, grads):
+    """What a caller of the timed training step receives from its last step, as float32 / float64 .npy files: the
+    sampled token ids, their log-probabilities, the values and rewards (`per_row`: tokens / logp / values / rewards,
+    rows x S), the loss, mean reward and mean advantage (`stats`), and every parameter's gradient (`grads`, written as
+    grad.<name>).  The weights after the Adam update are left out: Adam's first step moves an entry by
+    ~lr * g / (|g| + eps), so last-bit differences of a near-zero gradient (float atomics) become differences far above
+    rounding in the weight, while the gradient itself shows them as what they are.  Batches above DUMP_ROWS rows keep a
+    fixed, seeded sample of rows, listed in rows.npy, so that the files stay below 64 MB.  With several GPUs these are
+    rank 0's rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    B = int(per_row["tokens"].shape[0])
+    rows = np.arange(B)
+    if B > DUMP_ROWS:
+        rows = np.sort(np.random.RandomState(0).choice(B, DUMP_ROWS, replace=False))
+        np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+    out = {k: np.asarray(per_row[k], dtype=np.float32)[rows] for k in ("tokens", "logp", "values", "rewards")}
+    out.update(loss=np.float64(stats[0]), mean_reward=np.float64(stats[1]), mean_advantage=np.float64(stats[2]))
+    for name, g in grads.items():
+        out["grad." + name] = np.asarray(g, dtype=np.float32)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def cpu_reference(rows_per_step, warm_rows=64):
     """The reference algorithm as executed (oracle/ref_port: per-step prefix re-runs, batch-as-time RNN calls, numpy
     sampling, autograd backward, Adam) on all host cores.  `rows_per_step` lists the rows of each timed step (leading
     rows of the bench workload); one un-timed step of `warm_rows` rows comes first (thread pool, allocator, Adam state).
-    Returns (captions/s over the timed steps, cores, [seconds per step])."""
+    Returns (captions/s over the timed steps, cores, [seconds per step], the last step's result)."""
     from oracle import ref_port        # the one place bench.py executes oracle/: the CPU reference being timed
     from icrl_b200 import synth
     cores = os.cpu_count() or 1
@@ -147,24 +178,27 @@ def cpu_reference(rows_per_step, warm_rows=64):
     times = []
     for i, rows in enumerate([warm_rows] + list(rows_per_step)):
         t0 = time.perf_counter()
-        ref_port.a2c_minibatch(nets, f[:rows], c[:rows], np.ascontiguousarray(u[:, :rows]))
+        res = ref_port.a2c_minibatch(nets, f[:rows], c[:rows], np.ascontiguousarray(u[:, :rows]))
         opt.step()
         if i > 0:
             times.append(time.perf_counter() - t0)
-    return sum(rows_per_step) / sum(times), torch.get_num_threads(), times
+    return sum(rows_per_step) / sum(times), torch.get_num_threads(), times, res
 
 
 def main_reference(args, rank):
     """Reference arm: rank 0 alone times the reference's CPU implementation of the path on the box's host cores.  The
     first timed step is the FULL workload (every row of the global batch: one carried-state chain over all of them, as
-    the reference runs it); the remaining steps are bounded samples (--cpu-sample leading rows; the cost is linear in
-    rows) so that the run ends within minutes; value = rows processed / time over all timed steps."""
+    the reference runs it); the remaining --steps - 1 steps are bounded samples (--cpu-sample leading rows; the cost is
+    linear in rows) so that the run ends within minutes; value = rows processed / time over all timed steps."""
     if rank != 0:
         return
     sample = min(args.cpu_sample, args.batch)
-    n_sample = max(0, min(args.steps, 20) - 1)
+    n_sample = args.steps - 1
     rows = [args.batch] + [sample] * n_sample
-    cps, cores, times = cpu_reference(rows)
+    cps, cores, times, res = cpu_reference(rows)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res, (res["loss"], res["mean_reward"], res["mean_adv"]),
+                     {k: g.numpy() for k, g in res["grads"].items()})
     desc = ("step 1: all %d captions of the workload (%.1f s); %d further steps of the first %d captions each (%.2f s "
             "mean); 1 un-timed warm-up step of 64 captions; value = captions processed / time over the timed steps" % (
                 args.batch, times[0], n_sample, sample, (sum(times[1:]) / n_sample) if n_sample else 0.0))
@@ -275,18 +309,32 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MIN)
         return int(t.item()) == 1
 
-    def timed(run_step, steps, warmup):
+    def timed(run_step, steps, warmup, reset=None):
+        """Mean ms per step over `steps` steps after `warmup` un-timed ones.  `reset`, if given, runs before every step
+        and outside the timed intervals (each step is then timed by its own pair of events)."""
         for _ in range(warmup):
+            if reset:
+                reset()
             run_step()
         barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         l0 = eng.launches.value
-        e0.record()
-        for _ in range(steps):
-            run_step()
-        e1.record()
-        barrier()
-        ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
+        if reset is None:
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(steps):
+                run_step()
+            e1.record()
+            barrier()
+            ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
+        else:
+            ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
+            for e0, e1 in ev:
+                reset()
+                e0.record()
+                run_step()
+                e1.record()
+            barrier()
+            ms = torch.tensor([sum(e0.elapsed_time(e1) for e0, e1 in ev)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item()) / steps, (eng.launches.value - l0) // steps
@@ -299,27 +347,6 @@ def main():
         c1 = seg_counters()
         return {k: c1[k] - c0[k] for k in c0}
 
-    # ---- warm-up: W (>= 3) steps, then up to 16 more checked steps while the engine is still re-sizing its chain warm-ups
-    # (every step verified; the warm-up of each chain follows the measured contraction rate, engine._adapt_warm)
-    prep = eng.prepare(fl, cl, ul, plan=plan)
-    clocks = ClockSampler(local)
-    clocks.start()
-    n_warm = 0
-    for _ in range(max(args.warmup, 3)):
-        dp.step(prep, global_rows=B)
-        n_warm += 1
-    for _ in range(16):
-        settled = len(eng.segment_stats["warm_history"]) == 0 or \
-            eng.segment_stats["warm_history"][-1][0] + 3 < eng.segment_stats["steps"]
-        if all_min(settled):
-            break
-        dp.step(prep, global_rows=B)
-        n_warm += 1
-    barrier()
-
-    # Both timed legs start from the SAME training state (weights, Adam moments, chain warm-ups): the optimizer keeps
-    # training across the timed steps, and with these synthetic targets the value LSTM forgets more slowly step by step
-    # (its warm-up grows), so a leg that ran 20 steps later would time a different workload.
     def snapshot():
         st = {"warm": dict(eng.warm), "clean": dict(eng._clean), "hold": dict(eng._hold)}
         if args.torch_adam:
@@ -330,8 +357,9 @@ def main():
             st["flat"] = (opt.flat_param.clone(), opt.exp_avg.clone(), opt.exp_avg_sq.clone(), opt.t)
         return st
 
-    def restore(st):
-        eng.warm, eng._clean, eng._hold = dict(st["warm"]), dict(st["clean"]), dict(st["hold"])
+    def restore(st, chains=True):
+        if chains:
+            eng.warm, eng._clean, eng._hold = dict(st["warm"]), dict(st["clean"]), dict(st["hold"])
         if args.torch_adam:
             with torch.no_grad():
                 for p, q in zip(A.parameters(), st["params"]):
@@ -343,14 +371,49 @@ def main():
             opt.exp_avg_sq.copy_(st["flat"][2])
             opt.t = st["flat"][3]
 
-    state0 = snapshot()
+    # Every warm-up and timed step of the two legs starts from the seeded weights and a fresh optimizer state; only the
+    # engine's chain warm-ups carry over from step to step.  A step that continued training would start from weights
+    # that depend on the rounding of every earlier step's gradients (float atomics), which Adam turns into steps of ~lr
+    # on near-zero entries: with the same arguments, the timed steps then compute the same thing from the same inputs
+    # on every run.
+    init = snapshot()
+
+    def reset():
+        restore(init, chains=False)
+
+    # ---- warm-up: W (>= 3) steps, then up to 16 more checked steps while the engine is still re-sizing its chain warm-ups
+    # (every step verified; the warm-up of each chain follows the measured contraction rate, engine._adapt_warm)
+    prep = eng.prepare(fl, cl, ul, plan=plan)
+    clocks = ClockSampler(local)
+    clocks.start()
+    n_warm = 0
+    for _ in range(max(args.warmup, 3)):
+        reset()
+        dp.step(prep, global_rows=B)
+        n_warm += 1
+    for _ in range(16):
+        settled = len(eng.segment_stats["warm_history"]) == 0 or \
+            eng.segment_stats["warm_history"][-1][0] + 3 < eng.segment_stats["steps"]
+        if all_min(settled):
+            break
+        reset()
+        dp.step(prep, global_rows=B)
+        n_warm += 1
+    barrier()
+    reset()
+    state0 = snapshot()           # the seeded weights with the chain warm-ups the warm-up settled on
 
     # ---- leg 1: minibatch resident in HBM.  The steps run unchecked (no host read inside the timed region) and are
     # verified together afterwards (the joint-check words are running maxima); a failure re-times with a check per step.
+    last = {}
+
+    def step_hbm(check):
+        last["res"] = dp.step(prep, global_rows=B, check=check)
+
     c0 = seg_counters()
     eng.phase_events = []
     t_wall0 = time.time()
-    ms_step, launches = timed(lambda: dp.step(prep, global_rows=B, check=False), args.steps, 0)
+    ms_step, launches = timed(lambda: step_hbm(False), args.steps, 0, reset)
     clk = clocks.stop(t_wall0, time.time())
     phases = {k: sum(v) / len(v) for k, v in eng.phase_times_ms().items()}
     eng.phase_events = None
@@ -362,12 +425,16 @@ def main():
         # Time again with every step checked (re-runs with longer warm-ups included); every rank takes this branch.
         value_checked_per_step = True
         eng.phase_events = []
-        ms_step, launches = timed(lambda: dp.step(prep, global_rows=B), args.steps, 2)
+        ms_step, launches = timed(lambda: step_hbm(True), args.steps, 2, reset)
         phases = {k: sum(v) / len(v) for k, v in eng.phase_times_ms().items()}
         eng.phase_events = None
         lay = eng.piece_layout if args.chain_engine == "tc" else None
         seg_layout = eng.segment_layout
     value_seg = seg_delta(c0)
+    if args.dump_outputs and rank == 0:
+        res = last["res"]                                  # before the later legs overwrite the gradients
+        dump_outputs(args.dump_outputs, {k: res[k].float().cpu().numpy() for k in ("tokens", "logp", "values", "rewards")},
+                     res["stats"].double().cpu().numpy(), {k: p.grad.float().cpu().numpy() for k, p in A.named_parameters()})
 
     # ---- leg 2: end to end through the public API from pinned host buffers, every step checked, loss read on the host
     e2e = None
@@ -382,7 +449,7 @@ def main():
 
         restore(state0)
         c0 = seg_counters()
-        ms_e2e, _ = timed(step_e2e, args.steps, 1)      # one un-timed step: first touch of the pinned buffers
+        ms_e2e, _ = timed(step_e2e, args.steps, 1, reset)   # one un-timed step: first touch of the pinned buffers
         e2e = {"value": B / (ms_e2e * 1e-3), "unit": "captions/s", "ms_per_step": ms_e2e,
                "h2d_bytes_per_step": int(fl.nbytes + (hi - lo) * 4 + ul.nbytes), "d2h_bytes_per_step": 80,
                "chain_checks": seg_delta(c0)}
@@ -514,7 +581,10 @@ def main():
                    "global_batch": B, "local_batch": Bl, "parallelism": "dp%d" % world, "vocab": 1004,
                    "optimizer": "torch.optim.Adam" if args.torch_adam else "FlatAdam (one kernel over the flat bucket)",
                    "chain_shards_per_rank": args.chain_shards, "chain_segments": chain_cfg,
-                   "l2_flush": "not needed: per-step working set (chain stash, GBs) >> 126 MB L2"},
+                   "l2_flush": "not needed: per-step working set (chain stash, GBs) >> 126 MB L2",
+                   "timed_steps_start": "every warm-up and timed step starts from the seeded weights and a fresh "
+                                        "optimizer state (the first training step, replayed); only the chain warm-ups "
+                                        "adapt from step to step"},
         "clocks": clk, "gpu_launches": int(launches), "phases_ms": phases, "roofline": roofline,
         "roofline_decode": decode,
     }
@@ -530,7 +600,7 @@ def main():
         out["curriculum"] = curriculum
     if world == 1 and not args.no_cpu_baseline:
         Bs = min(args.cpu_sample, B)
-        cps, cores, times = cpu_reference([Bs])
+        cps, cores, times, _ = cpu_reference([Bs])
         out["cpu_baseline"] = {"value": cps, "unit": "captions/s", "cores": cores, "kind": "port",
                                "sample": "1 timed step of the first %d of the %d captions (%.1f s) after an un-timed 64-caption "
                                          "step; the reference's cost is linear in rows (serial RNN chains); the reference arm "

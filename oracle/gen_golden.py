@@ -2,7 +2,7 @@
 
 TEST INFRASTRUCTURE (see oracle/__init__).  Usage:  python -m oracle.gen_golden [--only NAME]
 
-The reference modules are imported from /root/reference (never copied); the three
+The reference modules are imported from oracle.reference_dir() (oracle/_ref/ or the checkout); the three
 packages it imports but this image lacks (h5py, gensim, pycocoevalcap) are stubbed in
 sys.modules -- none of them is touched on the A2C path.  Inputs and weights come from
 oracle.synth (seeded, portable), so only OUTPUTS are stored.  Gradients are stored as
@@ -25,11 +25,15 @@ import types
 import numpy as np
 import torch
 
-from . import synth
+from . import reference_dir, synth
 
-REF = "/root/reference"
+REF = reference_dir() or ""
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 GRAD_SAMPLES = 512
+LOGIT_ROWS = 64
+# torch's CPU kernels split some reductions by the intra-op thread count, so the fixtures are reproducible bit for bit
+# only with the count they were generated with
+THREADS = 8
 
 
 def import_reference():
@@ -163,6 +167,9 @@ def case_a2c(name, seed, B, L, level=None, wordvec_dim=512, bidirectional=False)
     f, c = synth.make_inputs(seed, B, L)
     out = run_reference_a2c(w, f, c, seed, level, pretrained=wordvec_dim != 512, bidirectional=bidirectional)
     out.update(seed=seed, B=B, L=L, level=-1 if level is None else level, wordvec_dim=wordvec_dim)
+    if B > LOGIT_ROWS:          # a fixed, seeded sample of rows of the last step's logits keeps the fixture below 1 MB
+        rows = np.sort(np.random.RandomState(0).choice(B, LOGIT_ROWS, replace=False))
+        out.update(last_logits=out["last_logits"][rows], last_logits_rows=rows)
     np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
     print(name, "loss", out["loss"], "tokens", out["tokens"].shape)
 
@@ -296,10 +303,10 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--only", default=None)
     args = ap.parse_args()
-    if not os.path.isdir(REF):
-        raise SystemExit("gen_golden needs /root/reference (build container only)")
+    if not REF or not os.path.isdir(REF):
+        raise SystemExit("gen_golden needs the reference sources in oracle/_ref/ or ICRL_REFERENCE_DIR (default /root/reference)")
     os.makedirs(OUT, exist_ok=True)
-    torch.set_num_threads(os.cpu_count() or 1)
+    torch.set_num_threads(THREADS)
     for name, fn in CASES.items():
         if args.only in (None, name):
             fn()

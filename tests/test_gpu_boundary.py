@@ -10,12 +10,11 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import synth
+from oracle import reference_dir, synth
 from tests.helpers import check_grads_vs_golden, load_case, make_nets, named_grads
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 TOL, GTOL = 2e-6, 2e-5
 
 
@@ -76,13 +75,6 @@ def test_train_a2c_network_loads_checkpoints_and_trains(tmp_path):
     assert "AdvantageActorCriticNetwork" in open(save_paths["results_path"]).read()
 
 
-def _reference_dir():
-    for d in ("/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if os.path.exists(os.path.join(d, "trainers.py")) and os.path.exists(os.path.join(d, "utilities.py")):
-            return d
-    return None
-
-
 def _import_reference_trainers(ref_dir):
     """The reference's own trainers.py / utilities.py / metrics.py, unmodified, with `models` resolved to the drop-in
     module (INTEGRATION.md section 1) and the three absent third-party packages stubbed (SURVEY.md 8c)."""
@@ -129,11 +121,11 @@ def test_unmodified_reference_loop_runs_on_dropin_models(name, tmp_path):
     """`sys.modules["models"] = icrl_b200.models`, then the reference's OWN a2c_training / a2c_curriculum_training
     (imported from its source file, not restated) trains the drop-in networks: sampled tokens, the three logged scalars
     and all 18 gradients equal the golden fixtures the unmodified reference produced on its own models.
-    Needs the reference sources (/root/reference in the build container, or the git-ignored install baseline/_ref that
-    __graft_entry__.build() makes when the reference is present); skipped where neither exists."""
-    ref_dir = _reference_dir()
+    Needs the reference sources: the copy __graft_entry__.build() installs in oracle/_ref/, or the checkout itself
+    (ICRL_REFERENCE_DIR, by default /root/reference); skipped where neither exists."""
+    ref_dir = reference_dir()
     if ref_dir is None:
-        pytest.skip("reference sources not available on this machine")
+        pytest.skip("reference sources not found in oracle/_ref/ or ICRL_REFERENCE_DIR (default /root/reference)")
     g, seed, f, c, u, level = load_case(name)
     A, R, w = make_nets(seed)
     T, U, restore = _import_reference_trainers(ref_dir)

@@ -9,9 +9,19 @@ import pytest
 import torch
 
 from oracle import ref_port, single_pass, synth
-from oracle.gen_golden import grad_sample_index
+from oracle.gen_golden import THREADS, grad_sample_index
 
 A2C_CASES = ["a2c_b8_l6", "a2c_b32_l9", "curr_b16_l10_lv4", "curr_b24_l20_lv6"]
+
+
+@pytest.fixture(autouse=True)
+def _golden_thread_count():
+    """ref_port matches the fixtures bit for bit only with the intra-op thread count they were generated with, whatever
+    the host's core count."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 def _load(golden_dir, name):
