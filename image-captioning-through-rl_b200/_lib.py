@@ -58,7 +58,7 @@ SIGNATURES = {
     "icrl_pack_chain_tc_weights": [P, I, P, P, LP],
     "icrl_chain_tc_fwd": [P, I, I, L, I] + [P] * 10 + [LP],
     "icrl_chains_tc_fwd_fused": [P, I, L, I] + [P] * 9 + [I, L, I] + [P] * 8 + [LP],
-    "icrl_chain_tc_lstm_bwd": [P, I, L, I, P, P, P, P, P, L, P, P, P, P, LP],
+    "icrl_chain_tc_lstm_bwd": [P, I, L, I, P, P, P, P, P, L, P, L, P, P, P, P, LP],
     "icrl_chain_tc_set_profile": [P],
     "icrl_chain_tc_set_bias": [F, F],
     "icrl_chain_tc_bwd_max_pieces": [],
@@ -78,6 +78,7 @@ SIGNATURES = {
     "icrl_value_head_fwd": [P, I, I, P, P, P, P, P, LP],
     "icrl_value_head_bwd": [P, I, I] + [P] * 14 + [LP],
     "icrl_value_chain_param_grads": [P, I, I, I] + [P] * 8 + [Z] + [P] * 5 + [I, I, I, I, LP],
+    "icrl_value_chain_param_grads_pairs": [P, I, I, I, P, P, L] + [P] * 7 + [Z] + [P] * 5 + [I, I, I, I, LP],
     "icrl_wgrad_tc_pack_b": [P, I, I, L, P, I, P, Z, I, LP],
     "icrl_reward_cosine_fwd": [P, I, I, P, P, P, LP],
     "icrl_a2c_loss_fwd_bwd": [P, I, I, P, P, P, F, P, P, P, P, LP],

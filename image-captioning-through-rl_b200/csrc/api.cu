@@ -487,9 +487,10 @@ int icrl_chains_tc_fwd_fused(void* stream, int v_pieces, long long v_seg, int v_
 
 int icrl_chain_tc_lstm_bwd(void* stream, int pieces, long long seg, int warm, const void* packed,
                            const float* stash_gates, const float* stash_c, const int* take, const float* dh_take,
-                           long long take_rows, float* dgates, void* ws, float* cp_state, float* err, int* launches) {
+                           long long take_rows, void* dg_pairs, long long pair_rows, float* dg_inv_scale, void* ws,
+                           float* cp_state, float* err, int* launches) {
   TRY(icrl_chain_tc_lstm_bwd_impl(S_(stream), pieces, seg, warm, packed, stash_gates, stash_c, take, dh_take, take_rows,
-                                  dgates, ws, cp_state, err));
+                                  dg_pairs, pair_rows, dg_inv_scale, ws, cp_state, err));
   bump(launches, 3);                       // |dh_take| maximum, the persistent cluster kernel, the joint check
   return ICRL_OK;
 }
@@ -616,6 +617,19 @@ int icrl_value_head_bwd(void* stream, int B, int S, const float* features, const
   return ICRL_OK;
 }
 
+// dW_ih = dtable^T E, dE = dtable W_ih (when dE is set), db_ih = db_hh = column sums of dtable
+static int gate_table_grads(cudaStream_t st, int V, int D, const float* dtable, const float* E, const float* W_ih,
+                            float* colsum_ws, float* gemm_ws, size_t gemm_ws_bytes, float* dE, float* dW_ih, float* db_ih,
+                            float* db_hh, int* launches) {
+  TRY(icrl_gemm_f32_impl(st, 1, 0, 4 * H, D, V, dtable, 4 * H, E, D, dW_ih, D, nullptr, 0.f, gemm_ws, gemm_ws_bytes, launches));
+  if (dE)
+    TRY(icrl_gemm_f32_impl(st, 0, 0, V, D, 4 * H, dtable, 4 * H, W_ih, D, dE, D, nullptr, 0.f, gemm_ws, gemm_ws_bytes, launches));
+  TRY(icrl_wcolsum(st, V, 4 * H, dtable, nullptr, 0, colsum_ws, db_ih));
+  bump(launches, 2);
+  ICRL_CUDA(cudaMemcpyAsync(db_hh, db_ih, 4 * H * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  return ICRL_OK;
+}
+
 int icrl_value_chain_param_grads(void* stream, int T, int V, int D, const int* tok_stream, const float* dgates,
                                  const float* stash_h, const float* E, const float* W_ih, float* dtable,
                                  float* colsum_ws, float* gemm_ws, size_t gemm_ws_bytes, float* dE, float* dW_ih,
@@ -629,7 +643,7 @@ int icrl_value_chain_param_grads(void* stream, int T, int V, int D, const int* t
   ICRL_CUDA(cudaMemsetAsync(dtable, 0, (size_t)V * 4 * H * sizeof(float), st));
   if (B > 0) {
     ICRL_REQUIRE(T == icrl_stream_len(B, p0, S, 0), "T is not the length of the (B, p0, S) stream");
-    colmax = reinterpret_cast<unsigned*>(colsum_ws);             // consumed by the transposes below, before colsum_ws is reused
+    colmax = reinterpret_cast<unsigned*>(colsum_ws);             // consumed by the split below, before colsum_ws is reused
     TRY(icrl_scatter_add_stream(st, B, p0, S, 0, 4 * H, dgates, tok_stream, dtable, colmax));
   } else {
     TRY(icrl_scatter_add_rows(st, T, 4 * H, dgates, tok_stream, dtable));
@@ -645,13 +659,23 @@ int icrl_value_chain_param_grads(void* stream, int T, int V, int D, const int* t
     TRY(icrl_gemm_f32_impl(st, 1, 0, 4 * H, H, T, dgates, 4 * H, stash_h, H, dW_hh, H, nullptr, 0.f, gemm_ws,
                            gemm_ws_bytes, launches));
   }
-  TRY(icrl_gemm_f32_impl(st, 1, 0, 4 * H, D, V, dtable, 4 * H, E, D, dW_ih, D, nullptr, 0.f, gemm_ws, gemm_ws_bytes, launches));
-  if (dE)
-    TRY(icrl_gemm_f32_impl(st, 0, 0, V, D, 4 * H, dtable, 4 * H, W_ih, D, dE, D, nullptr, 0.f, gemm_ws, gemm_ws_bytes, launches));
-  TRY(icrl_wcolsum(st, V, 4 * H, dtable, nullptr, 0, colsum_ws, db_ih));
-  bump(launches, 2);
-  ICRL_CUDA(cudaMemcpyAsync(db_hh, db_ih, 4 * H * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  return ICRL_OK;
+  return gate_table_grads(st, V, D, dtable, E, W_ih, colsum_ws, gemm_ws, gemm_ws_bytes, dE, dW_ih, db_ih, db_hh, launches);
+}
+
+int icrl_value_chain_param_grads_pairs(void* stream, int T, int V, int D, const int* tok_stream, const void* dg_pairs,
+                                       long long pair_rows, const float* dg_inv_scale, const float* stash_h, const float* E,
+                                       const float* W_ih, float* dtable, float* colsum_ws, float* gemm_ws,
+                                       size_t gemm_ws_bytes, float* dE, float* dW_ih, float* dW_hh, float* db_ih,
+                                       float* db_hh, int B, int p0, int S, int h_packed, int* launches) {
+  cudaStream_t st = S_(stream);
+  ICRL_REQUIRE(B > 0 && T == icrl_stream_len(B, p0, S, 0), "T is not the length of the (B, p0, S) stream");
+  ICRL_REQUIRE(gemm_ws_bytes >= icrl_wgrad_tc_ws_bytes_impl(4 * H, H, T, 2), "gate-gradient pairs need the wgrad_tc workspace");
+  ICRL_CUDA(cudaMemsetAsync(dtable, 0, (size_t)V * 4 * H * sizeof(float), st));
+  TRY(icrl_scatter_add_stream_pairs(st, B, p0, S, 0, dg_pairs, pair_rows, dg_inv_scale, tok_stream, dtable));
+  TRY(icrl_wgrad_tc_gate_pairs_impl(st, H, T, dg_pairs, pair_rows, dg_inv_scale, stash_h, H, dW_hh, H, gemm_ws, gemm_ws_bytes,
+                                    2, h_packed));
+  bump(launches, 3 - (h_packed ? 1 : 0));
+  return gate_table_grads(st, V, D, dtable, E, W_ih, colsum_ws, gemm_ws, gemm_ws_bytes, dE, dW_ih, db_ih, db_hh, launches);
 }
 
 int icrl_reward_cosine_fwd(void* stream, int B, int S, const float* ve, const float* se, float* rewards,

@@ -29,8 +29,8 @@
 // through L2 and TMA-multicast to the 4 CTAs of a K half; B = W_hh^T slice; partial sums swapped through DSMEM); each
 // CTA owns the cell arithmetic of 64 hidden units.  Gate gradients span many orders of magnitude, so the exchanged copy is
 // scaled by a power of two derived from max |dL/dh_take| (fp16 keeps 22 bits down to 2^-18 of that maximum; overflow
-// is detected and reported).  The fp32 gate gradients of live positions go to `dgates` for the parameter-gradient
-// contractions exactly as the serial kernel writes them.
+// is detected and reported).  The gate gradients of live positions go to the parameter-gradient contractions as that
+// same scaled split, in planes [2][rows][2048] with the columns of icrl_gate_pair_col (the policy's BPTT writes fp32).
 #include "tc_ptx.cuh"
 #include "internal.h"
 
@@ -483,7 +483,10 @@ struct BwdArgs {
   const float* stash_c;    // [rows + stride_t][512]: c after the cell of row r lives at row r + stride_t
   const int* take;         // [rows] row of dh_take injected at the position, or -1
   const float* dh_take;    // [take_rows][512]
-  float* dgates;           // [P*seg + warm][2048] pre-activation gate gradients of the live positions
+  float* dgates;           // [rows][2048] fp32 pre-activation gate gradients of the live positions (policy BPTT), or null
+  __half* dg_pair;         // or [2][pair_rows][2048]: their scaled fp16 split, columns in icrl_gate_pair_col order
+  long long pair_rows;
+  float* dg_inv_scale;     // device word: 1 / scale of dg_pair (written when dg_pair is set)
   __half* dgx;             // [2 buffers][2 parts][Ppad][2048] scaled fp16 split of the gate gradients (exchange)
   const float* dh_max;     // device word: max |dh_take| (scale of the recurrence)
   float* bstate;           // [2 checkpoints][2 sides][P][2][512] (dh, dc) at the joints (null: no checkpoints)
@@ -502,6 +505,11 @@ __device__ __forceinline__ float bwd_scale(float m) {
   ex = 4 - ex;
   ex = ex > 100 ? 100 : (ex < -100 ? -100 : ex);
   return ldexpf(1.f, ex);
+}
+
+__device__ __forceinline__ void st_global_v8(__half* dst, const uint2* v) {      // 32 bytes, 32-byte aligned
+  asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst), "r"(v[0].x), "r"(v[0].y), "r"(v[1].x),
+               "r"(v[1].y), "r"(v[2].x), "r"(v[2].y), "r"(v[3].x), "r"(v[3].y) : "memory");
 }
 
 __device__ __forceinline__ unsigned mapa_u32(unsigned addr, unsigned rank) {
@@ -631,6 +639,7 @@ chain_tc_bwd_kernel(const __grid_constant__ CUtensorMap map_dg, const __grid_con
     unsigned char* gst = smem + ew * B_GST_WARP;
     const long long sk = p.stride_k, stt = p.stride_t;
     const float S = bwd_scale(*p.dh_max), invS = 1.f / S;
+    if (p.dg_pair && blockIdx.x == 0 && ew == 0 && lane == 0) *p.dg_inv_scale = invS;
     const float mg = p.main_gain;
     float dc[4][8];                            // carried dL/dc of this thread's piece: [8-unit group][unit]
 #pragma unroll
@@ -822,7 +831,7 @@ chain_tc_bwd_kernel(const __grid_constant__ CUtensorMap map_dg, const __grid_con
       __syncwarp();
       const long long u2 = prof ? clock64() : 0;
       // (S) one pass over the staged gate gradients, 8 lanes per row: the scaled fp16 split (the next step's A operand of
-      //     every CTA of the cluster), the fp32 values of the live positions (parameter-gradient contractions), the joint
+      //     every CTA of the cluster), the live positions' gate gradients (parameter-gradient contractions), the joint
       //     checkpoints
       {
         const int c4 = lane & 7;
@@ -836,14 +845,22 @@ chain_tc_bwd_kernel(const __grid_constant__ CUtensorMap map_dg, const __grid_con
             const bool live = kr == P - 1 || it >= p.warm;
             const int uc = ucolw + c4 * 4;
             __half* xp = p.dgx + ((size_t)((((it + 1) & 1) * 2) * Ppad + kr)) * (4 * H) + uc;
+            uint2 hi[4], lo[4];
 #pragma unroll
             for (int a = 0; a < 4; ++a) {
               const float4 d = *reinterpret_cast<const float4*>(e + a * 4096);
-              uint2 hi, lo;
-              split4_f16(make_float4(d.x * S, d.y * S, d.z * S, d.w * S), hi, lo);
-              *reinterpret_cast<uint2*>(xp + a * H) = hi;
-              *reinterpret_cast<uint2*>(xp + (size_t)Ppad * (4 * H) + a * H) = lo;
-              if (live) *reinterpret_cast<float4*>(p.dgates + pos * (4 * H) + a * H + uc) = d;
+              split4_f16(make_float4(d.x * S, d.y * S, d.z * S, d.w * S), hi[a], lo[a]);
+              *reinterpret_cast<uint2*>(xp + a * H) = hi[a];
+              *reinterpret_cast<uint2*>(xp + (size_t)Ppad * (4 * H) + a * H) = lo[a];
+              if (live && p.dgates) *reinterpret_cast<float4*>(p.dgates + pos * (4 * H) + a * H + uc) = d;
+            }
+            if (live && p.dg_pair) {
+              // the same split for the parameter-gradient contractions: this lane's 4 units of all 4 gates are 16
+              // adjacent columns (icrl_gate_pair_col), one 32-byte store per plane -- 4 row segments of 128 bytes per
+              // warp and row, as many as the fp32 values would cost
+              __half* pp = p.dg_pair + pos * (4 * H) + icrl_gate_pair_col(uc);
+              st_global_v8(pp, hi);
+              st_global_v8(pp + (size_t)p.pair_rows * (4 * H), lo);
             }
             if (cp_it) {
               const float4 dh4 = *reinterpret_cast<const float4*>(e + 4 * 4096);
@@ -1232,9 +1249,11 @@ int launch_bwd(cudaStream_t st, const __half* dgx, const __half* whhT, int Ppad,
 
 int icrl_chain_tc_lstm_bwd_impl(cudaStream_t st, int P, long long seg, int warm, const void* packed,
                                 const float* stash_g, const float* stash_c, const int* take, const float* dh_take,
-                                long long take_rows, float* dgates, void* ws, float* cp_state, float* err) {
+                                long long take_rows, void* dg_pair, long long pair_rows, float* dg_inv_scale, void* ws,
+                                float* cp_state, float* err) {
   ICRL_REQUIRE(P >= 2 && seg >= 1 && warm >= 1, "chain pieces need P >= 2, seg >= 1, warm >= 1");
-  ICRL_REQUIRE(packed && stash_g && stash_c && take && dh_take && dgates && ws && cp_state && err, "null argument");
+  ICRL_REQUIRE(packed && stash_g && stash_c && take && dh_take && dg_pair && dg_inv_scale && ws && cp_state && err, "null argument");
+  ICRL_REQUIRE(pair_rows >= P * seg + warm && (reinterpret_cast<uintptr_t>(dg_pair) & 31) == 0, "gate-gradient pairs: too few rows or unaligned");
   const int Ppad = pad_pieces(P);
   __half* dgx = reinterpret_cast<__half*>(ws);
   const __half* whhT = reinterpret_cast<const __half*>(packed) + (size_t)2 * 4 * H * H;
@@ -1245,7 +1264,8 @@ int icrl_chain_tc_lstm_bwd_impl(cudaStream_t st, int P, long long seg, int warm,
   BwdArgs a;
   a.P = P; a.Ppad = Ppad; a.steps = (int)(seg + warm); a.warm = warm; a.cp_half = cp_half_of(warm);
   a.stride_k = seg; a.stride_t = 1; a.dh0_out = nullptr;
-  a.stash_g = stash_g; a.stash_c = stash_c; a.take = take; a.dh_take = dh_take; a.dgates = dgates; a.dgx = dgx;
+  a.stash_g = stash_g; a.stash_c = stash_c; a.take = take; a.dh_take = dh_take; a.dgates = nullptr; a.dgx = dgx;
+  a.dg_pair = reinterpret_cast<__half*>(dg_pair); a.pair_rows = pair_rows; a.dg_inv_scale = dg_inv_scale;
   a.dh_max = err + 4; a.bstate = cp_state; a.overflow = err + 5; a.prof = g_chain_tc_prof ? g_chain_tc_prof + 8 : nullptr;
   int rc;
   if ((rc = launch_bwd(st, dgx, whhT, Ppad, &a))) return rc;
@@ -1291,6 +1311,7 @@ int icrl_policy_bptt_tc_impl(cudaStream_t st, int B, int n_cell, int p0, const v
   a.P = B; a.Ppad = Ppad; a.steps = n_cell; a.warm = 0; a.cp_half = -1;
   a.stride_k = 1; a.stride_t = B; a.dh0_out = dh0;
   a.stash_g = Gs; a.stash_c = Cs; a.take = take; a.dh_take = dHv; a.dgates = DG; a.dgx = dgx;
+  a.dg_pair = nullptr; a.pair_rows = 0; a.dg_inv_scale = nullptr;
   a.dh_max = err + 4; a.bstate = nullptr; a.overflow = err + 5; a.prof = nullptr;
   int rc;
   if ((rc = launch_bwd(st, dgx, whhT, Ppad, &a))) return rc;

@@ -36,6 +36,18 @@ void icrl_set_error(const char* fmt, ...);
 
 static inline int icrl_cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 
+// Column order of the LSTM gate gradients that the chain backward stores as fp16 pairs (chain_tc.cu, pass (S)) and the
+// weight-gradient contraction and gate-table scatter read: within each block of 32 hidden units the 128 columns are
+// ordered [unit quad q][gate a][unit j of the quad] instead of [gate a][unit], so that the lane that owns units
+// 4q .. 4q+3 of all four gates stores one contiguous 32-byte run per plane.  natural = a * 512 + u.
+__host__ __device__ __forceinline__ int icrl_gate_pair_col(int natural) {
+  const int a = natural / ICRL_H, u = natural % ICRL_H;
+  return 128 * (u >> 5) + 16 * ((u >> 2) & 7) + 4 * a + (u & 3);
+}
+__host__ __device__ __forceinline__ int icrl_gate_pair_natural(int col) {
+  return ICRL_H * ((col >> 2) & 3) + 32 * (col >> 7) + 4 * ((col >> 4) & 7) + (col & 3);
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

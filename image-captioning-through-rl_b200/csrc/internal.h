@@ -16,6 +16,8 @@ int icrl_softmax_bwd(cudaStream_t st, int B, int S, int V, float* z, int ldl, co
 int icrl_scatter_add_rows(cudaStream_t st, long long R, int C, const float* src, const int* idx, float* dst);
 int icrl_scatter_add_stream(cudaStream_t st, int B, int p0, int S, int extra, int C, const float* src, const int* tok_stream,
                             float* dst, unsigned* colmax);
+int icrl_scatter_add_stream_pairs(cudaStream_t st, int B, int p0, int S, int extra, const void* pairs, long long pair_rows,
+                                  const float* inv_scale, const int* tok_stream, float* dst);
 int icrl_wcolsum_chunks(long long R);
 int icrl_wcolsum(cudaStream_t st, long long R, int C, const float* X, const float* w, long long row_mod,
                  float* partial, float* out);
@@ -82,6 +84,9 @@ size_t icrl_wgrad_tc_ws_bytes_impl(int M, int N, long long T, int splits);
 int icrl_wgrad_tc_impl(cudaStream_t st, int M, int N, long long T, const float* A, int lda, const float* B, int ldb,
                        float* C, int ldc, void* ws, size_t ws_bytes, int splits, const unsigned* colmax = nullptr,
                        int b_packed = 0);
+int icrl_wgrad_tc_gate_pairs_impl(cudaStream_t st, int N, long long T, const void* pairs, long long pair_rows,
+                                  const float* inv_scale, const float* B, int ldb, float* C, int ldc, void* ws,
+                                  size_t ws_bytes, int splits, int b_packed);
 int icrl_wgrad_tc_pack_b_impl(cudaStream_t st, int M, int N, long long T, const float* B, int ldb, void* ws, size_t ws_bytes,
                               int splits);
 int icrl_adam_flat_impl(cudaStream_t st, long long n, float* p, const float* g, float* m, float* v, float lr, float b1,
@@ -100,7 +105,8 @@ int icrl_chain_tc_fwd_impl(cudaStream_t st, int kind, int P, long long seg, int 
                            float* stash_g, void* ws, float* cp_state, float* err);
 int icrl_chain_tc_lstm_bwd_impl(cudaStream_t st, int P, long long seg, int warm, const void* packed,
                                 const float* stash_g, const float* stash_c, const int* take, const float* dh_take,
-                                long long take_rows, float* dgates, void* ws, float* cp_state, float* err);
+                                long long take_rows, void* dg_pair, long long pair_rows, float* dg_inv_scale, void* ws,
+                                float* cp_state, float* err);
 size_t icrl_policy_bptt_tc_ws_bytes_impl(int B, int n_cell);
 int icrl_policy_bptt_tc_impl(cudaStream_t st, int B, int n_cell, int p0, const void* packed, const float* Gs,
                              const float* Cs, const float* dHv, float* DG, float* dh0, void* ws, float* err);

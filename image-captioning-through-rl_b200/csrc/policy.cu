@@ -2,6 +2,7 @@
 //   LSTM cell update and its backward (models.py:80; gate order i,f,g,o),
 //   softmax -> numpy-semantics inverse-CDF sampling or greedy argmax -> log-prob
 //   (trainers.py:444-458, :69), softmax backward, and the gate-table gradient scatter.
+#include <cuda_fp16.h>
 #include "common.cuh"
 
 namespace {
@@ -158,11 +159,29 @@ __global__ void scatter_add_rows_v4_kernel(long long R, int C4, const float4* __
 // one per stream position: B * n_col * C/4 of them instead of T * C/4 (10 times fewer at 19 rollout steps), which turns
 // the scatter from atomic-throughput-bound into a streaming read of src.  The kernel also returns the column |max| of
 // src (the weight-gradient GEMM's per-column scale: wgrad_tc.cu) from the values it has in registers anyway.
-// blockDim.x = C/4; thread c owns columns 4c .. 4c+3 of every row.
-__global__ void scatter_add_stream_kernel(int B, int p0, int S, int extra, const float4* __restrict__ src,
-                                          const int* __restrict__ tok_stream, float* __restrict__ dst,
-                                          unsigned* __restrict__ colmax) {
-  const int C4 = blockDim.x, c = threadIdx.x;
+// blockDim.x = C/4; thread c owns the 4 adjacent columns src.col(c) .. +3 of every row.
+struct RowsF32 {                              // src [T][C] fp32
+  const float4* src;
+  __device__ float4 load(long long pos, int c) const { return __ldg(src + pos * blockDim.x + c); }
+  __device__ int col(int c) const { return 4 * c; }
+};
+struct GatePairs {                            // the chain backward's [2][rows][2048] fp16 pairs (icrl_gate_pair_col order)
+  const uint2* hi;                            // 4 halves per thread and row
+  long long plane;                            // rows * 512
+  const float* inv_scale;
+  __device__ float4 load(long long pos, int c) const {
+    const uint2 h = __ldg(hi + pos * 512 + c), l = __ldg(hi + plane + pos * 512 + c);
+    const float2 h01 = __half22float2(*reinterpret_cast<const __half2*>(&h.x)), h23 = __half22float2(*reinterpret_cast<const __half2*>(&h.y));
+    const float2 l01 = __half22float2(*reinterpret_cast<const __half2*>(&l.x)), l23 = __half22float2(*reinterpret_cast<const __half2*>(&l.y));
+    const float s = __ldg(inv_scale), li = 1.f / 2048.f;
+    return make_float4(fmaf(l01.x, li, h01.x) * s, fmaf(l01.y, li, h01.y) * s, fmaf(l23.x, li, h23.x) * s, fmaf(l23.y, li, h23.y) * s);
+  }
+  __device__ int col(int c) const { return icrl_gate_pair_natural(4 * c); }
+};
+template <class Src>
+__global__ void scatter_add_stream_kernel(int B, int p0, int S, int extra, const Src src, const int* __restrict__ tok_stream,
+                                          float* __restrict__ dst, unsigned* __restrict__ colmax) {
+  const int C = 4 * blockDim.x, c = threadIdx.x;
   const int n_col = p0 + S - 1 + extra;
   const long long rows = (long long)n_col * B;
   float4 mx = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -178,19 +197,20 @@ __global__ void scatter_add_stream_kernel(int B, int p0, int S, int extra, const
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     int s = s0;
     for (; s + 3 < S; s += 4) {
-      const float4 v0 = __ldg(src + pos(s) * C4 + c), v1 = __ldg(src + pos(s + 1) * C4 + c);
-      const float4 v2 = __ldg(src + pos(s + 2) * C4 + c), v3 = __ldg(src + pos(s + 3) * C4 + c);
+      const float4 v0 = src.load(pos(s), c), v1 = src.load(pos(s + 1), c);
+      const float4 v2 = src.load(pos(s + 2), c), v3 = src.load(pos(s + 3), c);
       take(acc, v0); take(acc, v1); take(acc, v2); take(acc, v3);
     }
-    for (; s < S; ++s) take(acc, __ldg(src + pos(s) * C4 + c));
-    float* d = dst + ((size_t)tok_stream[pos(s0)] * C4 + c) * 4;
+    for (; s < S; ++s) take(acc, src.load(pos(s), c));
+    float* d = dst + (size_t)tok_stream[pos(s0)] * C + src.col(c);
     asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(d), "f"(acc.x), "f"(acc.y), "f"(acc.z), "f"(acc.w) : "memory");
   }
   if (colmax) {                                                        // non-negative floats order like their bit patterns
-    atomicMax(colmax + 4 * c, __float_as_uint(mx.x));
-    atomicMax(colmax + 4 * c + 1, __float_as_uint(mx.y));
-    atomicMax(colmax + 4 * c + 2, __float_as_uint(mx.z));
-    atomicMax(colmax + 4 * c + 3, __float_as_uint(mx.w));
+    const int c0 = src.col(c);
+    atomicMax(colmax + c0, __float_as_uint(mx.x));
+    atomicMax(colmax + c0 + 1, __float_as_uint(mx.y));
+    atomicMax(colmax + c0 + 2, __float_as_uint(mx.z));
+    atomicMax(colmax + c0 + 3, __float_as_uint(mx.w));
   }
 }
 
@@ -281,7 +301,22 @@ int icrl_scatter_add_stream(cudaStream_t st, int B, int p0, int S, int extra, in
   if (colmax) ICRL_CUDA(cudaMemsetAsync(colmax, 0, (size_t)C * sizeof(unsigned), st));
   const long long rows = (long long)(p0 + S - 1 + extra) * B;
   const int blocks = (int)min((long long)148 * 4, rows);
-  scatter_add_stream_kernel<<<blocks, C / 4, 0, st>>>(B, p0, S, extra, reinterpret_cast<const float4*>(src), tok_stream, dst, colmax);
+  scatter_add_stream_kernel<<<blocks, C / 4, 0, st>>>(B, p0, S, extra, RowsF32{reinterpret_cast<const float4*>(src)}, tok_stream,
+                                                      dst, colmax);
+  ICRL_LAUNCH_CHECK();
+  return ICRL_OK;
+}
+
+// The same with src = the chain backward's gate-gradient pairs (planes [2][pair_rows][2048], icrl_gate_pair_col order,
+// values (hi + lo'/2048) * *inv_scale); dst [V][2048] in natural column order.
+int icrl_scatter_add_stream_pairs(cudaStream_t st, int B, int p0, int S, int extra, const void* pairs, long long pair_rows,
+                                  const float* inv_scale, const int* tok_stream, float* dst) {
+  ICRL_REQUIRE(B >= 1 && p0 >= 1 && S >= 1 && extra >= 0, "bad stream shape");
+  ICRL_REQUIRE(((reinterpret_cast<uintptr_t>(pairs) | reinterpret_cast<uintptr_t>(dst)) & 15) == 0, "unaligned rows");
+  const long long rows = (long long)(p0 + S - 1 + extra) * B;
+  const int blocks = (int)min((long long)148 * 4, rows);
+  const GatePairs src{reinterpret_cast<const uint2*>(pairs), pair_rows * 512, inv_scale};
+  scatter_add_stream_kernel<<<blocks, 512, 0, st>>>(B, p0, S, extra, src, tok_stream, dst, nullptr);
   ICRL_LAUNCH_CHECK();
   return ICRL_OK;
 }

@@ -1,18 +1,22 @@
 // Weight-gradient contraction of the value chain on tcgen05 (SURVEY.md K14):
 //   dW_hh[m][n] = sum_t dgates[t][m] * h_prev[t][n],   M = 2048, N = 512, K = T (number of serial steps, up to ~10^6).
-// The operands arrive time-major ([T][M], [T][N] fp32), so two pre-passes put them into the K-major fp16-split form
-// the MMA wants:
-//   1. column |max| of dgates over t  -> a power-of-two scale per gate row m (gradients are ~1e-4 .. 1e-12 and
+// The operands are time-major ([T][M], [T][N]): the MMA reads them MN-major as they lie, as fp16 pairs x*s = hi + lo'/2048
+// (22 mantissa bits) in planes [2][T][C].  The chain backward writes the gate gradients in that form itself
+// (chain_tc.cu, pass (S): one power-of-two scale per launch, columns in the order of icrl_gate_pair_col); fp32 operands
+// go through one elementwise pre-pass first:
+//   1. column |max| of A over t  -> a power-of-two scale per row m of the result (gradients are ~1e-4 .. 1e-12 and
 //      would fall into fp16 subnormals / underflow; h is in (-1, 1) and needs none)
-//   2. transpose + split: x*s = hi + lo'/2048 (fp16 pair, 22 mantissa bits) -> [2][rows][Tp] with Tp = T rounded to 64
-// GEMM: 128x128 tiles, split-K over gridDim.z, 3-stage TMA ring of 64-wide K blocks (hi and lo' of an operand in ONE
-// 3-D box), 2 MMAs per K step (hi * [hi | lo'] -> [main | correction], lo'*hi -> correction accumulator).  Because the tensor core
-// truncates on every accumulate (gemm_tc.cu header), a TMEM accumulator only ever sums 512 K elements: after 8 K blocks
-// the epilogue warps add main + correction/2048 into fp32 REGISTERS (round to nearest) while the MMAs continue in the
-// second accumulator set.  Each split writes its partial tile; a last kernel sums the splits and undoes the row scale.
+//   2. split: [T][C] fp32 -> [2][T][C] fp16 (same layout, no transpose)
+// GEMM: 128x128 tiles, split-K over gridDim.z, 3-stage TMA ring of 64-deep K blocks (SW128 boxes of 64 columns x 64 rows;
+// rows past T are zero-filled by the tensor map), 2 MMAs per K step (hi * [hi | lo'] -> [main | correction], lo'*hi ->
+// correction accumulator).  Because the tensor core truncates on every accumulate (gemm_tc.cu header), a TMEM accumulator
+// only ever sums 512 K elements: after 8 K blocks the epilogue warps add main + correction/2048 into fp32 REGISTERS (round
+// to nearest) while the MMAs continue in the second accumulator set.  Each split writes its partial tile; a last kernel
+// sums the splits, undoes the scale and puts the rows in natural order.
 #include <cuda.h>
 #include <cuda_fp16.h>
 #include "common.cuh"
+#include "tc_ptx.cuh"
 
 namespace {
 
@@ -24,8 +28,9 @@ constexpr int FLUSH_KB = 8;                                // K blocks per TMEM 
 constexpr int TMEM_COLS = 512;                             // 2 sets x (main 128 + correction 128)
 constexpr int THREADS = 192;
 constexpr int CLN = 4;                                      // CTAs of a cluster: the 4 N tiles of one (M tile, split) share A
-constexpr int A_SLICE_ROWS = BM / CLN, A_SLICE = A_SLICE_ROWS * BK * 2;    // 32 rows = 4 KB per part fetched per CTA
-constexpr float LO_SCALE = 2048.f, LO_INV = 1.f / 2048.f;
+constexpr int A_SLICE_ROWS = BK / 2, A_SLICE = 64 * A_SLICE_ROWS * 2;    // 64 columns x 32 K rows = 4 KB per part and CTA
+static_assert(CLN * A_SLICE == OP_TILE / 2, "the 4 CTAs of a cluster fetch one quarter of the A tile each");
+constexpr float LO_INV = 1.f / 2048.f;
 
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
@@ -87,13 +92,17 @@ __device__ __forceinline__ void tc_mma(unsigned tmem_d, unsigned long long da, u
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}\n" ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc),
       "r"(accumulate) : "memory");
 }
-// K-major, 128B swizzle (see gemm_tc.cu)
+// MN-major, 128B swizzle: atoms of 64 MN elements (128 bytes) x 8 K rows; LBO = 8 KB from one 64-column box to the next
+// along MN, SBO = 1 KB from one group of 8 K rows to the next.  A K step of 16 advances the start by 2 KB.
+constexpr unsigned BOX_BYTES = 64 * BK * 2;                // 64 columns x 64 K rows: 8 KB
 __device__ __forceinline__ unsigned long long smem_desc(unsigned addr) {
-  return (unsigned long long)((addr & 0x3FFFF) >> 4) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
+  return (unsigned long long)((addr & 0x3FFFF) >> 4) | ((unsigned long long)(BOX_BYTES >> 4) << 16) | (64ull << 32) |
+         (1ull << 46) | (2ull << 61);
 }
-// F32 accumulate, fp16 x fp16, K-major, N = 128, M = 128
-constexpr unsigned IDESC = (1u << 4) | ((unsigned)(BN >> 3) << 17) | ((unsigned)(BM >> 4) << 24);
-constexpr unsigned IDESC2 = (1u << 4) | ((unsigned)(2 * BN >> 3) << 17) | ((unsigned)(BM >> 4) << 24);     // N = 256
+constexpr unsigned long long DESC_K_STEP = UMMA_K * 128 / 16;
+// F32 accumulate, fp16 x fp16, A and B MN-major (bits 15, 16), N = 128 / 256, M = 128
+constexpr unsigned IDESC = (1u << 4) | (1u << 15) | (1u << 16) | ((unsigned)(BN >> 3) << 17) | ((unsigned)(BM >> 4) << 24);
+constexpr unsigned IDESC2 = (1u << 4) | (1u << 15) | (1u << 16) | ((unsigned)(2 * BN >> 3) << 17) | ((unsigned)(BM >> 4) << 24);
 
 __device__ __forceinline__ void tmem_ld32x2(unsigned ta, unsigned tb, float* a, float* b) {
   unsigned r[64];
@@ -128,96 +137,44 @@ __global__ void col_absmax_kernel(long long T, int C, const float* __restrict__ 
   atomicMax(mx + c, __float_as_uint(m));               // non-negative floats order like their bit patterns
 }
 
-// out_hi/out_lo [C][Tp] fp16 <- X [T][C] fp32 (row stride ldx); scale[c] = 2^-e with max|X[:,c]| in [2^(e-1), 2^e)
-// (null mx: no scaling).  Columns t in [T, Tp) are zero.
-__global__ void transpose_split_kernel(long long T, long long Tp, int C, const float* __restrict__ X, int ldx,
-                                       const unsigned* __restrict__ mx, __half* __restrict__ out_hi,
-                                       __half* __restrict__ out_lo, float* __restrict__ inv_scale) {
-  __shared__ float tile[32][33];
-  const int c0 = blockIdx.x * 32;
-  const long long t0 = (long long)blockIdx.y * 32;
-  const int tx = threadIdx.x, ty = threadIdx.y;          // 32 x 8
-  for (int r = ty; r < 32; r += 8) {
-    const long long t = t0 + r;
-    const int c = c0 + tx;
-    tile[r][tx] = (t < T && c < C) ? X[(size_t)t * ldx + c] : 0.f;
-  }
-  __syncthreads();
-  for (int r = ty; r < 32; r += 8) {
-    const int c = c0 + r;
-    const long long t = t0 + tx;
-    if (c < C && t < Tp) {
-      float s = 1.f;
-      if (mx) {
-        const float m = __uint_as_float(mx[c]);
+// out [2][T][C] fp16 (hi plane, then lo' plane) <- X [T][C] fp32 (row stride ldx), elementwise and in place of the
+// layout: x * s = hi + lo'/2048 with s = 2^-e for max|X[:,c]| in [2^(e-1), 2^e) (null mx: s = 1), inv_scale[c] = 2^e.
+// Four columns per thread (C % 4 == 0); float4 loads when vec (ldx % 4 == 0 and a 16-byte aligned X).
+__global__ void __launch_bounds__(256) split_kernel(long long T, int C, const float* __restrict__ X, int ldx, int vec,
+                                                    const unsigned* __restrict__ mx, __half* __restrict__ out,
+                                                    float* __restrict__ inv_scale) {
+  const int C4 = C / 4;
+  const long long total = T * C4;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long t = i / C4;
+    const int c = 4 * (int)(i - t * C4);
+    const float* x = X + (size_t)t * ldx + c;
+    float4 v = vec ? __ldg(reinterpret_cast<const float4*>(x)) : make_float4(__ldg(x), __ldg(x + 1), __ldg(x + 2), __ldg(x + 3));
+    if (mx) {
+      float s[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float m = __uint_as_float(mx[c + j]);
         int e = 0;
         if (m > 0.f) frexpf(m, &e);
-        s = exp2f((float)-e);
-        if (blockIdx.y == 0 && tx == 0) inv_scale[c] = exp2f((float)e);
+        s[j] = exp2f((float)-e);
+        if (t == 0) inv_scale[c + j] = exp2f((float)e);
       }
-      const float v = tile[tx][r] * s;
-      const __half h = __float2half_rn(v);
-      out_hi[(size_t)c * Tp + t] = h;
-      out_lo[(size_t)c * Tp + t] = __float2half_rn((v - __half2float(h)) * LO_SCALE);
+      v = make_float4(v.x * s[0], v.y * s[1], v.z * s[2], v.w * s[3]);
     }
-  }
-}
-
-// The same pass on 64 x 64 tiles with 16-byte accesses on both sides (float4 rows in, 8 halves along t out): the 32 x 32
-// version above moved 4 + 2 bytes per access and ran at a third of the copy bandwidth (7.5 ms per step at B = 4096, more
-// than the contraction it feeds).  Needs C % 4 == 0, ldx % 4 == 0 and a 16-byte aligned X.
-__global__ void __launch_bounds__(256) transpose_split64_kernel(long long T, long long Tp, int C, const float* __restrict__ X,
-                                                                int ldx, const unsigned* __restrict__ mx,
-                                                                __half* __restrict__ out_hi, __half* __restrict__ out_lo,
-                                                                float* __restrict__ inv_scale) {
-  __shared__ float tile[64][65];
-  const int c0 = blockIdx.y * 64;
-  const long long t0 = (long long)blockIdx.x * 64;
-  const int tid = threadIdx.x;
-  {
-    const int q = tid & 15, r0 = tid >> 4;
-#pragma unroll
-    for (int p = 0; p < 4; ++p) {
-      const int r = r0 + 16 * p;
-      const long long t = t0 + r;
-      const int c = c0 + 4 * q;
-      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (t < T && c < C) v = __ldg(reinterpret_cast<const float4*>(X + (size_t)t * ldx + c));
-      tile[r][4 * q] = v.x; tile[r][4 * q + 1] = v.y; tile[r][4 * q + 2] = v.z; tile[r][4 * q + 3] = v.w;
-    }
-  }
-  __syncthreads();
-  const int tch = tid & 7;
-#pragma unroll
-  for (int pass = 0; pass < 2; ++pass) {
-    const int cc = (tid >> 3) + 32 * pass, c = c0 + cc;
-    if (c < C) {
-      float s = 1.f;
-      if (mx) {
-        const float m = __uint_as_float(mx[c]);
-        int e = 0;
-        if (m > 0.f) frexpf(m, &e);
-        s = exp2f((float)-e);
-        if (blockIdx.x == 0 && tch == 0) inv_scale[c] = exp2f((float)e);
-      }
-      __half hi[8], lo[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const float v = tile[tch * 8 + i][cc] * s;
-        hi[i] = __float2half_rn(v);
-        lo[i] = __float2half_rn((v - __half2float(hi[i])) * LO_SCALE);
-      }
-      const size_t o = (size_t)c * Tp + t0 + tch * 8;
-      *reinterpret_cast<uint4*>(out_hi + o) = *reinterpret_cast<const uint4*>(hi);
-      *reinterpret_cast<uint4*>(out_lo + o) = *reinterpret_cast<const uint4*>(lo);
-    }
+    uint2 hi, lo;
+    icrl_tc::split4_f16(v, hi, lo);
+    *reinterpret_cast<uint2*>(out + (size_t)t * C + c) = hi;
+    *reinterpret_cast<uint2*>(out + (size_t)(T + t) * C + c) = lo;
   }
 }
 
 // ------------------------------------------------------------------------------------------------ GEMM
-// map_a: 3-D {Tp, rows, 2 parts}, box {64, 32, 1}; map_b: box {64, 128, 2}.  partial [gridDim.z][M][N].
-// The 4 CTAs of a cluster (the N tiles of one M tile and split) consume the same A tile: each fetches a quarter of its
-// rows and TMA-multicasts it to all four, so A crosses L2 -> SM once per cluster instead of once per CTA and the four
+// map_a / map_b: 3-D {columns, T, 2 parts}; boxes of 64 columns x 32 (A) / 64 (B) K rows.  partial [gridDim.z][M][N].
+// Stage: A_hi [2 boxes of 64 columns][64 K], A_lo' likewise, then B as [hi, lo'][2 boxes][64 K], so that the four
+// B boxes are the 256 columns [B_hi | B_lo'] of one instruction.
+// The 4 CTAs of a cluster (the N tiles of one M tile and split) consume the same A tile: each fetches a quarter of it
+// (one column box, one half of its K rows) and TMA-multicasts it to all four, so A crosses L2 -> SM once per cluster instead of once per CTA and the four
 // stay in lockstep (a ring stage is refilled only after all four have consumed it).  (Also sharing the B tile between two
 // M tiles -- clusters of 4 x 2 -- was measured and is slower: the 128 CTAs of the value chain's contraction are 16 clusters
 // of 8, of which a B200 holds 15 at a time, so the last cluster runs as a second wave.)
@@ -265,11 +222,13 @@ wgrad_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
         const unsigned full = bar_full + 8 * s;
         mbar_expect_tx(full, STAGE_BYTES);
         const unsigned base = smem_u32(smem + s * STAGE_BYTES);
-        const unsigned a_dst = base + rank * A_SLICE;
-        const int a_row = m0 + (int)rank * A_SLICE_ROWS;
-        tma_load_3d_mcast(a_dst, &map_a, (kb0 + i) * BK, a_row, 0, full, (unsigned short)0xF);
-        tma_load_3d_mcast(a_dst + OP_TILE / 2, &map_a, (kb0 + i) * BK, a_row, 1, full, (unsigned short)0xF);
-        tma_load_3d(base + OP_TILE, &map_b, (kb0 + i) * BK, n0, 0, full);
+        const unsigned a_dst = base + rank * A_SLICE;      // box rank >> 1, K rows [32 (rank & 1), +32)
+        const int a_col = m0 + 64 * (int)(rank >> 1), a_k = (kb0 + i) * BK + A_SLICE_ROWS * (int)(rank & 1);
+        tma_load_3d_mcast(a_dst, &map_a, a_col, a_k, 0, full, (unsigned short)0xF);
+        tma_load_3d_mcast(a_dst + OP_TILE / 2, &map_a, a_col, a_k, 1, full, (unsigned short)0xF);
+#pragma unroll
+        for (int pb = 0; pb < 4; ++pb)                      // [hi, lo'] x [columns n0 .. +63, n0 + 64 .. +127]
+          tma_load_3d(base + OP_TILE + pb * BOX_BYTES, &map_b, n0 + 64 * (pb & 1), (kb0 + i) * BK, pb >> 1, full);
       }
     }
   } else if (warp == 1) {
@@ -285,15 +244,15 @@ wgrad_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
         tc_fence_after();
         const unsigned base = smem_u32(smem + s * STAGE_BYTES);
         const unsigned long long dA0 = smem_desc(base), dA1 = smem_desc(base + OP_TILE / 2);
-        const unsigned long long dB0 = smem_desc(base + OP_TILE);       // 256 rows: hi, then lo' (adjacent in the stage)
+        const unsigned long long dB0 = smem_desc(base + OP_TILE);       // 256 columns: hi, then lo' (adjacent)
         if (elect_one()) {
 #pragma unroll
           for (int k = 0; k < BK / UMMA_K; ++k) {
             const unsigned first = (i == i0 && k == 0) ? 0u : 1u;
             // [main | correction] = A_hi x [B_hi | B_lo'] in ONE N = 256 instruction (A_hi is read from shared memory once
             // instead of twice: operand reads + TMA fill bound this kernel, chain_tc.cu BwdCfg), then correction += A_lo' x B_hi
-            tc_mma(acc_main, dA0 + 2 * k, dB0 + 2 * k, IDESC2, first);
-            tc_mma(acc_corr, dA1 + 2 * k, dB0 + 2 * k, IDESC, 1u);
+            tc_mma(acc_main, dA0 + DESC_K_STEP * k, dB0 + DESC_K_STEP * k, IDESC2, first);
+            tc_mma(acc_corr, dA1 + DESC_K_STEP * k, dB0 + DESC_K_STEP * k, IDESC, 1u);
           }
           tc_commit_mcast(bar_empty + 8 * s, (unsigned short)0xF);
         }
@@ -339,22 +298,24 @@ wgrad_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
   }
 }
 
-// C[m][n] = inv_scale[m] * sum_s partial[s][m][n]
+// C[row(m)][n] = inv_scale[m * scale_stride] * sum_s partial[s][m][n]; row(m) = m, or the natural gate column of stored
+// column m for operands in the chain backward's order (permuted)
 __global__ void wgrad_reduce_kernel(int M, int N, int S, const float* __restrict__ partial, const float* __restrict__ inv_scale,
-                                    float* __restrict__ C, int ldc) {
+                                    int scale_stride, int permuted, float* __restrict__ C, int ldc) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)M * N) return;
   const int m = (int)(i / N), n = (int)(i % N);
   float s = 0.f;
   for (int k = 0; k < S; ++k) s += partial[((size_t)k * M + m) * N + n];
-  C[(size_t)m * ldc + n] = s * inv_scale[m];
+  C[(size_t)(permuted ? icrl_gate_pair_natural(m) : m) * ldc + n] = s * inv_scale[(size_t)m * scale_stride];
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-int make_map(CUtensorMap* map, const void* ptr, long long Tp, int rows, int box_rows, int box_parts) {
+// planes [2][plane_rows][C] fp16, of which rows [0, T) are read; box: 64 columns x box_k rows of one plane
+int make_map(CUtensorMap* map, const void* ptr, int C, long long T, long long plane_rows, int box_k) {
   static EncodeTiledFn fn = nullptr;
   if (!fn) {
     cudaDriverEntryPointQueryResult qres;
@@ -363,47 +324,84 @@ int make_map(CUtensorMap* map, const void* ptr, long long Tp, int rows, int box_
     ICRL_REQUIRE(q && qres == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled unavailable");
     fn = reinterpret_cast<EncodeTiledFn>(q);
   }
-  const cuuint64_t dims[3] = {(cuuint64_t)Tp, (cuuint64_t)rows, 2};
-  const cuuint64_t strides[2] = {(cuuint64_t)Tp * 2, (cuuint64_t)rows * Tp * 2};
-  const cuuint32_t box[3] = {(cuuint32_t)BK, (cuuint32_t)box_rows, (cuuint32_t)box_parts};
+  const cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)T, 2};
+  const cuuint64_t strides[2] = {(cuuint64_t)C * 2, (cuuint64_t)plane_rows * C * 2};
+  const cuuint32_t box[3] = {64, (cuuint32_t)box_k, 1};
   const cuuint32_t estr[3] = {1, 1, 1};
   const CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, estr,
                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    icrl_set_error("cuTensorMapEncodeTiled (wgrad) failed with CUresult %d (Tp %lld, rows %d)", (int)r, Tp, rows);
+    icrl_set_error("cuTensorMapEncodeTiled (wgrad) failed with CUresult %d (C %d, T %lld)", (int)r, C, T);
     return ICRL_ERR_CUDA;
   }
   return ICRL_OK;
 }
 
-inline long long round_up(long long a, long long b) { return (a + b - 1) / b * b; }
+struct Ws {                                  // workspace of icrl_wgrad_tc_ws_bytes_impl(M, N, T, splits)
+  __half* a;                                 // [2][T][M]
+  __half* b;                                 // [2][T][N]
+  float* partial;                            // [splits][M][N]
+  unsigned* mx;                              // [M] column maxima of A
+  float* inv_scale;                          // [M]
+};
+Ws carve(void* ws, int M, int N, long long T, int splits) {
+  Ws w;
+  w.a = reinterpret_cast<__half*>(ws);
+  w.b = w.a + (size_t)2 * M * T;
+  w.partial = reinterpret_cast<float*>(w.b + (size_t)2 * N * T);
+  w.mx = reinterpret_cast<unsigned*>(w.partial + (size_t)splits * M * N);
+  w.inv_scale = reinterpret_cast<float*>(w.mx + M);
+  return w;
+}
+
+int split(cudaStream_t st, long long T, int C, const float* X, int ldx, const unsigned* mx, __half* out, float* inv_scale) {
+  const int vec = ldx % 4 == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0;
+  const int blocks = (int)min((long long)148 * 8, (T * (C / 4) + 255) / 256);
+  split_kernel<<<blocks, 256, 0, st>>>(T, C, X, ldx, vec, mx, out, inv_scale);
+  ICRL_LAUNCH_CHECK();
+  return ICRL_OK;
+}
+
+// partial sums of A^T B for A planes [2][a_rows][M] and the B planes in the workspace, then the reduction into C
+int contract(cudaStream_t st, int M, int N, long long T, const __half* a, long long a_rows, const Ws& w, int splits,
+             const float* inv_scale, int scale_stride, int permuted, float* C, int ldc) {
+  static bool attr_set = false;
+  if (!attr_set) {
+    ICRL_CUDA(cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    attr_set = true;
+  }
+  CUtensorMap ma, mb;
+  int rc;
+  if ((rc = make_map(&ma, a, M, T, a_rows, A_SLICE_ROWS))) return rc;
+  if ((rc = make_map(&mb, w.b, N, T, T, BK))) return rc;
+  dim3 grid(N / BN, M / BM, splits);
+  wgrad_kernel<<<grid, THREADS, SMEM_BYTES, st>>>(ma, mb, M, N, icrl_cdiv(T, BK), w.partial);
+  ICRL_LAUNCH_CHECK();
+  wgrad_reduce_kernel<<<icrl_cdiv((long long)M * N, 256), 256, 0, st>>>(M, N, splits, w.partial, inv_scale, scale_stride,
+                                                                        permuted, C, ldc);
+  ICRL_LAUNCH_CHECK();
+  return ICRL_OK;
+}
 
 }  // namespace
 
 // workspace bytes for icrl_wgrad_tc_impl
 size_t icrl_wgrad_tc_ws_bytes_impl(int M, int N, long long T, int splits) {
-  const long long Tp = round_up(T, 64);
-  return (size_t)4 * Tp * (M + N)            // hi + lo' of both operands, fp16
+  return (size_t)4 * T * (M + N)             // hi + lo' of both operands, fp16
          + (size_t)splits * M * N * 4        // partial tiles
          + (size_t)M * 8 + 1024;             // column maxima + inverse scales (+ alignment)
 }
 
 // C [M][ldc] = A^T B with A [T][lda] (M columns used, scaled per column), B [T][ldb] (N columns used).
-// The B operand's pre-pass alone (transpose + split into the workspace of the same M, N, T, splits): B is often final long
-// before A (the value chain's h stash exists after the forward), so a caller can run this on another stream beside
-// whatever produces A and then pass b_packed = 1 to the contraction.
+// The B operand's pre-pass alone (split into the workspace of the same M, N, T, splits): B is often final long before A
+// (the value chain's h stash exists after the forward), so a caller can run this on another stream beside whatever
+// produces A and then pass b_packed = 1 to the contraction.
 int icrl_wgrad_tc_pack_b_impl(cudaStream_t st, int M, int N, long long T, const float* B, int ldb, void* ws, size_t ws_bytes,
                               int splits) {
   ICRL_REQUIRE(M % BM == 0 && N % (BN * CLN) == 0 && T > 0 && splits >= 1, "wgrad_tc needs M a multiple of 128, N of 512");
   ICRL_REQUIRE(ws && ws_bytes >= icrl_wgrad_tc_ws_bytes_impl(M, N, T, splits), "wgrad_tc workspace too small");
-  ICRL_REQUIRE(ldb % 4 == 0 && (reinterpret_cast<uintptr_t>(B) & 15) == 0, "wgrad_tc_pack_b needs 16-byte aligned rows");
-  const long long Tp = round_up(T, 64);
-  __half* b_pk = reinterpret_cast<__half*>(ws) + (size_t)2 * M * Tp;
-  dim3 gb((unsigned)(Tp / 64), N / 64);
-  transpose_split64_kernel<<<gb, 256, 0, st>>>(T, Tp, N, B, ldb, nullptr, b_pk, b_pk + (size_t)N * Tp, nullptr);
-  ICRL_LAUNCH_CHECK();
-  return ICRL_OK;
+  return split(st, T, N, B, ldb, nullptr, carve(ws, M, N, T, splits).b, nullptr);
 }
 
 // colmax (nullable): M words holding the bit patterns of max_t |A[t][m]| when the caller has them already (the gate-table
@@ -413,52 +411,32 @@ int icrl_wgrad_tc_impl(cudaStream_t st, int M, int N, long long T, const float* 
                        float* C, int ldc, void* ws, size_t ws_bytes, int splits, const unsigned* colmax, int b_packed) {
   ICRL_REQUIRE(M % BM == 0 && N % (BN * CLN) == 0 && T > 0 && splits >= 1, "wgrad_tc needs M a multiple of 128, N of 512");
   ICRL_REQUIRE(ws && ws_bytes >= icrl_wgrad_tc_ws_bytes_impl(M, N, T, splits), "wgrad_tc workspace too small");
-  static bool attr_set = false;
-  if (!attr_set) {
-    ICRL_CUDA(cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    attr_set = true;
-  }
-  const long long Tp = round_up(T, 64);
-  __half* a_pk = reinterpret_cast<__half*>(ws);                          // [2][M][Tp]
-  __half* b_pk = a_pk + (size_t)2 * M * Tp;                             // [2][N][Tp]
-  float* partial = reinterpret_cast<float*>(b_pk + (size_t)2 * N * Tp);  // [splits][M][N]
-  unsigned* mx = reinterpret_cast<unsigned*>(partial + (size_t)splits * M * N);
-  float* inv_scale = reinterpret_cast<float*>(mx + M);      // (before mx may be redirected to the caller's maxima)
-  if (colmax) {
-    mx = const_cast<unsigned*>(colmax);
-  } else {
-    ICRL_CUDA(cudaMemsetAsync(mx, 0, (size_t)M * sizeof(unsigned), st));
+  const Ws w = carve(ws, M, N, T, splits);
+  const unsigned* mx = colmax;
+  if (!mx) {
+    ICRL_CUDA(cudaMemsetAsync(w.mx, 0, (size_t)M * sizeof(unsigned), st));
     dim3 grid(icrl_cdiv(M, 128), (unsigned)min((long long)592, (T + 255) / 256));
-    col_absmax_kernel<<<grid, 128, 0, st>>>(T, M, A, lda, mx);
+    col_absmax_kernel<<<grid, 128, 0, st>>>(T, M, A, lda, w.mx);
     ICRL_LAUNCH_CHECK();
+    mx = w.mx;
   }
-  const bool vec = lda % 4 == 0 && ldb % 4 == 0 && (reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(B) & 15) == 0;
-  if (vec) {
-    dim3 ga((unsigned)(Tp / 64), M / 64), gb((unsigned)(Tp / 64), N / 64);
-    transpose_split64_kernel<<<ga, 256, 0, st>>>(T, Tp, M, A, lda, mx, a_pk, a_pk + (size_t)M * Tp, inv_scale);
-    ICRL_LAUNCH_CHECK();
-    if (!b_packed) {
-      transpose_split64_kernel<<<gb, 256, 0, st>>>(T, Tp, N, B, ldb, nullptr, b_pk, b_pk + (size_t)N * Tp, nullptr);
-      ICRL_LAUNCH_CHECK();
-    }
-  } else {
-    dim3 blk(32, 8);
-    dim3 ga(icrl_cdiv(M, 32), (unsigned)(Tp / 32)), gb(icrl_cdiv(N, 32), (unsigned)(Tp / 32));
-    transpose_split_kernel<<<ga, blk, 0, st>>>(T, Tp, M, A, lda, mx, a_pk, a_pk + (size_t)M * Tp, inv_scale);
-    ICRL_LAUNCH_CHECK();
-    if (!b_packed) {
-      transpose_split_kernel<<<gb, blk, 0, st>>>(T, Tp, N, B, ldb, nullptr, b_pk, b_pk + (size_t)N * Tp, nullptr);
-      ICRL_LAUNCH_CHECK();
-    }
-  }
-  CUtensorMap ma, mb;
   int rc;
-  if ((rc = make_map(&ma, a_pk, Tp, M, A_SLICE_ROWS, 1))) return rc;
-  if ((rc = make_map(&mb, b_pk, Tp, N, BN, 2))) return rc;
-  dim3 grid(N / BN, M / BM, splits);
-  wgrad_kernel<<<grid, THREADS, SMEM_BYTES, st>>>(ma, mb, M, N, (int)(Tp / BK), partial);
-  ICRL_LAUNCH_CHECK();
-  wgrad_reduce_kernel<<<icrl_cdiv((long long)M * N, 256), 256, 0, st>>>(M, N, splits, partial, inv_scale, C, ldc);
-  ICRL_LAUNCH_CHECK();
-  return ICRL_OK;
+  if ((rc = split(st, T, M, A, lda, mx, w.a, w.inv_scale))) return rc;
+  if (!b_packed && (rc = split(st, T, N, B, ldb, nullptr, w.b, nullptr))) return rc;
+  return contract(st, M, N, T, w.a, T, w, splits, w.inv_scale, 1, 0, C, ldc);
+}
+
+// dW_hh [2048][ldc] from the chain backward's gate-gradient pairs: planes [2][pair_rows][2048] in the column order of
+// icrl_gate_pair_col, scaled by the power of two whose inverse is the device word *inv_scale; B [T][ldb] as above.
+int icrl_wgrad_tc_gate_pairs_impl(cudaStream_t st, int N, long long T, const void* pairs, long long pair_rows,
+                                  const float* inv_scale, const float* B, int ldb, float* C, int ldc, void* ws,
+                                  size_t ws_bytes, int splits, int b_packed) {
+  constexpr int M = 4 * ICRL_H;
+  ICRL_REQUIRE(N % (BN * CLN) == 0 && T > 0 && T <= pair_rows && splits >= 1, "wgrad_tc gate pairs: bad shape");
+  ICRL_REQUIRE(pairs && inv_scale && (reinterpret_cast<uintptr_t>(pairs) & 15) == 0, "wgrad_tc gate pairs: bad pointer");
+  ICRL_REQUIRE(ws && ws_bytes >= icrl_wgrad_tc_ws_bytes_impl(M, N, T, splits), "wgrad_tc workspace too small");
+  const Ws w = carve(ws, M, N, T, splits);
+  int rc;
+  if (!b_packed && (rc = split(st, T, N, B, ldb, nullptr, w.b, nullptr))) return rc;
+  return contract(st, M, N, T, reinterpret_cast<const __half*>(pairs), pair_rows, w, splits, inv_scale, 0, 1, C, ldc);
 }

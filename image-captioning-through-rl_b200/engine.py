@@ -120,7 +120,8 @@ class A2CEngine:
         # i.e. exactly what K data-parallel ranks compute (SURVEY.md 8e/H6).  K = 1 is the reference's single
         # carried-state chain over the whole batch.  The K chains advance in lockstep on the same CTAs.
         # wgrad: "tc" = the K = T weight-gradient contraction of the value chain on tcgen05 (wgrad_tc.cu; needs a
-        # workspace of ~10 KB per serial step), "simt" = fp32 CUDA-core GEMM with split-K.
+        # workspace of ~10 KB per serial step), "simt" = fp32 CUDA-core GEMM with split-K.  Steps whose value chain ran
+        # as tcgen05 pieces contract on tcgen05 either way: their gate gradients exist only as its fp16 pairs.
         if wgrad not in ("tc", "simt"):
             raise ValueError("wgrad must be 'tc' or 'simt'")
         self.wgrad = wgrad
@@ -615,8 +616,8 @@ class A2CEngine:
             h_packed = None
             with torch.cuda.stream(self._side_stream):
                 if self.wgrad == "tc" and self.chain_shards == 1:
-                    # the h stash is final since the forward: its transpose + split (B operand of dW_hh = dgates^T h) leaves
-                    # the critical path and runs beside the chain backward
+                    # the h stash is final since the forward: its split (B operand of dW_hh = dgates^T h) leaves the
+                    # critical path and runs beside the chain backward
                     _, gemm_ws, gemm_ws_floats, _ = self._bwd_workspaces(B, S, Tv, "")
                     _lib.call("icrl_wgrad_tc_pack_b", self._stream, 4 * H, H, Tv, _p(self._bufs["v_stash_h"]), H, _p(gemm_ws),
                               gemm_ws_floats * 4, 2, self.launches.ref)
@@ -641,7 +642,7 @@ class A2CEngine:
         cs_rows = max(SB, V, B)
         colsum_ws = self._buf("colsum_ws" + tag, int(_lib.call("icrl_colsum_ws_floats", cs_rows, 4 * H)) + 2 * H + 4 * H * 8)
         gemm_ws_floats = 24 * 4 * H * H
-        if self.wgrad == "tc":
+        if self.wgrad == "tc" or (not tag and self._tc is not None):
             if tag:       # policy side: dW_v (M = 1024) and dW_hh (M = 2048) contractions over S*B resp. n_cell*B rows
                 n = max(int(_lib.call("icrl_wgrad_tc_ws_bytes", 4 * H, H, (self._n_cell_max) * B, 2)),
                         int(_lib.call("icrl_wgrad_tc_ws_bytes", 1024, H, SB, 2)))
@@ -660,15 +661,24 @@ class A2CEngine:
         g = self._g
         colsum_ws, gemm_ws, gemm_ws_floats, dtable = self._bwd_workspaces(B, S, Tv, "")
         K = self.chain_shards
-        dgates = self._buf("v_dgates", K * (self._padded(Tv, 0) + 1) * 4 * H)
+        # fp32 gate gradients [rows][2048] (serial and segment kernels), or the tcgen05 pieces' fp16 pairs
+        # [2][rows][2048] (same bytes) with their inverse scale in v_dg_scale
+        rows = K * (self._padded(Tv, 0) + 1)
+        dgates = self._buf("v_dgates", rows * 4 * H)
+        dg_scale = self._buf("v_dg_scale", 1)
         if not launch_only_chain:
             lstm = Vn.valrnn.lstm
+            D = Vn.valrnn.caption_embedding.weight.shape[1]
+            tail = (_p(b["v_stash_h"]), _p(Vn.valrnn.caption_embedding.weight), _p(lstm.weight_ih_l0), _p(dtable), _p(colsum_ws),
+                    _p(gemm_ws), gemm_ws_floats * 4, _p(g(Vn.valrnn.caption_embedding.weight, True)), _p(g(lstm.weight_ih_l0)),
+                    _p(g(lstm.weight_hh_l0)), _p(g(lstm.bias_ih_l0)), _p(g(lstm.bias_hh_l0)))
             with self._phase("value_param_grads"):
-              _lib.call("icrl_value_chain_param_grads", st, Tv if K == 1 else K * (Tv + 1), V, Vn.valrnn.caption_embedding.weight.shape[1], _p(b["v_stream"]), _p(dgates), _p(b["v_stash_h"]),
-                      _p(Vn.valrnn.caption_embedding.weight), _p(lstm.weight_ih_l0), _p(dtable), _p(colsum_ws), _p(gemm_ws),
-                      gemm_ws_floats * 4, _p(g(Vn.valrnn.caption_embedding.weight, True)), _p(g(lstm.weight_ih_l0)),
-                      _p(g(lstm.weight_hh_l0)), _p(g(lstm.bias_ih_l0)), _p(g(lstm.bias_hh_l0)),
-                      B if K == 1 else 0, p0, S, int(bool(h_packed)), L)
+              if self._tc is not None:
+                _lib.call("icrl_value_chain_param_grads_pairs", st, Tv, V, D, _p(b["v_stream"]), _p(dgates), rows, _p(dg_scale),
+                          *tail, B, p0, S, int(bool(h_packed)), L)
+              else:
+                _lib.call("icrl_value_chain_param_grads", st, Tv if K == 1 else K * (Tv + 1), V, D, _p(b["v_stream"]), _p(dgates),
+                          *tail, B if K == 1 else 0, p0, S, int(bool(h_packed)), L)
             return
         # value head -> dh at the take positions + head gradients
         dh_take = self._buf("v_dh_take", SB * H)
@@ -683,7 +693,7 @@ class A2CEngine:
             ws, _ = self._tc_scratch("v", Pv)
             cp = self._buf("tc_cp_b", int(_lib.call("icrl_chain_tc_cp_floats", Pv)))
             _lib.call("icrl_chain_tc_lstm_bwd", st, Pv, seg_v, warm_v, _p(b["v_chain_pk"]), _p(b["v_stash_g"]), _p(b["v_stash_c"]),
-                      _p(b["v_take"]), _p(dh_take), SB, _p(dgates), _p(ws), _p(cp), _p(self._tc_err[8:]), L)
+                      _p(b["v_take"]), _p(dh_take), SB, _p(dgates), rows, _p(dg_scale), _p(ws), _p(cp), _p(self._tc_err[8:]), L)
           elif self._seg is not None:
             Kf, seg_v, _, warm = self._seg
             # backward pieces: 16 (8 per CTA group in one kernel step) when the forward has 16 or 32, else at most 8

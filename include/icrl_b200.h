@@ -86,8 +86,9 @@ int icrl_policy_rollout_fwd_tc(void* stream, int B, int V, int p0, int S, int gr
 
 /* ---- weight-gradient contraction on tcgen05 (wgrad_tc.cu): C [M][ldc] = A^T B for time-major fp32 operands A [T][lda]
  *      (M columns), B [T][ldb] (N columns); M a multiple of 128, N of 512 (the 4 N tiles of an M tile form a cluster
- *      that shares the A tile by TMA multicast).  Operands are transposed, scaled per A column and
- *      split into fp16 pairs by two pre-passes; f32 accumulation in TMEM is flushed to registers every 512 K elements.
+ *      that shares the A tile by TMA multicast).  Operands are scaled per A column and split into fp16
+ *      pairs [2][T][C] by an elementwise pre-pass and read MN-major by the MMA; f32 accumulation in TMEM is flushed to
+ *      registers every 512 K elements.
  *      ws: icrl_wgrad_tc_ws_bytes(M, N, T, splits) device bytes.  icrl_value_chain_param_grads takes this path by
  *      itself when its gemm_ws is at least icrl_wgrad_tc_ws_bytes(2048, 512, T, 2) bytes. */
 size_t icrl_wgrad_tc_ws_bytes(int M, int N, long long T, int splits);
@@ -288,7 +289,13 @@ int icrl_chains_tc_fwd_fused(void* stream, int v_pieces, long long v_seg, int v_
                              float* r_stash_h, void* r_ws, float* r_cp_state, float* r_err, int* launches);
 int icrl_chain_tc_lstm_bwd(void* stream, int pieces, long long seg, int warm, const void* packed,
                            const float* stash_gates, const float* stash_c, const int* take, const float* dh_take,
-                           long long take_rows, float* dgates, void* ws, float* cp_state, float* err, int* launches);
+                           long long take_rows, void* dg_pairs, long long pair_rows, float* dg_inv_scale, void* ws,
+                           float* cp_state, float* err, int* launches);
+/*      The gate gradients of the live positions come out as the fp16 pairs the recurrence itself runs on: dg_pairs =
+ *      [2][pair_rows][2048] halves (hi plane, then lo' plane; pair_rows >= pieces * seg + warm, 32-byte aligned), value =
+ *      (hi + lo'/2048) * *dg_inv_scale (one power of two per launch, written to the device word dg_inv_scale), columns of
+ *      each block of 32 hidden units in the order [unit quad][gate][unit of the quad] (natural a*512 + u -> stored
+ *      128 (u / 32) + 16 ((u % 32) / 4) + 4 a + u % 4).  icrl_value_chain_param_grads_pairs consumes them. */
 /* Debug aid: buf != NULL (24 device int64): cycle sums of cluster 0 / CTA 0's first epilogue warp, forward [0..5] =
  * {accumulator wait, gather, cell update, stores, cluster barrier, steps}, backward [8..13] likewise, [16..21] the reward
  * chain's first cluster when the forward launch is fused. */
@@ -328,12 +335,20 @@ int icrl_value_head_bwd(void* stream, int B, int S, const float* features, const
  *      scatter then sums the positions that consumed the same (column, row) token before one vector reduction each
  *      (ten times fewer reductions at 19 rollout steps) and hands the column maxima of dgates to the contraction.
  *      B = 0: any token stream of T positions (one reduction per position).
- *      h_packed = 1: gemm_ws already holds the transposed fp16 split of stash_h (icrl_wgrad_tc_pack_b(2048, 512, T, ...)). */
+ *      h_packed = 1: gemm_ws already holds the fp16 split of stash_h (icrl_wgrad_tc_pack_b(2048, 512, T, ...)). */
 int icrl_value_chain_param_grads(void* stream, int T, int V, int D, const int* tok_stream, const float* dgates,
                                  const float* stash_h, const float* E, const float* W_ih, float* dtable,
                                  float* colsum_ws, float* gemm_ws, size_t gemm_ws_bytes, float* dE, float* dW_ih,
                                  float* dW_hh, float* db_ih, float* db_hh, int B, int p0, int S, int h_packed,
                                  int* launches);
+/*      The same from icrl_chain_tc_lstm_bwd's gate-gradient pairs (dg_pairs, pair_rows, dg_inv_scale as written there)
+ *      instead of fp32 dgates; the contraction reads them as they lie.  Needs B > 0 (the stream's shape) and the wgrad_tc
+ *      workspace (gemm_ws_bytes >= icrl_wgrad_tc_ws_bytes(2048, 512, T, 2)). */
+int icrl_value_chain_param_grads_pairs(void* stream, int T, int V, int D, const int* tok_stream, const void* dg_pairs,
+                                       long long pair_rows, const float* dg_inv_scale, const float* stash_h, const float* E,
+                                       const float* W_ih, float* dtable, float* colsum_ws, float* gemm_ws,
+                                       size_t gemm_ws_bytes, float* dE, float* dW_ih, float* dW_hh, float* db_ih,
+                                       float* db_hh, int B, int p0, int S, int h_packed, int* launches);
 /*      reward (models.py:259-260 + GetRewards trainers.py:117-120): rewards [B][S] = cos(ve[b], se[s][b]). */
 int icrl_reward_cosine_fwd(void* stream, int B, int S, const float* ve, const float* se, float* rewards,
                            int* launches);
