@@ -47,10 +47,6 @@ SIGNATURES = {
     "icrl_build_stream_sharded": [P, I, I, I, I, I, P, P, P, P, LP],
     "icrl_chains_fwd_fused_sharded": [P, I, P, I, P, P, P, P, P, P, I, P, P, P, P, P, LP],
     "icrl_chain_lstm_bwd_sharded": [P, I, I, P, P, P, P, P, P, P, LP],
-    "icrl_chain_segment_len": [L, I, I],
-    "icrl_chain_segment_ws_floats": [],
-    "icrl_chains_fwd_fused_segmented": [P, I, I, P, I, P, P, P, P, P, P, I, P, P, P, P, P, P, LP],
-    "icrl_chain_lstm_bwd_segmented": [P, I, I, I, P, P, P, P, P, L, P, P, P, LP],
     "icrl_chain_tc_max_pieces": [],
     "icrl_chain_tc_weight_halves": [I],
     "icrl_chain_tc_ws_bytes": [I],
@@ -84,8 +80,7 @@ SIGNATURES = {
     "icrl_a2c_loss_fwd_bwd": [P, I, I, P, P, P, F, P, P, P, P, LP],
 }
 _RESTYPES = {"icrl_last_error": c_char_p, "icrl_wgrad_tc_ws_bytes": c_size_t, "icrl_decode_weight_halves": c_size_t, "icrl_colsum_ws_floats": c_size_t, "icrl_stream_len": c_longlong,
-             "icrl_chain_sync_bytes": c_size_t, "icrl_chain_segment_len": c_longlong, "icrl_chain_segment_ws_floats": c_size_t,
-             "icrl_chain_tc_weight_halves": c_size_t, "icrl_chain_tc_ws_bytes": c_size_t, "icrl_chain_tc_cp_floats": c_size_t,
+             "icrl_chain_sync_bytes": c_size_t, "icrl_chain_tc_weight_halves": c_size_t, "icrl_chain_tc_ws_bytes": c_size_t, "icrl_chain_tc_cp_floats": c_size_t,
              "icrl_policy_bwd_tc_ws_bytes": c_size_t}
 _NO_STATUS = set(_RESTYPES) | {"icrl_version", "icrl_chain_tc_max_pieces", "icrl_chain_tc_bwd_max_pieces", "icrl_vocab_pad"}
 

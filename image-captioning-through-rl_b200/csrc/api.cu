@@ -401,8 +401,7 @@ int icrl_chains_fwd_fused_sharded(void* stream, int shards, const int* v_stream,
                                   const int* r_stream, int r_T, const float* r_table, const float* r_W_hh,
                                   const float* r_b_hn, float* r_stash_h, void* sync_state, int* launches) {
   TRY(icrl_chains_fwd_fused_batched_impl(S_(stream), shards, v_stream, v_T, v_table, v_W_hh, v_stash_h, v_stash_c,
-                                         v_stash_gates, r_stream, r_T, r_table, r_W_hh, r_b_hn, r_stash_h, sync_state, 0,
-                                         nullptr, nullptr));
+                                         v_stash_gates, r_stream, r_T, r_table, r_W_hh, r_b_hn, r_stash_h, sync_state));
   bump(launches, 1);
   return ICRL_OK;
 }
@@ -411,41 +410,8 @@ int icrl_chain_lstm_bwd_sharded(void* stream, int shards, int T, const float* W_
                                 const float* stash_c, const int* take, const float* dh_take, float* dgates,
                                 void* sync_state, int* launches) {
   TRY(icrl_chain_lstm_bwd_batched_impl(S_(stream), shards, T, W_hh, stash_gates, stash_c, take, dh_take, dgates,
-                                       sync_state, 0, nullptr, 0, nullptr));
+                                       sync_state));
   bump(launches, 1);
-  return ICRL_OK;
-}
-
-long long icrl_chain_segment_len(long long T, int segments, int warm) {
-  if (segments < 2 || warm < 1 || T <= warm) return 0;
-  const long long seg = (T - warm + segments - 1) / segments;
-  return seg >= 2ll * warm ? seg : 0;
-}
-
-size_t icrl_chain_segment_ws_floats(void) { return 8 + 2 * 32 * 2 * 512 + 32 * 4 * 512; }
-
-int icrl_chains_fwd_fused_segmented(void* stream, int segments, int warm, const int* v_stream, int v_seg,
-                                    const float* v_table, const float* v_W_hh, float* v_stash_h, float* v_stash_c,
-                                    float* v_stash_gates, const int* r_stream, int r_seg, const float* r_table,
-                                    const float* r_W_hh, const float* r_b_hn, float* r_stash_h, float* segment_ws,
-                                    void* sync_state, int* launches) {
-  ICRL_REQUIRE(warm >= 1 && segment_ws, "segmented chains need a warm-up length and the segment workspace");
-  ICRL_REQUIRE(((long long)r_seg * segments + warm) < (1ll << 31) && ((long long)v_seg * segments + warm) < (1ll << 31),
-               "token stream longer than 2^31");
-  TRY(icrl_chains_fwd_fused_batched_impl(S_(stream), segments, v_stream, v_seg, v_table, v_W_hh, v_stash_h, v_stash_c,
-                                         v_stash_gates, r_stream, r_seg, r_table, r_W_hh, r_b_hn, r_stash_h, sync_state,
-                                         warm, segment_ws + 8, segment_ws));
-  bump(launches, v_seg > 0 ? 3 : 2);
-  return ICRL_OK;
-}
-
-int icrl_chain_lstm_bwd_segmented(void* stream, int segments, int warm, int seg, const float* W_hh,
-                                  const float* stash_gates, const float* stash_c, const int* take, const float* dh_take,
-                                  long long take_rows, float* dgates, float* segment_ws, void* sync_state, int* launches) {
-  ICRL_REQUIRE(warm >= 1 && segment_ws, "segmented chains need a warm-up length and the segment workspace");
-  TRY(icrl_chain_lstm_bwd_batched_impl(S_(stream), segments, seg, W_hh, stash_gates, stash_c, take, dh_take, dgates,
-                                       sync_state, warm, segment_ws + 8 + 2 * 32 * 2 * 512, take_rows * 512, segment_ws));
-  bump(launches, 2);
   return ICRL_OK;
 }
 

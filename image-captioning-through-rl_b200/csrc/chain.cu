@@ -18,11 +18,9 @@
 //     compute dh_{t-1}[u].
 //   * every spin is bounded (watchdog) and checks a global abort word, so a scheduling failure
 //     returns ICRL_ERR_WATCHDOG instead of hanging the GPU.
-//   * batched kernels (second half of the file): the same CTAs advance several recurrences in lockstep, sharing the
-//     register-resident weights and one exchange round trip -- either independent row shards from zero state
-//     ("chain shards", the numbers of K data-parallel ranks) or consecutive pieces of the ONE chain that start from zero
-//     state a warm-up early, discard those steps and are checked against the previous piece ("chain segments", the
-//     engine's default: the single chain's numbers to float rounding at 5-6x its speed; DESIGN.md 4.1).
+//   * batched kernels (second half of the file): the same CTAs advance K = 2, 4 or 8 independent row shards of the
+//     batch from zero state in lockstep ("chain shards", the numbers of K data-parallel ranks), sharing the
+//     register-resident weights and one exchange round trip.
 #include <cooperative_groups.h>
 #include "common.cuh"
 
@@ -439,7 +437,7 @@ __global__ void __launch_bounds__(THREADS, 1) chain_lstm_bwd_kernel(ChainBwdArgs
 // All per-step arrays of a shard use the same row stride (T + 1): stream [NB][stride], stash_h / stash_c
 // [NB][stride][H], stash_gates / dgates [NB][stride][4H] (row T unused / zero), take [NB][stride].
 
-constexpr int NB_MAX = 32;        // shards per forward launch (2 chunks of 16): exchange areas and check buffers are sized for it
+constexpr int NB_MAX = 8;         // shards per launch: the exchange areas are sized for it
 
 struct ChainFwdBatchArgs {
   const int* stream;          // [NB][stride]
@@ -451,30 +449,21 @@ struct ChainFwdBatchArgs {
   float* stash_h;             // [NB][stride][H]; row 0 = 0, row t+1 = h_t
   float* stash_c;             // LSTM: [NB][stride][H] or null
   float* stash_gates;         // LSTM: [NB][stride][4H] or null
-  unsigned long long* xchg;   // [chunks][2][NB][H] tagged words, zeroed before launch
+  unsigned long long* xchg;   // [2][NB][H] tagged words, zeroed before launch
   int* abort_flag;
   long long* prof;            // debug: {exchange wait, GEMV + reduce, pointwise + publish} cycles of CTA 0 thread 0, T
-  // Time-segment mode (warm > 0): the NB "shards" are consecutive segments of ONE chain.  stride = segment length,
-  // T = stride + warm, so shard b runs positions [b*stride, (b+1)*stride + warm) of the shared stream / stash arrays.
-  // Shards b >= 1 start from zero state `warm` positions early and discard those steps (nothing is stored for them);
-  // the state they reach at the end of the warm-up goes to warm_state for the caller's check against the state
-  // shard b-1 computes at the same position.
-  int warm;
-  float* warm_state;          // [NB][2][H]: h, c of shard b after its warm-up (rows of shard 0 unused)
 };
 
 // (Tried and dropped for this exchange, both slower at NB = 8: a unit-major word layout [unit][NB], 393 -> 426 ms, and
 // plain data + one release flag per unit polled with acquire loads, 393 -> 508 ms: the release store waits for the
 // warp's stash writes.)
-// NCH > 1 (built: 2 chunks of 8 or of 16): the NB * NCH shards are walked as NCH chunks of NB per step.  Chunk q
-// publishes its hidden vectors, then the CTA computes the other chunks before it polls for chunk q's next vectors: the exchange round trip through L2 (the wait
-// that bounds a single chunk) is covered by the other chunks' arithmetic.  Shard index = q * NB + lane group.
-template <int NG, int NB, int NCH>
-__device__ void chain_fwd_batched_body(const ChainFwdBatchArgs& p, int cta, float* sh_h /* [NCH][2][NB][H] */) {
+template <int NG, int NB>
+__device__ void chain_fwd_batched_body(const ChainFwdBatchArgs& p, int cta, float* sh_h /* [2][NB][H] */) {
   constexpr int GL = 32 / NB;                          // lanes per shard group after the transposed reduction
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int unit = cta * UNITS + warp;
-  const int b = lane / GL, sub = lane % GL;            // this lane's shard (within a chunk) for the pointwise stage
+  const int b = lane / GL, sub = lane % GL;            // this lane's shard for the pointwise stage
+  const int* my_stream = p.stream + (size_t)b * p.stride;
 
   float w[NG][16];
 #pragma unroll
@@ -485,147 +474,108 @@ __device__ void chain_fwd_batched_body(const ChainFwdBatchArgs& p, int cta, floa
       w[g][4 * j + 0] = t.x; w[g][4 * j + 1] = t.y; w[g][4 * j + 2] = t.z; w[g][4 * j + 3] = t.w;
     }
   const float bhn = (NG == 3) ? p.b_hn[unit] : 0.f;
-  float c[NCH], hprev[NCH], xg[NCH][NG];
-  int tok_next[NCH];
-#pragma unroll
-  for (int q = 0; q < NCH; ++q) {
-    const int bg = q * NB + b;
-    const int* my_stream = p.stream + (size_t)bg * p.stride;
-    c[q] = 0.f; hprev[q] = 0.f;
-    if (sub == 0 && !(p.warm > 0 && bg > 0)) {         // (later segments of one chain store nothing before their warm-up ends)
-      p.stash_h[(size_t)bg * p.stride * H + unit] = 0.f;
-      if (NG == 4 && p.stash_c) p.stash_c[(size_t)bg * p.stride * H + unit] = 0.f;
-    }
-    tok_next[q] = p.T > 1 ? my_stream[1] : 0;
+  float c = 0.f, hprev = 0.f, xg[NG];
+  if (sub == 0) {
+    p.stash_h[(size_t)b * p.stride * H + unit] = 0.f;
+    if (NG == 4 && p.stash_c) p.stash_c[(size_t)b * p.stride * H + unit] = 0.f;
+  }
+  int tok_next = p.T > 1 ? my_stream[1] : 0;
+  {
     const int tok0 = my_stream[0];
 #pragma unroll
-    for (int g = 0; g < NG; ++g) xg[q][g] = p.table[(size_t)tok0 * (NG * H) + g * H + unit];
+    for (int g = 0; g < NG; ++g) xg[g] = p.table[(size_t)tok0 * (NG * H) + g * H + unit];
   }
-  for (int i = threadIdx.x; i < NCH * 2 * NB * H; i += THREADS) sh_h[i] = 0.f;      // step-0 vectors: zero state
+  for (int i = threadIdx.x; i < 2 * NB * H; i += THREADS) sh_h[i] = 0.f;      // step-0 vectors: zero state
 
   long long prof_wait = 0, prof_gemv = 0, prof_rest = 0;
   const bool prof = p.prof != nullptr && cta == 0 && threadIdx.x == 0;
-  unsigned long long pre_a[NB], pre_b[NB];             // polled exchange words (tag, value) of the chunk about to run
   for (int t = 0; t < p.T; ++t) {
+    const long long c0 = prof ? clock64() : 0;
     const int buf = t & 1;
-    // (unrolled on purpose: with `#pragma unroll 1` the per-chunk state moves to thread-local memory and the two-chunk
-    // kernel measured 121.6 ms instead of 110.0 ms at B = 2048)
-#pragma unroll
-    for (int q = 0; q < NCH; ++q) {
-      const long long c0 = prof ? clock64() : 0;
-      const int bg = q * NB + b;
-      const bool seg_tail = p.warm > 0 && bg > 0;      // a later segment of one chain: its first `warm` steps are discarded
-      const int* my_stream = p.stream + (size_t)bg * p.stride;
-      unsigned long long* xq = p.xchg + (size_t)q * (2 * NB * H);
-      float* hb = sh_h + (size_t)(q * 2 + buf) * NB * H;
-      bool ok = true;
-      if (t > 0) {
-        const unsigned long long* src = xq + (size_t)((t - 1) & 1) * NB * H;
-        if (NCH == 1) exchange_issue<NB>(src, pre_a, pre_b);          // (chunked: already in flight, see below)
-        ok = exchange_complete<NB>(src, (unsigned)t, hb, p.abort_flag, pre_a, pre_b);
-      }
-      if (__syncthreads_or(!ok)) {
-        if (threadIdx.x == 0) atomicExch(p.abort_flag, 1);
-        return;
-      }
-      if (NCH > 1) {
-        // first poll of the NEXT chunk's vectors (published one chunk ago) rides under this chunk's arithmetic, so
-        // an exchange that has arrived costs no L2 round trip on the critical path
-        const int qn = (q + 1) % NCH, tn = q + 1 < NCH ? t : t + 1;
-        if (tn > 0 && tn < p.T)
-          exchange_issue<NB>(p.xchg + (size_t)qn * (2 * NB * H) + (size_t)((tn - 1) & 1) * NB * H, pre_a, pre_b);
-      }
-      const long long c1 = prof ? clock64() : 0;
-      float xg_n[NG];
-      {
-        const int tk = tok_next[q];
-        if (t + 1 < p.T) {
-#pragma unroll
-          for (int g = 0; g < NG; ++g) xg_n[g] = p.table[(size_t)tk * (NG * H) + g * H + unit];
-        } else {
-#pragma unroll
-          for (int g = 0; g < NG; ++g) xg_n[g] = 0.f;
-        }
-        tok_next[q] = (t + 2 < p.T) ? my_stream[t + 2] : 0;
-      }
-      // batch-NB GEMV: NG rows x 512 against NB hidden vectors, weights in registers
-      float acc[NG][NB];
-#pragma unroll
-      for (int g = 0; g < NG; ++g)
-#pragma unroll
-        for (int v = 0; v < NB; ++v) acc[g][v] = 0.f;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-#pragma unroll
-        for (int v = 0; v < NB; ++v) {
-          const float4 hv = *reinterpret_cast<const float4*>(&hb[v * H + 128 * j + 4 * lane]);
-#pragma unroll
-          for (int g = 0; g < NG; ++g) {
-            acc[g][v] = fmaf(w[g][4 * j + 0], hv.x, acc[g][v]);
-            acc[g][v] = fmaf(w[g][4 * j + 1], hv.y, acc[g][v]);
-            acc[g][v] = fmaf(w[g][4 * j + 2], hv.z, acc[g][v]);
-            acc[g][v] = fmaf(w[g][4 * j + 3], hv.w, acc[g][v]);
-          }
-        }
-      }
-      float sum[NG];
-#pragma unroll
-      for (int g = 0; g < NG; ++g) sum[g] = reduce_transposed<NB>(acc[g], lane);
-      const long long c2 = prof ? clock64() : 0;
-
-      const bool live = !seg_tail || t >= p.warm;      // warm-up steps of a later segment leave no trace
-      const bool warm_end = seg_tail && t == p.warm - 1;
-      const size_t row = (size_t)bg * p.stride + t;    // this shard's row of the per-step arrays
-      float hnew;
-      if constexpr (NG == 4) {
-        const float i = act_sigmoid(sum[0] + xg[q][0]);
-        const float f = act_sigmoid(sum[1] + xg[q][1]);
-        const float g = act_tanh(sum[2] + xg[q][2]);
-        const float o = act_sigmoid(sum[3 % NG] + xg[q][3 % NG]);
-        c[q] = f * c[q] + i * g;
-        hnew = o * act_tanh(c[q]);
-        if (p.stash_gates && live) {                   // the GL lanes of a shard share the four stores
-          if constexpr (GL >= 4) {
-            if (sub < 4) p.stash_gates[row * 4 * H + sub * H + unit] = sub == 0 ? i : (sub == 1 ? f : (sub == 2 ? g : o));
-          } else {
-            p.stash_gates[row * 4 * H + sub * H + unit] = sub == 0 ? i : f;
-            p.stash_gates[row * 4 * H + (2 + sub) * H + unit] = sub == 0 ? g : o;
-          }
-        }
-        if (sub == 4 % GL) {
-          if (p.stash_c && live) p.stash_c[(row + 1) * H + unit] = c[q];
-          if (warm_end) p.warm_state[(size_t)(2 * bg + 1) * H + unit] = c[q];
-        }
-      } else {
-        const float r = act_sigmoid(sum[0] + xg[q][0]);
-        const float z = act_sigmoid(sum[1] + xg[q][1]);
-        const float n = act_tanh(xg[q][2] + r * (sum[2] + bhn));
-        hnew = (1.f - z) * n + z * hprev[q];
-      }
-      hprev[q] = hnew;
-      if (sub == 6 % GL) st_tagged(xq + ((size_t)buf * NB + b) * H + unit, hnew, (unsigned)(t + 1));
-      if (sub == 5 % GL) {
-        if (live) p.stash_h[(row + 1) * H + unit] = hnew;
-        if (warm_end) p.warm_state[(size_t)(2 * bg) * H + unit] = hnew;
-      }
-#pragma unroll
-      for (int g = 0; g < NG; ++g) xg[q][g] = xg_n[g];
-      if (prof) { const long long c3 = clock64(); prof_wait += c1 - c0; prof_gemv += c2 - c1; prof_rest += c3 - c2; }
+    float* hb = sh_h + (size_t)buf * NB * H;
+    bool ok = true;
+    if (t > 0) ok = fetch_exchange_all<NB>(p.xchg + (size_t)((t - 1) & 1) * NB * H, (unsigned)t, hb, p.abort_flag);
+    if (__syncthreads_or(!ok)) {
+      if (threadIdx.x == 0) atomicExch(p.abort_flag, 1);
+      return;
     }
+    const long long c1 = prof ? clock64() : 0;
+    float xg_n[NG];
+    {
+      const int tk = tok_next;
+      if (t + 1 < p.T) {
+#pragma unroll
+        for (int g = 0; g < NG; ++g) xg_n[g] = p.table[(size_t)tk * (NG * H) + g * H + unit];
+      } else {
+#pragma unroll
+        for (int g = 0; g < NG; ++g) xg_n[g] = 0.f;
+      }
+      tok_next = (t + 2 < p.T) ? my_stream[t + 2] : 0;
+    }
+    // batch-NB GEMV: NG rows x 512 against NB hidden vectors, weights in registers
+    float acc[NG][NB];
+#pragma unroll
+    for (int g = 0; g < NG; ++g)
+#pragma unroll
+      for (int v = 0; v < NB; ++v) acc[g][v] = 0.f;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+#pragma unroll
+      for (int v = 0; v < NB; ++v) {
+        const float4 hv = *reinterpret_cast<const float4*>(&hb[v * H + 128 * j + 4 * lane]);
+#pragma unroll
+        for (int g = 0; g < NG; ++g) {
+          acc[g][v] = fmaf(w[g][4 * j + 0], hv.x, acc[g][v]);
+          acc[g][v] = fmaf(w[g][4 * j + 1], hv.y, acc[g][v]);
+          acc[g][v] = fmaf(w[g][4 * j + 2], hv.z, acc[g][v]);
+          acc[g][v] = fmaf(w[g][4 * j + 3], hv.w, acc[g][v]);
+        }
+      }
+    }
+    float sum[NG];
+#pragma unroll
+    for (int g = 0; g < NG; ++g) sum[g] = reduce_transposed<NB>(acc[g], lane);
+    const long long c2 = prof ? clock64() : 0;
+
+    const size_t row = (size_t)b * p.stride + t;       // this shard's row of the per-step arrays
+    float hnew;
+    if constexpr (NG == 4) {
+      const float i = act_sigmoid(sum[0] + xg[0]);
+      const float f = act_sigmoid(sum[1] + xg[1]);
+      const float g = act_tanh(sum[2] + xg[2]);
+      const float o = act_sigmoid(sum[3 % NG] + xg[3 % NG]);
+      c = f * c + i * g;
+      hnew = o * act_tanh(c);
+      if (p.stash_gates) {                             // the GL lanes of a shard share the four stores
+        if constexpr (GL >= 4) {
+          if (sub < 4) p.stash_gates[row * 4 * H + sub * H + unit] = sub == 0 ? i : (sub == 1 ? f : (sub == 2 ? g : o));
+        } else {
+          p.stash_gates[row * 4 * H + sub * H + unit] = sub == 0 ? i : f;
+          p.stash_gates[row * 4 * H + (2 + sub) * H + unit] = sub == 0 ? g : o;
+        }
+      }
+      if (p.stash_c && sub == 4 % GL) p.stash_c[(row + 1) * H + unit] = c;
+    } else {
+      const float r = act_sigmoid(sum[0] + xg[0]);
+      const float z = act_sigmoid(sum[1] + xg[1]);
+      const float n = act_tanh(xg[2] + r * (sum[2] + bhn));
+      hnew = (1.f - z) * n + z * hprev;
+    }
+    hprev = hnew;
+    if (sub == 6 % GL) st_tagged(p.xchg + ((size_t)buf * NB + b) * H + unit, hnew, (unsigned)(t + 1));
+    if (sub == 5 % GL) p.stash_h[(row + 1) * H + unit] = hnew;
+#pragma unroll
+    for (int g = 0; g < NG; ++g) xg[g] = xg_n[g];
+    if (prof) { const long long c3 = clock64(); prof_wait += c1 - c0; prof_gemv += c2 - c1; prof_rest += c3 - c2; }
   }
   if (prof) { p.prof[0] = prof_wait; p.prof[1] = prof_gemv; p.prof[2] = prof_rest; p.prof[3] = p.T; }
 }
 
-template <int NB, int NCH>
+template <int NB>
 __global__ void __launch_bounds__(THREADS, 1) chains_fwd_fused_batched_kernel(ChainFwdBatchArgs lstm, ChainFwdBatchArgs gru) {
   extern __shared__ __align__(16) float sh_dyn[];
-  if (blockIdx.x < CHAIN_CTAS) chain_fwd_batched_body<4, NB, NCH>(lstm, blockIdx.x, sh_dyn);
-  else chain_fwd_batched_body<3, NB, NCH>(gru, blockIdx.x - CHAIN_CTAS, sh_dyn);
-}
-template <int NB, int NCH>
-__global__ void __launch_bounds__(THREADS, 1) chain_gru_fwd_batched_kernel(ChainFwdBatchArgs gru) {
-  extern __shared__ __align__(16) float sh_dyn[];
-  chain_fwd_batched_body<3, NB, NCH>(gru, blockIdx.x, sh_dyn);
+  if (blockIdx.x < CHAIN_CTAS) chain_fwd_batched_body<4, NB>(lstm, blockIdx.x, sh_dyn);
+  else chain_fwd_batched_body<3, NB>(gru, blockIdx.x - CHAIN_CTAS, sh_dyn);
 }
 
 struct ChainBwdBatchArgs {
@@ -640,30 +590,22 @@ struct ChainBwdBatchArgs {
   unsigned long long* xchg;   // [2][shards][H]
   int shards;                 // total shards = gridDim.x / CHAIN_CTAS * NB
   int* abort_flag;
-  // Time-segment mode (warm > 0; see ChainFwdBatchArgs): shard k runs positions (k+1)*stride + warm - 1 down to k*stride of
-  // ONE chain.  All but the last shard start `warm` positions late with dh = dc = 0 and discard those steps; the
-  // gate gradients of their last warm-up step go to warm_dg for the caller's check against the row the next shard writes.
-  int warm;
-  float* warm_dg;             // [shards][4H]
   long long* prof;            // debug: cycles of CTA 0 thread 0 {coefficients + requests, poll wait, gate gradients + stores,
                               // barrier, contraction + reduce, barrier + publish}, then T
 };
 
-// Backward recurrence of NB shards per 64-CTA group (see chain_lstm_bwd_kernel for the single-chain scheme).
-// NCH > 1: every 64-CTA group walks NB * NCH shards as NCH chunks of NB per step (shard = (group * NCH + q) * NB + v).
-// A chunk publishes its dh vectors and the group works on the other chunks before it needs them back, and both the
-// stash rows and the first poll of the next chunk are requested one chunk ahead, so neither the L2 exchange nor the
-// stash reads sit on the critical path.
-template <int NB, int NCH, bool PROF>
+// Backward recurrence of NB shards per 64-CTA group (see chain_lstm_bwd_kernel for the single-chain scheme).  The stash
+// rows of the next step are requested before this step's gate gradients are computed, so they land under its arithmetic.
+template <int NB, bool PROF>
 __global__ void __launch_bounds__(THREADS, 1) chain_lstm_bwd_batched_kernel(ChainBwdBatchArgs p) {
   extern __shared__ __align__(16) float sh_dyn[];      // [2][NB][4H]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int group = blockIdx.x / CHAIN_CTAS, cta = blockIdx.x % CHAIN_CTAS;
-  const int sb0 = group * NCH * NB;                    // first shard of this group
+  const int sb = group * NB;                           // first shard of this group
   const int unit = cta * UNITS + warp;
   const int pu = 2 * threadIdx.x;
   const bool owner = (pu >= cta * UNITS) && (pu < cta * UNITS + UNITS);
-  const int myb = (lane >> 3) < NB ? (lane >> 3) : 0;  // shard (within a chunk) whose dh lane 8*myb publishes
+  const int myb = (lane >> 3) < NB ? (lane >> 3) : 0;  // shard whose dh lane 8*myb publishes
 
   // contraction split over the warps as in chain_lstm_bwd_kernel: wl[i][k] = W_hh[256w + 8 lane + k][8 cta + i]
   __shared__ float sh_part[UNITS][NB * UNITS];         // [warp][shard * 8 + unit]
@@ -676,8 +618,7 @@ __global__ void __launch_bounds__(THREADS, 1) chain_lstm_bwd_batched_kernel(Chai
     wl[4][k] = x1.x; wl[5][k] = x1.y; wl[6][k] = x1.z; wl[7][k] = x1.w;
   }
 
-  float2 dc[NCH][NB], gi[NB], gf[NB], gg[NB], go[NB], cc[NB], cp[NB];
-  int tk_prev[NCH];
+  float2 dc[NB], gi[NB], gf[NB], gg[NB], go[NB], cc[NB], cp[NB];
   auto load_step = [&](int shard, int t, float2& a_i, float2& a_f, float2& a_g, float2& a_o, float2& a_cc, float2& a_cp) {
     const float* ga = p.stash_gates + ((size_t)shard * p.stride + t) * 4 * H + pu;
     const float* ca = p.stash_c + ((size_t)shard * p.stride + t) * H + pu;
@@ -689,203 +630,28 @@ __global__ void __launch_bounds__(THREADS, 1) chain_lstm_bwd_batched_kernel(Chai
     a_cp = *reinterpret_cast<const float2*>(ca);
   };
 #pragma unroll
-  for (int q = 0; q < NCH; ++q) {
+  for (int v = 0; v < NB; ++v) dc[v] = make_float2(0.f, 0.f);
+  int tk_prev = p.T > 1 ? p.take[(size_t)(sb + myb) * p.stride + p.T - 2] : -1;
 #pragma unroll
-    for (int v = 0; v < NB; ++v) dc[q][v] = make_float2(0.f, 0.f);
-    tk_prev[q] = p.T > 1 ? p.take[(size_t)(sb0 + q * NB + myb) * p.stride + p.T - 2] : -1;
-  }
-#pragma unroll
-  for (int v = 0; v < NB; ++v) load_step(sb0 + v, p.T - 1, gi[v], gf[v], gg[v], go[v], cc[v], cp[v]);
-  unsigned long long pa[NB], pb[NB];                   // polled dh words of the chunk about to run
+  for (int v = 0; v < NB; ++v) load_step(sb + v, p.T - 1, gi[v], gf[v], gg[v], go[v], cc[v], cp[v]);
+  unsigned long long pa[NB], pb[NB];                   // polled dh words
   const bool prof = PROF && blockIdx.x == 0 && threadIdx.x == 0;       // PROF: the cycle-split build of the kernel
   long long pr[PROF ? 6 : 1] = {};
 
   for (int it = 0; it < p.T; ++it) {
     const int t = p.T - 1 - it;
+    const long long k0 = prof ? clock64() : 0;
+    float* dgb = sh_dyn + (it & 1) * NB * 4 * H;
+    bool ok = true;
+    const unsigned long long* src = p.xchg + ((size_t)((it - 1) & 1) * p.shards + sb) * H + pu;
+    if (it > 0) {
 #pragma unroll
-    for (int q = 0; q < NCH; ++q) {
-      const long long k0 = prof ? clock64() : 0;
-      const int sb = sb0 + q * NB;                     // first shard of this chunk
-      const int buf = (NCH == 1 ? it : it * NCH + q) & 1;
-      float* dgb = sh_dyn + buf * NB * 4 * H;
-      bool ok = true;
-      const unsigned long long* src = p.xchg + ((size_t)((it - 1) & 1) * p.shards + sb) * H + pu;
-      if (NCH == 1 && it > 0) {
-#pragma unroll
-        for (int v = 0; v < NB; ++v) ld_tagged2(src + (size_t)v * H, pa[v], pb[v]);
-      }
-      // coefficients that do not depend on dh
-      float2 kc[NB], ko[NB], ki[NB], kf[NB], kg[NB], fgate[NB], dh[NB];
-#pragma unroll
-      for (int v = 0; v < NB; ++v) {
-        const float tcx = act_tanh(cc[v].x), tcy = act_tanh(cc[v].y);
-        kc[v] = make_float2(go[v].x * (1.f - tcx * tcx), go[v].y * (1.f - tcy * tcy));
-        ko[v] = make_float2(tcx * go[v].x * (1.f - go[v].x), tcy * go[v].y * (1.f - go[v].y));
-        ki[v] = make_float2(gg[v].x * gi[v].x * (1.f - gi[v].x), gg[v].y * gi[v].y * (1.f - gi[v].y));
-        kf[v] = make_float2(cp[v].x * gf[v].x * (1.f - gf[v].x), cp[v].y * gf[v].y * (1.f - gf[v].y));
-        kg[v] = make_float2(gi[v].x * (1.f - gg[v].x * gg[v].x), gi[v].y * (1.f - gg[v].y * gg[v].y));
-        fgate[v] = gf[v];
-      }
-      const float inj = tk_prev[q] >= 0 ? p.dh_take[(size_t)tk_prev[q] * H + unit] : 0.f;
-      tk_prev[q] = t > 1 ? p.take[(size_t)(sb + myb) * p.stride + t - 2] : -1;
-      const long long k1 = prof ? clock64() : 0;
-      if (it == 0) {                                   // the recurrence starts with the gradient injected at the last position
-#pragma unroll
-        for (int v = 0; v < NB; ++v) {
-          dh[v] = make_float2(0.f, 0.f);
-          const int tk = p.take[(size_t)(sb + v) * p.stride + p.T - 1];
-          if (tk >= 0) dh[v] = *reinterpret_cast<const float2*>(p.dh_take + (size_t)tk * H + pu);
-        }
-      } else {
-        unsigned pending = (1u << NB) - 1u, spins = 0;     // rounds: all missing words are re-read together
-        while (true) {
-#pragma unroll
-          for (int v = 0; v < NB; ++v)
-            if ((pending >> v & 1u) && (unsigned)(pa[v] >> 32) == (unsigned)it && (unsigned)(pb[v] >> 32) == (unsigned)it)
-              pending &= ~(1u << v);
-          if (pending == 0) break;
-          if (++spins >= SPIN_LIMIT || ((spins & 1023u) == 0 && *(volatile int*)p.abort_flag != 0)) { ok = false; break; }
-#pragma unroll
-          for (int v = 0; v < NB; ++v)
-            if (pending >> v & 1u) ld_tagged2(src + (size_t)v * H, pa[v], pb[v]);
-        }
-#pragma unroll
-        for (int v = 0; v < NB; ++v) dh[v] = make_float2(__uint_as_float((unsigned)pa[v]), __uint_as_float((unsigned)pb[v]));
-      }
-      const long long k2 = prof ? clock64() : 0;
-      // requests for the chunk that runs next: its stash rows and (chunked) the first poll of its dh words
-      {
-        const int qn = (q + 1) % NCH, itn = q + 1 < NCH ? it : it + 1;
-        if (itn < p.T) {
-#pragma unroll
-          for (int v = 0; v < NB; ++v)
-            load_step(sb0 + qn * NB + v, p.T - 1 - itn, gi[v], gf[v], gg[v], go[v], cc[v], cp[v]);
-          if (NCH > 1 && itn > 0) {
-            const unsigned long long* srcn = p.xchg + ((size_t)((itn - 1) & 1) * p.shards + sb0 + qn * NB) * H + pu;
-#pragma unroll
-            for (int v = 0; v < NB; ++v) ld_tagged2(srcn + (size_t)v * H, pa[v], pb[v]);
-          }
-        }
-      }
-#pragma unroll
-      for (int v = 0; v < NB; ++v) {
-        const float dctx = dc[q][v].x + dh[v].x * kc[v].x, dcty = dc[q][v].y + dh[v].y * kc[v].y;
-        dc[q][v] = make_float2(dctx * fgate[v].x, dcty * fgate[v].y);
-        const float2 d_i = make_float2(dctx * ki[v].x, dcty * ki[v].y), d_f = make_float2(dctx * kf[v].x, dcty * kf[v].y);
-        const float2 d_g = make_float2(dctx * kg[v].x, dcty * kg[v].y), d_o = make_float2(dh[v].x * ko[v].x, dh[v].y * ko[v].y);
-        float* sd = dgb + v * 4 * H + pu;
-        *reinterpret_cast<float2*>(sd) = d_i;
-        *reinterpret_cast<float2*>(sd + H) = d_f;
-        *reinterpret_cast<float2*>(sd + 2 * H) = d_g;
-        *reinterpret_cast<float2*>(sd + 3 * H) = d_o;
-        const bool live = p.warm == 0 || it >= p.warm || sb + v == p.shards - 1;
-        if (owner && (live || it == p.warm - 1)) {
-          float* out = live ? p.dgates + ((size_t)(sb + v) * p.stride + t) * 4 * H + pu
-                            : p.warm_dg + (size_t)(sb + v) * 4 * H + pu;
-          *reinterpret_cast<float2*>(out) = d_i;
-          *reinterpret_cast<float2*>(out + H) = d_f;
-          *reinterpret_cast<float2*>(out + 2 * H) = d_g;
-          *reinterpret_cast<float2*>(out + 3 * H) = d_o;
-        }
-      }
-      const long long k3 = prof ? clock64() : 0;
-      if (__syncthreads_or(!ok)) {
-        if (threadIdx.x == 0) atomicExch(p.abort_flag, 1);
-        return;
-      }
-      const long long k4 = prof ? clock64() : 0;
-      long long k5 = k4;
-      if (t > 0) {
-        float part[NB * UNITS];
-#pragma unroll
-        for (int v = 0; v < NB; ++v) {
-          const float4 d0 = *reinterpret_cast<const float4*>(&dgb[v * 4 * H + 256 * warp + 8 * lane]);
-          const float4 d1 = *reinterpret_cast<const float4*>(&dgb[v * 4 * H + 256 * warp + 8 * lane + 4]);
-#pragma unroll
-          for (int i = 0; i < UNITS; ++i) {
-            float a = wl[i][0] * d0.x;
-            a = fmaf(wl[i][1], d0.y, a); a = fmaf(wl[i][2], d0.z, a); a = fmaf(wl[i][3], d0.w, a);
-            a = fmaf(wl[i][4], d1.x, a); a = fmaf(wl[i][5], d1.y, a); a = fmaf(wl[i][6], d1.z, a); a = fmaf(wl[i][7], d1.w, a);
-            part[v * UNITS + i] = a;
-          }
-        }
-        constexpr int R = NB * UNITS;                   // 8, 16 or 32 values: lane l ends with element l >> (5 - log2 R)
-        const float ps = reduce_transposed<R>(part, lane);
-        if ((lane & (32 / R - 1)) == 0) sh_part[warp][lane / (32 / R)] = ps;
-        k5 = prof ? clock64() : 0;
-        __syncthreads();
-        if (lane < R) {
-          float r = sh_part[lane & 7][(lane >> 3) * UNITS + warp];   // lane 8v + w': warp w' partial of (shard v, unit `warp`)
-          r += __shfl_xor_sync((unsigned)((1ull << R) - 1), r, 1);
-          r += __shfl_xor_sync((unsigned)((1ull << R) - 1), r, 2);
-          r += __shfl_xor_sync((unsigned)((1ull << R) - 1), r, 4);
-          if ((lane & 7) == 0) st_tagged(p.xchg + ((size_t)(it & 1) * p.shards + sb + (lane >> 3)) * H + unit, r + inj, (unsigned)(it + 1));
-        }
-      }
-      if constexpr (PROF) {
-        if (prof) {
-          const long long k6 = clock64();
-          pr[0] += k1 - k0; pr[1] += k2 - k1; pr[2] += k3 - k2; pr[3] += k4 - k3; pr[4] += k5 - k4; pr[5] += k6 - k5;
-        }
-      }
+      for (int v = 0; v < NB; ++v) ld_tagged2(src + (size_t)v * H, pa[v], pb[v]);
     }
-  }
-  if constexpr (PROF) {
-    if (prof) {
+    // coefficients that do not depend on dh
+    float2 kc[NB], ko[NB], ki[NB], kf[NB], kg[NB], fgate[NB], dh[NB];
 #pragma unroll
-      for (int i = 0; i < 6; ++i) p.prof[i] = pr[i];
-      p.prof[6] = p.T;
-    }
-  }
-}
-
-
-// Eight shards per 64-CTA group in ONE chunk.  A backward step costs about 1.0 us of fixed work (poll round trip, two
-// barriers, butterfly, publish) plus 0.32 us per shard, so eight shards per step amortise the fixed part twice as well as
-// four (B = 2048: 113.8 -> 95.9 ms per launch).  The per-shard register state does not fit eight times, so the
-// gate-gradient stage runs as two halves of four that share one set of stash registers: half 0 of a step is requested
-// during the previous step, half 1 at the top of the step (it lands under the poll wait and half 0's arithmetic).  All
-// eight dh vectors are polled together at the top.  (A generalisation to quarters with per-quarter polls -- 8 or 16
-// shards per group -- measured 107.5 / 117.8 ms: every quarter then waits for its own L2 round trip.)
-__global__ void __launch_bounds__(THREADS, 1) chain_lstm_bwd_batched8_kernel(ChainBwdBatchArgs p) {
-  constexpr int NB = 8, HB = 4;
-  extern __shared__ __align__(16) float sh_dyn[];      // [NB][4H] gate gradients of the current step
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int group = blockIdx.x / CHAIN_CTAS, cta = blockIdx.x % CHAIN_CTAS;
-  const int sb = group * NB;                           // first shard of this group
-  const int unit = cta * UNITS + warp;
-  const int pu = 2 * threadIdx.x;
-  const bool owner = (pu >= cta * UNITS) && (pu < cta * UNITS + UNITS);
-  const int myb = lane >> 3;                           // shard (within a half) whose dh lane 8*myb publishes
-
-  __shared__ float sh_part[2][UNITS][HB * UNITS];      // [half][warp][shard * 8 + unit]
-  float wl[UNITS][8];                                  // wl[i][k] = W_hh[256w + 8 lane + k][8 cta + i]
-#pragma unroll
-  for (int k = 0; k < 8; ++k) {
-    const float* src = p.w_hh + (size_t)(256 * warp + 8 * lane + k) * H + cta * UNITS;
-    const float4 x0 = *reinterpret_cast<const float4*>(src), x1 = *reinterpret_cast<const float4*>(src + 4);
-    wl[0][k] = x0.x; wl[1][k] = x0.y; wl[2][k] = x0.z; wl[3][k] = x0.w;
-    wl[4][k] = x1.x; wl[5][k] = x1.y; wl[6][k] = x1.z; wl[7][k] = x1.w;
-  }
-
-  float2 dc[NB], gi[HB], gf[HB], gg[HB], go[HB], cc[HB], cp[HB];
-  auto load_half = [&](int half, int t) {
-#pragma unroll
-    for (int v = 0; v < HB; ++v) {
-      const float* ga = p.stash_gates + ((size_t)(sb + half * HB + v) * p.stride + t) * 4 * H + pu;
-      const float* ca = p.stash_c + ((size_t)(sb + half * HB + v) * p.stride + t) * H + pu;
-      gi[v] = *reinterpret_cast<const float2*>(ga);
-      gf[v] = *reinterpret_cast<const float2*>(ga + H);
-      gg[v] = *reinterpret_cast<const float2*>(ga + 2 * H);
-      go[v] = *reinterpret_cast<const float2*>(ga + 3 * H);
-      cc[v] = *reinterpret_cast<const float2*>(ca + H);
-      cp[v] = *reinterpret_cast<const float2*>(ca);
-    }
-  };
-  float2 kc[HB], ko[HB], ki[HB], kf[HB], kg[HB], fgate[HB];
-  auto coefficients = [&]() {                          // everything of the gate gradients that does not depend on dh
-#pragma unroll
-    for (int v = 0; v < HB; ++v) {
+    for (int v = 0; v < NB; ++v) {
       const float tcx = act_tanh(cc[v].x), tcy = act_tanh(cc[v].y);
       kc[v] = make_float2(go[v].x * (1.f - tcx * tcx), go[v].y * (1.f - tcy * tcy));
       ko[v] = make_float2(tcx * go[v].x * (1.f - go[v].x), tcy * go[v].y * (1.f - go[v].y));
@@ -894,32 +660,9 @@ __global__ void __launch_bounds__(THREADS, 1) chain_lstm_bwd_batched8_kernel(Cha
       kg[v] = make_float2(gi[v].x * (1.f - gg[v].x * gg[v].x), gi[v].y * (1.f - gg[v].y * gg[v].y));
       fgate[v] = gf[v];
     }
-  };
-#pragma unroll
-  for (int v = 0; v < NB; ++v) dc[v] = make_float2(0.f, 0.f);
-  int tk_prev[2];
-#pragma unroll
-  for (int h = 0; h < 2; ++h) tk_prev[h] = p.T > 1 ? p.take[(size_t)(sb + h * HB + myb) * p.stride + p.T - 2] : -1;
-  load_half(0, p.T - 1);
-
-  for (int it = 0; it < p.T; ++it) {
-    const int t = p.T - 1 - it;
-    bool ok = true;
-    unsigned long long pa[NB], pb[NB];
-    const unsigned long long* src = p.xchg + ((size_t)((it - 1) & 1) * p.shards + sb) * H + pu;
-    if (it > 0) {
-#pragma unroll
-      for (int v = 0; v < NB; ++v) ld_tagged2(src + (size_t)v * H, pa[v], pb[v]);
-    }
-    coefficients();                                    // half 0 (its rows were requested during the previous step)
-    load_half(1, t);
-    float inj[2];
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      inj[h] = tk_prev[h] >= 0 ? p.dh_take[(size_t)tk_prev[h] * H + unit] : 0.f;
-      tk_prev[h] = t > 1 ? p.take[(size_t)(sb + h * HB + myb) * p.stride + t - 2] : -1;
-    }
-    float2 dh[NB];
+    const float inj = tk_prev >= 0 ? p.dh_take[(size_t)tk_prev * H + unit] : 0.f;
+    tk_prev = t > 1 ? p.take[(size_t)(sb + myb) * p.stride + t - 2] : -1;
+    const long long k1 = prof ? clock64() : 0;
     if (it == 0) {                                     // the recurrence starts with the gradient injected at the last position
 #pragma unroll
       for (int v = 0; v < NB; ++v) {
@@ -943,72 +686,79 @@ __global__ void __launch_bounds__(THREADS, 1) chain_lstm_bwd_batched8_kernel(Cha
 #pragma unroll
       for (int v = 0; v < NB; ++v) dh[v] = make_float2(__uint_as_float((unsigned)pa[v]), __uint_as_float((unsigned)pb[v]));
     }
+    const long long k2 = prof ? clock64() : 0;
+    if (t > 0) {                                       // the next step's stash rows
 #pragma unroll
-    for (int half = 0; half < 2; ++half) {
-      if (half == 1) {
-        coefficients();                                // half 1 (requested at the top of this step)
-        if (t > 0) load_half(0, t - 1);                // half 0 of the next step
-      }
+      for (int v = 0; v < NB; ++v) load_step(sb + v, t - 1, gi[v], gf[v], gg[v], go[v], cc[v], cp[v]);
+    }
 #pragma unroll
-      for (int v = 0; v < HB; ++v) {
-        const int s = half * HB + v;                   // shard within the group
-        const float dctx = dc[s].x + dh[s].x * kc[v].x, dcty = dc[s].y + dh[s].y * kc[v].y;
-        dc[s] = make_float2(dctx * fgate[v].x, dcty * fgate[v].y);
-        const float2 d_i = make_float2(dctx * ki[v].x, dcty * ki[v].y), d_f = make_float2(dctx * kf[v].x, dcty * kf[v].y);
-        const float2 d_g = make_float2(dctx * kg[v].x, dcty * kg[v].y), d_o = make_float2(dh[s].x * ko[v].x, dh[s].y * ko[v].y);
-        float* sd = sh_dyn + s * 4 * H + pu;
-        *reinterpret_cast<float2*>(sd) = d_i;
-        *reinterpret_cast<float2*>(sd + H) = d_f;
-        *reinterpret_cast<float2*>(sd + 2 * H) = d_g;
-        *reinterpret_cast<float2*>(sd + 3 * H) = d_o;
-        const bool live = p.warm == 0 || it >= p.warm || sb + s == p.shards - 1;
-        if (owner && (live || it == p.warm - 1)) {
-          float* out = live ? p.dgates + ((size_t)(sb + s) * p.stride + t) * 4 * H + pu
-                            : p.warm_dg + (size_t)(sb + s) * 4 * H + pu;
-          *reinterpret_cast<float2*>(out) = d_i;
-          *reinterpret_cast<float2*>(out + H) = d_f;
-          *reinterpret_cast<float2*>(out + 2 * H) = d_g;
-          *reinterpret_cast<float2*>(out + 3 * H) = d_o;
-        }
+    for (int v = 0; v < NB; ++v) {
+      const float dctx = dc[v].x + dh[v].x * kc[v].x, dcty = dc[v].y + dh[v].y * kc[v].y;
+      dc[v] = make_float2(dctx * fgate[v].x, dcty * fgate[v].y);
+      const float2 d_i = make_float2(dctx * ki[v].x, dcty * ki[v].y), d_f = make_float2(dctx * kf[v].x, dcty * kf[v].y);
+      const float2 d_g = make_float2(dctx * kg[v].x, dcty * kg[v].y), d_o = make_float2(dh[v].x * ko[v].x, dh[v].y * ko[v].y);
+      float* sd = dgb + v * 4 * H + pu;
+      *reinterpret_cast<float2*>(sd) = d_i;
+      *reinterpret_cast<float2*>(sd + H) = d_f;
+      *reinterpret_cast<float2*>(sd + 2 * H) = d_g;
+      *reinterpret_cast<float2*>(sd + 3 * H) = d_o;
+      if (owner) {
+        float* out = p.dgates + ((size_t)(sb + v) * p.stride + t) * 4 * H + pu;
+        *reinterpret_cast<float2*>(out) = d_i;
+        *reinterpret_cast<float2*>(out + H) = d_f;
+        *reinterpret_cast<float2*>(out + 2 * H) = d_g;
+        *reinterpret_cast<float2*>(out + 3 * H) = d_o;
       }
     }
+    const long long k3 = prof ? clock64() : 0;
     if (__syncthreads_or(!ok)) {
       if (threadIdx.x == 0) atomicExch(p.abort_flag, 1);
       return;
     }
+    const long long k4 = prof ? clock64() : 0;
+    long long k5 = k4;
     if (t > 0) {
+      float part[NB * UNITS];
 #pragma unroll
-      for (int half = 0; half < 2; ++half) {
-        float part[HB * UNITS];
+      for (int v = 0; v < NB; ++v) {
+        const float4 d0 = *reinterpret_cast<const float4*>(&dgb[v * 4 * H + 256 * warp + 8 * lane]);
+        const float4 d1 = *reinterpret_cast<const float4*>(&dgb[v * 4 * H + 256 * warp + 8 * lane + 4]);
 #pragma unroll
-        for (int v = 0; v < HB; ++v) {
-          const float* dg = sh_dyn + (half * HB + v) * 4 * H + 256 * warp + 8 * lane;
-          const float4 d0 = *reinterpret_cast<const float4*>(dg);
-          const float4 d1 = *reinterpret_cast<const float4*>(dg + 4);
-#pragma unroll
-          for (int i = 0; i < UNITS; ++i) {
-            float a = wl[i][0] * d0.x;
-            a = fmaf(wl[i][1], d0.y, a); a = fmaf(wl[i][2], d0.z, a); a = fmaf(wl[i][3], d0.w, a);
-            a = fmaf(wl[i][4], d1.x, a); a = fmaf(wl[i][5], d1.y, a); a = fmaf(wl[i][6], d1.z, a); a = fmaf(wl[i][7], d1.w, a);
-            part[v * UNITS + i] = a;
-          }
+        for (int i = 0; i < UNITS; ++i) {
+          float a = wl[i][0] * d0.x;
+          a = fmaf(wl[i][1], d0.y, a); a = fmaf(wl[i][2], d0.z, a); a = fmaf(wl[i][3], d0.w, a);
+          a = fmaf(wl[i][4], d1.x, a); a = fmaf(wl[i][5], d1.y, a); a = fmaf(wl[i][6], d1.z, a); a = fmaf(wl[i][7], d1.w, a);
+          part[v * UNITS + i] = a;
         }
-        sh_part[half][warp][lane] = reduce_transposed<HB * UNITS>(part, lane);     // 32 values: lane l ends with element l
       }
+      constexpr int R = NB * UNITS;                     // 8, 16 or 32 values: lane l ends with element l >> (5 - log2 R)
+      const float ps = reduce_transposed<R>(part, lane);
+      if ((lane & (32 / R - 1)) == 0) sh_part[warp][lane / (32 / R)] = ps;
+      k5 = prof ? clock64() : 0;
       __syncthreads();
-#pragma unroll
-      for (int half = 0; half < 2; ++half) {
-        float r = sh_part[half][lane & 7][(lane >> 3) * UNITS + warp];   // lane 8v + w': warp w' partial of (shard v, unit `warp`)
-        r += __shfl_xor_sync(0xffffffffu, r, 1);
-        r += __shfl_xor_sync(0xffffffffu, r, 2);
-        r += __shfl_xor_sync(0xffffffffu, r, 4);
-        if ((lane & 7) == 0)
-          st_tagged(p.xchg + ((size_t)(it & 1) * p.shards + sb + half * HB + (lane >> 3)) * H + unit, r + inj[half], (unsigned)(it + 1));
+      if (lane < R) {
+        float r = sh_part[lane & 7][(lane >> 3) * UNITS + warp];   // lane 8v + w': warp w' partial of (shard v, unit `warp`)
+        r += __shfl_xor_sync((unsigned)((1ull << R) - 1), r, 1);
+        r += __shfl_xor_sync((unsigned)((1ull << R) - 1), r, 2);
+        r += __shfl_xor_sync((unsigned)((1ull << R) - 1), r, 4);
+        if ((lane & 7) == 0) st_tagged(p.xchg + ((size_t)(it & 1) * p.shards + sb + (lane >> 3)) * H + unit, r + inj, (unsigned)(it + 1));
+      }
+    }
+    if constexpr (PROF) {
+      if (prof) {
+        const long long k6 = clock64();
+        pr[0] += k1 - k0; pr[1] += k2 - k1; pr[2] += k3 - k2; pr[3] += k4 - k3; pr[4] += k5 - k4; pr[5] += k6 - k5;
       }
     }
   }
+  if constexpr (PROF) {
+    if (prof) {
+#pragma unroll
+      for (int i = 0; i < 6; ++i) p.prof[i] = pr[i];
+      p.prof[6] = p.T;
+    }
+  }
 }
-
 
 struct ChainGruBwdArgs {
   int T;
@@ -1148,58 +898,6 @@ int coop_launch(const void* fn, int grid, void** args, cudaStream_t st) {
   return ICRL_OK;
 }
 
-
-// ---- time-segment checks.  err words are non-negative floats kept as a running maximum (integer atomicMax on the bit
-// pattern; a NaN difference has the largest pattern, so it trips the caller's threshold as well).
-__device__ __forceinline__ void err_max(float* slot, float v) { atomicMax(reinterpret_cast<int*>(slot), __float_as_int(fabsf(v))); }
-
-// Block k (k = 0..nb-2) compares the state segment k+1 reached after its warm-up with the state segment k computed at
-// the same position (stash row (k+1)*seg + warm).  err[0] = max |dh|, err[1] = max |dc| / max(1, |c|).
-__global__ void chain_warm_check_fwd_kernel(long long seg, int warm, const float* warm_state, const float* stash_h,
-                                            const float* stash_c, float* err) {
-  const int b = blockIdx.x + 1, u = threadIdx.x;
-  const size_t row = (size_t)b * seg + warm;
-  float dh = fabsf(warm_state[(size_t)(2 * b) * H + u] - stash_h[row * H + u]);
-  float dc = 0.f;                                      // the cell state is unbounded: error relative to max(1, |c|)
-  if (stash_c) {
-    const float ct = stash_c[row * H + u];
-    dc = fabsf(warm_state[(size_t)(2 * b + 1) * H + u] - ct) / fmaxf(1.f, fabsf(ct));
-  }
-  // warp maximum first (NaN-propagating through the integer compare)
-  int ih = __float_as_int(dh), ic = __float_as_int(dc);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    ih = max(ih, __shfl_xor_sync(0xffffffffu, ih, o));
-    ic = max(ic, __shfl_xor_sync(0xffffffffu, ic, o));
-  }
-  if ((threadIdx.x & 31) == 0) {
-    atomicMax(reinterpret_cast<int*>(err), ih);
-    if (stash_c) atomicMax(reinterpret_cast<int*>(err + 1), ic);
-  }
-}
-
-// Blocks 0..shards-2: gate gradients of segment k's last warm-up step against row (k+1)*seg written by segment k+1
-// (err[0] = max |difference|).  The remaining blocks reduce err[1] = max |dh_take| (the scale of the injected gradient).
-__global__ void chain_warm_check_bwd_kernel(int shards, long long seg, const float* warm_dg, const float* dgates,
-                                            const float* dh_take, long long n_take, float* err) {
-  int m = 0;
-  float* slot;
-  if ((int)blockIdx.x < shards - 1) {
-    const int k = blockIdx.x;
-    slot = err;
-    for (int i = threadIdx.x; i < 4 * H; i += blockDim.x)
-      m = max(m, __float_as_int(fabsf(warm_dg[(size_t)k * 4 * H + i] - dgates[((size_t)(k + 1) * seg) * 4 * H + i])));
-  } else {
-    slot = err + 1;
-    const long long nblk = gridDim.x - (shards - 1), blk = blockIdx.x - (shards - 1);
-    for (long long i = blk * blockDim.x + threadIdx.x; i < n_take; i += nblk * blockDim.x)
-      m = max(m, __float_as_int(fabsf(dh_take[i])));
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
-  if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<int*>(slot), m);
-}
-
 }  // namespace
 
 int icrl_chain_ctas() { return CHAIN_CTAS; }
@@ -1216,7 +914,7 @@ static ChainFwdArgs make_fwd(const int* stream, int T, const float* table, const
 
 // sync_state layout (device, caller-owned, >= icrl_chain_sync_bytes(), zeroed once by the caller):
 // [0,64) sticky abort word (+pad; cleared only by icrl_chain_check), then exchange buffers
-// (re-zeroed before every launch): lstm fwd 2*H, gru fwd 2*H, lstm bwd 2*H  64-bit words.
+// (re-zeroed before every launch): lstm fwd, gru fwd, lstm bwd, 2 * NB_MAX * H 64-bit words each.
 size_t icrl_chain_sync_bytes_impl() { return 64 + sizeof(unsigned long long) * 3 * (2 * NB_MAX * H); }
 
 static int* sync_abort(void* s) { return reinterpret_cast<int*>(s); }
@@ -1315,94 +1013,52 @@ static int coop_launch_smem(const void* fn, int grid, void** args, size_t smem, 
   return ICRL_OK;
 }
 
-// warm == 0: `nb` independent row shards, v_T / r_T steps each, arrays of shard k at row k * (T + 1).
-// warm  > 0: `nb` time segments of ONE chain; v_T / r_T are the segment lengths, every segment runs T + warm steps on the
-// shared arrays (row stride T) and the end-of-warm-up states are checked into seg_err[0..2] (see ChainFwdBatchArgs).
+// `nb` = 2, 4 or 8 independent row shards, v_T / r_T steps each, arrays of shard k at row k * (T + 1).
 int icrl_chains_fwd_fused_batched_impl(cudaStream_t st, int nb, const int* v_stream, int v_T, const float* v_table,
                                        const float* v_w_hh, float* v_stash_h, float* v_stash_c, float* v_stash_gates,
                                        const int* r_stream, int r_T, const float* r_table, const float* r_w_hh,
-                                       const float* r_b_hn, float* r_stash_h, void* sync_state, int warm,
-                                       float* warm_state, float* seg_err) {
-  ICRL_REQUIRE(nb == 2 || nb == 4 || nb == 8 || nb == 16 || nb == 32, "chain shards per launch must be 2, 4, 8, 16 or 32");
-  ICRL_REQUIRE(r_T > 0, "empty chain");
-  ICRL_REQUIRE(warm == 0 || (warm_state && seg_err && r_T >= warm && (v_T == 0 || v_T >= warm)),
-               "time segments must be at least as long as their warm-up");
+                                       const float* r_b_hn, float* r_stash_h, void* sync_state) {
+  ICRL_REQUIRE(nb == 2 || nb == 4 || nb == 8, "chain shards per launch must be 2, 4 or 8");
+  ICRL_REQUIRE(v_T > 0 && r_T > 0, "empty chain");
   ICRL_CUDA(cudaMemsetAsync(reinterpret_cast<char*>(sync_state) + 64, 0, icrl_chain_sync_bytes_impl() - 64, st));
-  const int pad = warm > 0 ? 0 : 1;
   ChainFwdBatchArgs a, b;
-  a.stream = v_stream; a.T = v_T + warm; a.stride = (long long)v_T + pad; a.table = v_table; a.w_hh = v_w_hh; a.b_hn = nullptr;
+  a.stream = v_stream; a.T = v_T; a.stride = (long long)v_T + 1; a.table = v_table; a.w_hh = v_w_hh; a.b_hn = nullptr;
   a.stash_h = v_stash_h; a.stash_c = v_stash_c; a.stash_gates = v_stash_gates; a.xchg = sync_xchg(sync_state, 0);
-  a.abort_flag = sync_abort(sync_state); a.prof = g_chain_prof; a.warm = warm; a.warm_state = warm_state;
-  b.stream = r_stream; b.T = r_T + warm; b.stride = (long long)r_T + pad; b.table = r_table; b.w_hh = r_w_hh; b.b_hn = r_b_hn;
+  a.abort_flag = sync_abort(sync_state); a.prof = g_chain_prof;
+  b.stream = r_stream; b.T = r_T; b.stride = (long long)r_T + 1; b.table = r_table; b.w_hh = r_w_hh; b.b_hn = r_b_hn;
   b.stash_h = r_stash_h; b.stash_c = nullptr; b.stash_gates = nullptr; b.xchg = sync_xchg(sync_state, 1);
   b.abort_flag = sync_abort(sync_state); b.prof = g_chain_prof ? g_chain_prof + 4 : nullptr;
-  b.warm = warm; b.warm_state = warm_state ? warm_state + (size_t)2 * NB_MAX * H : nullptr;
-  const size_t smem = (size_t)2 * nb * H * sizeof(float);      // [chunks][2][shards per chunk][H]
-  // 16 shards = 2 chunks of 8, 32 shards = 2 chunks of 16 (measured at B = 2048, ms per launch: 8 shards 146.5; 16 as
-  // 2 x 8 108.5; 24 as 3 x 8 107.0; 32 as 4 x 8 104.1, as 2 x 16 94.8)
-  if (v_T > 0) {
-    void* args[] = {&a, &b};
-    const void* fn = nb == 2 ? (const void*)chains_fwd_fused_batched_kernel<2, 1>
-                   : nb == 4 ? (const void*)chains_fwd_fused_batched_kernel<4, 1>
-                   : nb == 8 ? (const void*)chains_fwd_fused_batched_kernel<8, 1>
-                   : nb == 16 ? (const void*)chains_fwd_fused_batched_kernel<8, 2>
-                              : (const void*)chains_fwd_fused_batched_kernel<16, 2>;
-    const int rc = coop_launch_smem(fn, 2 * CHAIN_CTAS, args, smem, st);
-    if (rc != ICRL_OK) return rc;
-  } else {
-    void* args[] = {&b};
-    const void* fn = nb == 2 ? (const void*)chain_gru_fwd_batched_kernel<2, 1>
-                   : nb == 4 ? (const void*)chain_gru_fwd_batched_kernel<4, 1>
-                   : nb == 8 ? (const void*)chain_gru_fwd_batched_kernel<8, 1>
-                   : nb == 16 ? (const void*)chain_gru_fwd_batched_kernel<8, 2>
-                              : (const void*)chain_gru_fwd_batched_kernel<16, 2>;
-    const int rc = coop_launch_smem(fn, CHAIN_CTAS, args, smem, st);
-    if (rc != ICRL_OK) return rc;
-  }
-  if (warm > 0) {
-    if (v_T > 0)
-      chain_warm_check_fwd_kernel<<<nb - 1, H, 0, st>>>(v_T, warm, a.warm_state, v_stash_h, v_stash_c, seg_err);
-    chain_warm_check_fwd_kernel<<<nb - 1, H, 0, st>>>(r_T, warm, b.warm_state, r_stash_h, nullptr, seg_err + 2);
-    ICRL_CUDA(cudaGetLastError());
-  }
-  return ICRL_OK;
+  const size_t smem = (size_t)2 * nb * H * sizeof(float);      // [2][shards][H]
+  void* args[] = {&a, &b};
+  const void* fn = nb == 2 ? (const void*)chains_fwd_fused_batched_kernel<2>
+                 : nb == 4 ? (const void*)chains_fwd_fused_batched_kernel<4>
+                           : (const void*)chains_fwd_fused_batched_kernel<8>;
+  return coop_launch_smem(fn, 2 * CHAIN_CTAS, args, smem, st);
 }
 
 // shards = 2, 4 or 8 total; they are split over two 64-CTA groups (1, 2 or 4 shards per group).
-// warm > 0: time segments of one chain (T = segment length, arrays shared with row stride T); the warm-up check goes to
-// seg_err[3] (max |gate-gradient difference| at the segment joints) and seg_err[4] (max |dh_take|, n_take floats).
 int icrl_chain_lstm_bwd_batched_impl(cudaStream_t st, int shards, int T, const float* w_hh, const float* stash_gates,
                                      const float* stash_c, const int* take, const float* dh_take, float* dgates,
-                                     void* sync_state, int warm, float* warm_dg, long long n_take, float* seg_err) {
-  ICRL_REQUIRE(shards == 2 || shards == 4 || shards == 8 || shards == 16, "chain shards must be 2, 4, 8 or 16");
+                                     void* sync_state) {
+  ICRL_REQUIRE(shards == 2 || shards == 4 || shards == 8, "chain shards must be 2, 4 or 8");
   ICRL_REQUIRE(T > 0, "empty chain");
-  ICRL_REQUIRE(warm == 0 || (warm_dg && seg_err && T >= warm), "time segments must be at least as long as their warm-up");
   ICRL_CUDA(cudaMemsetAsync(reinterpret_cast<char*>(sync_state) + 64, 0, icrl_chain_sync_bytes_impl() - 64, st));
-  const long long stride = (long long)T + (warm > 0 ? 0 : 1);
-  if (warm == 0)
-    for (int k = 0; k < shards; ++k)                    // padding row T of every shard (feeds the weight-gradient GEMM)
-      ICRL_CUDA(cudaMemsetAsync(dgates + ((size_t)k * stride + T) * 4 * H, 0, 4 * H * sizeof(float), st));
+  const long long stride = (long long)T + 1;
+  for (int k = 0; k < shards; ++k)                      // padding row T of every shard (feeds the weight-gradient GEMM)
+    ICRL_CUDA(cudaMemsetAsync(dgates + ((size_t)k * stride + T) * 4 * H, 0, 4 * H * sizeof(float), st));
   ChainBwdBatchArgs a;
-  a.T = T + warm; a.stride = stride; a.w_hh = w_hh; a.stash_gates = stash_gates; a.stash_c = stash_c; a.take = take;
+  a.T = T; a.stride = stride; a.w_hh = w_hh; a.stash_gates = stash_gates; a.stash_c = stash_c; a.take = take;
   a.dh_take = dh_take; a.dgates = dgates; a.xchg = sync_xchg(sync_state, 2); a.shards = shards;
-  a.abort_flag = sync_abort(sync_state); a.warm = warm; a.warm_dg = warm_dg;
+  a.abort_flag = sync_abort(sync_state);
   a.prof = g_chain_prof ? g_chain_prof + 8 : nullptr;
   void* args[] = {&a};
-  // two 64-CTA groups of shards / 2 shards each.  Measured at B = 2048 (ms per launch): 8 shards as 4 per group 113.8;
-  // 16 shards as 8 per group in one chunk (chain_lstm_bwd_batched8_kernel) 95.9, as 2 chunks of 4 113.3; chunks of 2
-  // (8 shards as 2 x 2: 162.7, 16 as 4 x 2: 166.1) lose -- a chunk costs about 1.0 us + 0.32 us per shard.
+  // two 64-CTA groups of shards / 2 shards each (8 shards: 113.8 ms per launch at B = 2048, measured); a kernel step costs
+  // about 1.0 us of fixed work (poll round trip, two barriers, butterfly, publish) plus 0.32 us per shard
   const int nb = shards / 2;
-  const void* fn = shards == 2 ? (const void*)chain_lstm_bwd_batched_kernel<1, 1, false>
-                 : shards == 4 ? (const void*)chain_lstm_bwd_batched_kernel<2, 1, false>
-                 : shards == 8 ? (a.prof ? (const void*)chain_lstm_bwd_batched_kernel<4, 1, true>
-                                         : (const void*)chain_lstm_bwd_batched_kernel<4, 1, false>)
-                               : (const void*)chain_lstm_bwd_batched8_kernel;
-  const size_t smem = (size_t)(shards == 16 ? 1 : 2) * nb * 4 * H * sizeof(float);
-  const int rc = coop_launch_smem(fn, 2 * CHAIN_CTAS, args, smem, st);
-  if (rc != ICRL_OK) return rc;
-  if (warm > 0) {
-    chain_warm_check_bwd_kernel<<<shards - 1 + 64, 256, 0, st>>>(shards, T, warm_dg, dgates, dh_take, n_take, seg_err + 3);
-    ICRL_CUDA(cudaGetLastError());
-  }
-  return ICRL_OK;
+  const void* fn = shards == 2 ? (const void*)chain_lstm_bwd_batched_kernel<1, false>
+                 : shards == 4 ? (const void*)chain_lstm_bwd_batched_kernel<2, false>
+                 : a.prof      ? (const void*)chain_lstm_bwd_batched_kernel<4, true>
+                               : (const void*)chain_lstm_bwd_batched_kernel<4, false>;
+  const size_t smem = (size_t)2 * nb * 4 * H * sizeof(float);
+  return coop_launch_smem(fn, 2 * CHAIN_CTAS, args, smem, st);
 }

@@ -74,11 +74,10 @@ int icrl_build_stream_sharded_impl(cudaStream_t st, int B, int p0, int S, int ex
 int icrl_chains_fwd_fused_batched_impl(cudaStream_t st, int nb, const int* v_stream, int v_T, const float* v_table,
                                        const float* v_w_hh, float* v_stash_h, float* v_stash_c, float* v_stash_gates,
                                        const int* r_stream, int r_T, const float* r_table, const float* r_w_hh,
-                                       const float* r_b_hn, float* r_stash_h, void* sync_state, int warm,
-                                       float* warm_state, float* seg_err);
+                                       const float* r_b_hn, float* r_stash_h, void* sync_state);
 int icrl_chain_lstm_bwd_batched_impl(cudaStream_t st, int shards, int T, const float* w_hh, const float* stash_gates,
                                      const float* stash_c, const int* take, const float* dh_take, float* dgates,
-                                     void* sync_state, int warm, float* warm_dg, long long n_take, float* seg_err);
+                                     void* sync_state);
 void icrl_chain_set_profile_impl(long long* buf);
 size_t icrl_wgrad_tc_ws_bytes_impl(int M, int N, long long T, int splits);
 int icrl_wgrad_tc_impl(cudaStream_t st, int M, int N, long long T, const float* A, int lda, const float* B, int ldb,

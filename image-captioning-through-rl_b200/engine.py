@@ -8,8 +8,9 @@ Single-pass formulation (verified against the unmodified reference, SURVEY.md se
   policy   one incremental LSTM pass with sampling (instead of re-running the prefix every step)
   value    ONE serial LSTM chain over the column-major token stream, h taken at the last B
            positions of each step block; head evaluated in collapsed form.  By default the chain
-           is advanced as up to 32 consecutive pieces in lockstep, each with a discarded warm-up
-           that is verified against the previous piece on every step (chain segments, DESIGN 4.1)
+           is advanced as hundreds of consecutive pieces in lockstep on the tensor cores, each with
+           a discarded warm-up that is verified against the previous piece on every step (chain
+           pieces, DESIGN 4.1)
   reward   ONE serial GRU chain, semantic/visual embeds batched over all steps, fused cosine
   loss     advantage = values - rewards, gradient seeds for both networks
   backward policy BPTT (batched GEMMs + S serial cell steps), value-chain BPTT kernel, weight
@@ -79,10 +80,8 @@ def plan_rollout(captions, level=None):
 class A2CEngine:
     DECODE_MODES = ("fused", "tc", "simt")
 
-    CHAIN_ENGINES = ("tc", "simt")
-
     def __init__(self, a2c_network, reward_network, use_tc=None, decode="fused", chain_shards=1, wgrad="tc",
-                 chain_segments=32, chain_warmup=256, chain_tol=1e-5, chain_bwd_segments=None, chain_engine="tc",
+                 chain_segments=32, chain_warmup=256, chain_tol=1e-5, chain_engine="tc",
                  chain_pieces=None, chain_adapt=True, chain_warmup_min=32, policy_bptt="tc", chain_fuse_fwd=True, overlap_backward=True):
         self.policy = a2c_network.policy_network
         self.value = a2c_network.value_network
@@ -128,37 +127,26 @@ class A2CEngine:
         if chain_shards not in (1, 2, 4, 8):
             raise ValueError("chain_shards must be 1, 2, 4 or 8")
         self.chain_shards = int(chain_shards)
-        # chain_segments = K > 1 keeps the reference's ONE carried-state chain but advances K consecutive pieces of it in
-        # lockstep: piece k >= 1 starts from zero state `chain_warmup` positions early and throws those steps away.  A
-        # gated recurrence forgets its initial state, so the piece then carries the single chain's state up to float
-        # rounding.  That is verified on every step (state at the end of each warm-up vs the state the previous piece
-        # computes at the same position; gate gradients at the joints for the backward recurrence); a step whose check
-        # exceeds chain_tol is re-run on the serial kernels and the warm-up is lengthened.  Chains too short for K
-        # pieces of >= 2 warm-ups use fewer pieces or the serial kernels.  chain_segments = 1: always serial.
-        # More than 8 pieces run as two chunks inside a kernel step (16 = 2 x 8, 32 = 2 x 16): a chunk's exchange round
-        # trip is covered by the arithmetic of the other chunk.  The backward recurrence uses at most 16 pieces (8 per
-        # CTA group; every 2nd forward joint when the forward has 32).
+        # chain_segments = 1 runs the reference's ONE carried-state chain on the serial kernels; any other value cuts it
+        # into tcgen05 pieces (chain_engine below).
         if chain_segments not in (1, 2, 4, 8, 16, 32):
             raise ValueError("chain_segments must be 1, 2, 4, 8, 16 or 32")
-        # chain_bwd_segments: backward pieces (None = 16 when the forward has 16 or 32, else min(forward, 8)); experiments.
-        if chain_bwd_segments not in (None, 2, 4, 8, 16):
-            raise ValueError("chain_bwd_segments must be None, 2, 4, 8 or 16")
-        self.chain_bwd_segments = chain_bwd_segments
         self.chain_segments = 1 if self.chain_shards > 1 else int(chain_segments)
         self.chain_warmup = int(chain_warmup)
         self.chain_tol = float(chain_tol)
         if self.chain_warmup < 1:
             raise ValueError("chain_warmup must be positive")
-        # chain_engine: "tc" (default) = chain pieces on tcgen05 (chain_tc.cu): hundreds of lockstep pieces, 128 per cluster of
-        # 8 CTAs, one kernel step = H_prev [pieces x 512] . W_hh^T on the tensor cores.  The warm-up is sized PER CHAIN
-        # (value LSTM forward + backward, reward GRU) from the contraction rate measured on every step (errors half-way
-        # through and at the end of the warm-up): it grows before the check can fail and shrinks again after
-        # `_SHRINK_AFTER` clean steps; a failed check re-runs the chains with a longer warm-up, and only a chain that
-        # cannot be cut at all runs on the serial kernels.  "simt" = the CUDA-core segment kernels of chain.cu
-        # (chain_segments pieces, fixed warm-up, serial re-run on failure).  chain_segments = 1 forces the serial kernels.
-        if chain_engine not in self.CHAIN_ENGINES:
-            raise ValueError("chain_engine must be one of %s" % (self.CHAIN_ENGINES,))
-        self.chain_engine = chain_engine
+        # chain_engine "tc" = chain pieces on tcgen05 (chain_tc.cu): hundreds of lockstep pieces, 128 per cluster of 8 CTAs,
+        # one kernel step = H_prev [pieces x 512] . W_hh^T on the tensor cores.  Piece k >= 1 starts from zero state a
+        # warm-up early and throws those steps away: a gated recurrence forgets its initial state, so the piece then
+        # carries the single chain's state up to float rounding, which the joint check verifies on every step.  The
+        # warm-up is sized PER CHAIN (value LSTM forward + backward, reward GRU) from the contraction rate measured on
+        # every step (errors half-way through and at the end of the warm-up): it grows before the check can fail and
+        # shrinks again after `_SHRINK_AFTER` clean steps; a failed check re-runs the chains with a longer warm-up, and
+        # after _TC_ATTEMPTS failures, or for a chain too short to cut, the step runs on the serial kernels.
+        if chain_engine != "tc":
+            raise ValueError("chain_engine must be 'tc': the CUDA-core chain-segment engine ('simt') was removed; "
+                             "chain_segments=1 runs the serial kernels")
         self.chain_pieces = None if chain_pieces is None else int(chain_pieces)
         if self.chain_pieces is not None and self.chain_pieces < 2:
             raise ValueError("chain_pieces must be at least 2")
@@ -180,13 +168,10 @@ class A2CEngine:
         self._clean = {"v": 0, "r": 0, "b": 0}
         self._hold = {"v": 0, "r": 0, "b": 0}
         self._tc = None                   # {"v": (P, seg, warm) | None, "r": (P, seg, warm)} of the current step
-        self.segment_stats = {"steps": 0, "segmented_steps": 0, "fallbacks": 0, "reruns": 0, "max_err": [0.0] * 5,
-                              "tc_max_err": [0.0] * 16, "warm_history": []}
-        self._seg = None                  # (K, seg_v, seg_r, warm) of the current step, None = serial kernels
-        self._seg_strikes = 0
+        self.segment_stats = {"steps": 0, "segmented_steps": 0, "fallbacks": 0, "reruns": 0, "tc_max_err": [0.0] * 16,
+                              "warm_history": []}
         self._seg_unverified = False
         with torch.cuda.device(dev):
-            self._seg_ws = torch.zeros(int(_lib.call("icrl_chain_segment_ws_floats")), dtype=torch.float32, device=dev)
             self.sync_state = torch.zeros(int(_lib.call("icrl_chain_sync_bytes")), dtype=torch.uint8, device=dev)
             # [0:3] loss, mean reward, mean advantage; [4:20] joint-check words of the tc chain launches (value forward
             # 4..7, reward forward 8..11, value backward 12..17): read together in ONE device-to-host copy per step
@@ -307,7 +292,7 @@ class A2CEngine:
             self.pack_reward()
 
     def _use_tc_chains(self):
-        return self.chain_engine == "tc" and self.chain_segments > 1 and self.chain_shards == 1
+        return self.chain_segments > 1 and self.chain_shards == 1
 
     def _reward_changed(self):
         """The reward network is frozen during A2C training (trainers.py:372-373) and its derived operands are packed once;
@@ -434,34 +419,17 @@ class A2CEngine:
             return Tv, Tr
         Tv = int(_lib.call("icrl_stream_len", B, p0, S, 0))
         Tr = int(_lib.call("icrl_stream_len", B, p0, S, 1))
-        self._seg, self._tc = None, None
-        if not serial:
-            if self._use_tc_chains():
-                self._tc = self._pick_pieces(Tv, Tr)
-            elif self.chain_segments > 1:
-                self._seg = self._pick_segments(Tv, Tr)
+        self._tc = self._pick_pieces(Tv, Tr) if not serial and self._use_tc_chains() else None
         nv, nr = self._padded(Tv, 0), self._padded(Tr, 1)
         v_stream, v_take, v_pos = self._buf("v_stream", nv, i32), self._buf("v_take", nv, i32), self._buf("v_pos", S * B, i32)
         r_stream, r_pos = self._buf("r_stream", nr, i32), self._buf("r_pos", S * B, i32)
         _lib.call("icrl_build_stream", st, B, p0, S, 0, _p(tokcm), _p(v_stream), _p(v_take), _p(v_pos), L)
         _lib.call("icrl_build_stream", st, B, p0, S, 1, _p(tokcm), _p(r_stream), None, _p(r_pos), L)
-        if self._seg is not None or self._tc is not None:   # the last piece runs past the end of the chain: pad with token 0 / "no output"
+        if self._tc is not None:          # the last piece runs past the end of the chain: pad with token 0 / "no output"
             v_stream[Tv:nv].zero_()
             v_take[Tv:nv].fill_(-1)
             r_stream[Tr:nr].zero_()
         return Tv, Tr
-
-    def _pick_segments(self, Tv, Tr):
-        """(K, seg_v, seg_r, warm) for chains of Tv / Tr positions, or None when they are too short."""
-        warm = self.chain_warmup
-        for K in (32, 16, 8, 4, 2):
-            if K > self.chain_segments:
-                continue
-            seg_r = int(_lib.call("icrl_chain_segment_len", Tr, K, warm))
-            seg_v = int(_lib.call("icrl_chain_segment_len", Tv, K, warm)) if Tv > 0 else 0
-            if seg_r > 0 and (Tv == 0 or seg_v > 0):
-                return (K, seg_v, seg_r, warm)
-        return None
 
     def _pieces_for(self, T, warm, pmax=None):
         """(P, seg) for a chain of T positions cut into tcgen05 pieces with a `warm`-position warm-up, or None when it is
@@ -521,13 +489,10 @@ class A2CEngine:
 
     def _padded(self, T, which):
         """Positions the arrays of a chain must hold (which: 0 = value, 1 = reward)."""
-        if self._tc is not None:
-            lays = [self._tc["r"]] if which else [self._tc["v"], self._tc.get("b")]
-            return max([T] + [l[0] * l[1] + l[2] for l in lays if l is not None])
-        if self._seg is None:
+        if self._tc is None:
             return T
-        K, seg_v, seg_r, warm = self._seg
-        return K * (seg_r if which else seg_v) + warm
+        lays = [self._tc["r"]] if which else [self._tc["v"], self._tc.get("b")]
+        return max([T] + [l[0] * l[1] + l[2] for l in lays if l is not None])
 
     def _tc_scratch(self, key, P):
         """(ws, cp_state) of a tc chain launch; the tensors stay referenced by the engine."""
@@ -560,12 +525,6 @@ class A2CEngine:
                           None, _p(v_h), _p(v_c), _p(v_g), _p(ws_v), _p(cp_v), _p(self._tc_err[0:]), L)
                 _lib.call("icrl_chain_tc_fwd", st, 1, Pr, seg_r, warm_r, _p(b["r_stream"]), _p(b["r_table"]), _p(b["r_chain_pk"]),
                           _p(R.rewrnn.gru.bias_hh_l0[2 * H:]), _p(r_h), None, None, _p(ws_r), _p(cp_r), _p(self._tc_err[4:]), L)
-          elif self._seg is not None:
-            Ks, seg_v, seg_r, warm = self._seg
-            _lib.call("icrl_chains_fwd_fused_segmented", st, Ks, warm, _p(b["v_stream"]), seg_v, _p(b["v_table"]),
-                  _p(Vn.valrnn.lstm.weight_hh_l0), _p(v_h), _p(v_c), _p(v_g), _p(b["r_stream"]), seg_r, _p(b["r_table"]),
-                  _p(R.rewrnn.gru.weight_hh_l0), _p(R.rewrnn.gru.bias_hh_l0[2 * H:]), _p(r_h), _p(self._seg_ws),
-                  _p(self.sync_state), L)
           elif K > 1:
             _lib.call("icrl_chains_fwd_fused_sharded", st, K, _p(b["v_stream"]), Tv, _p(b["v_table"]),
                   _p(Vn.valrnn.lstm.weight_hh_l0), _p(v_h), _p(v_c), _p(v_g), _p(b["r_stream"]), Tr, _p(b["r_table"]),
@@ -661,7 +620,7 @@ class A2CEngine:
         g = self._g
         colsum_ws, gemm_ws, gemm_ws_floats, dtable = self._bwd_workspaces(B, S, Tv, "")
         K = self.chain_shards
-        # fp32 gate gradients [rows][2048] (serial and segment kernels), or the tcgen05 pieces' fp16 pairs
+        # fp32 gate gradients [rows][2048] (serial and shard kernels), or the tcgen05 pieces' fp16 pairs
         # [2][rows][2048] (same bytes) with their inverse scale in v_dg_scale
         rows = K * (self._padded(Tv, 0) + 1)
         dgates = self._buf("v_dgates", rows * 4 * H)
@@ -694,16 +653,6 @@ class A2CEngine:
             cp = self._buf("tc_cp_b", int(_lib.call("icrl_chain_tc_cp_floats", Pv)))
             _lib.call("icrl_chain_tc_lstm_bwd", st, Pv, seg_v, warm_v, _p(b["v_chain_pk"]), _p(b["v_stash_g"]), _p(b["v_stash_c"]),
                       _p(b["v_take"]), _p(dh_take), SB, _p(dgates), rows, _p(dg_scale), _p(ws), _p(cp), _p(self._tc_err[8:]), L)
-          elif self._seg is not None:
-            Kf, seg_v, _, warm = self._seg
-            # backward pieces: 16 (8 per CTA group in one kernel step) when the forward has 16 or 32, else at most 8
-            Ks = self.chain_bwd_segments or (16 if Kf in (16, 32) else min(Kf, 8))
-            while Kf % Ks:
-                Ks //= 2
-            seg_v *= Kf // Ks                       # every (Kf/Ks)-th forward joint: same padded length
-            _lib.call("icrl_chain_lstm_bwd_segmented", st, Ks, warm, seg_v, _p(Vn.valrnn.lstm.weight_hh_l0),
-                  _p(b["v_stash_g"]), _p(b["v_stash_c"]), _p(b["v_take"]), _p(dh_take), SB, _p(dgates), _p(self._seg_ws),
-                  _p(self.sync_state), L)
           elif K > 1:
             _lib.call("icrl_chain_lstm_bwd_sharded", st, K, Tv, _p(Vn.valrnn.lstm.weight_hh_l0), _p(b["v_stash_g"]),
                   _p(b["v_stash_c"]), _p(b["v_take"]), _p(dh_take), _p(dgates), _p(self.sync_state), L)
@@ -788,30 +737,25 @@ class A2CEngine:
                 return Tv, Tr, values, rewards
 
             # Attempts 0 .. _TC_ATTEMPTS-1 run the chains cut into pieces; a failed joint check lengthens the warm-up and
-            # tries again (tc engine) or goes straight to the serial kernels (simt engine); the last attempt is always
-            # the serial kernels, the guaranteed floor.  Gradients are overwritten, not accumulated, by a re-run.
+            # tries again; the last attempt is always the serial kernels, the guaranteed floor.  Gradients are
+            # overwritten, not accumulated, by a re-run.
             host, serial = None, False
             for attempt in range(self._TC_ATTEMPTS + 1):
                 serial = serial or attempt == self._TC_ATTEMPTS
                 Tv, Tr, values, rewards = run_chains(serial)
-                if self._seg is None and self._tc is None:
+                if self._tc is None:
                     break
                 self.segment_stats["segmented_steps"] += 1
                 if not check:
                     self._seg_unverified = True       # the caller owes a segments_verified() before trusting the steps
                     break
-                if self._tc is not None:
-                    ok, host = self._tc_ok()
-                    if not ok:
-                        host = None
-                        serial = self._tc_force_serial or attempt + 1 == self._TC_ATTEMPTS
-                        if serial:
-                            self.segment_stats["fallbacks"] += 1
-                else:
-                    ok = self._segments_ok()
-                    serial = True
+                ok, host = self._tc_ok()
                 if ok:
                     break
+                host = None
+                serial = self._tc_force_serial or attempt + 1 == self._TC_ATTEMPTS
+                if serial:
+                    self.segment_stats["fallbacks"] += 1
             stats = self._stat_err[:3].clone()
             if check and self._tc is None:
                 _lib.call("icrl_chain_check", self._stream, _p(self.sync_state))
@@ -890,40 +834,14 @@ class A2CEngine:
                                                      self.warm["v"], self.warm["r"], self.warm["b"]))
         return ok, host
 
-    def _segments_ok(self):
-        """Read (and re-arm) the warm-up checks of the segmented chain launches since the last call (synchronises).
-        False = some segment had not converged onto the single chain within chain_tol: the caller re-runs serially;
-        the warm-up is lengthened for the next steps, and after three failures in a row segments are switched off."""
-        e = self._seg_ws[:5].tolist()
-        self._seg_ws[:5].zero_()
-        self._seg_unverified = False
-        st = self.segment_stats
-        st["max_err"] = [max(a, b) if b == b else float("nan") for a, b in zip(st["max_err"], e)]
-        tol = self.chain_tol
-        ok = e[0] <= tol and e[1] <= tol and e[2] <= tol and e[3] <= tol * max(e[4], 1e-30)
-        if ok:
-            self._seg_strikes = 0
-            return True
-        import warnings
-        st["fallbacks"] += 1
-        self._seg_strikes += 1
-        self.chain_warmup *= 4
-        if self._seg_strikes >= 3:
-            self.chain_segments = 1
-        warnings.warn("chain segments did not converge onto the single chain within %g after the warm-up (|dh| %.3g, |dc| "
-                      "%.3g, reward |dh| %.3g, joint gate gradients %.3g of %.3g): re-running on the serial kernels; %s"
-                      % (tol, e[0], e[1], e[2], e[3], e[4],
-                         "segments are now off" if self.chain_segments == 1 else "warm-up is now %d" % self.chain_warmup))
-        return False
-
     @property
     def segment_layout(self):
         """(pieces, value-chain piece length, reward-chain piece length, warm-up) of the last step, or None when it ran on
         the serial kernels (chain too short, chain_segments = 1, or a failed warm-up check)."""
-        if self._tc is not None:
-            v, r = self._tc["v"], self._tc["r"]
-            return (r[0] if v is None else v[0], 0 if v is None else v[1], r[1], max(r[2], 0 if v is None else v[2]))
-        return self._seg
+        if self._tc is None:
+            return None
+        v, r = self._tc["v"], self._tc["r"]
+        return (r[0] if v is None else v[0], 0 if v is None else v[1], r[1], max(r[2], 0 if v is None else v[2]))
 
     @property
     def piece_layout(self):
@@ -936,9 +854,7 @@ class A2CEngine:
         if not self._seg_unverified:
             return True
         with torch.cuda.device(self.device):
-            if self._tc is not None:
-                return self._tc_ok()[0]
-            return self._segments_ok()
+            return self._tc_ok()[0]
 
     def get_rewards(self, features, captions):
         """GetRewards on whole captions from zero state (trainers.py:108-121): (B,1) tensor."""
@@ -953,12 +869,7 @@ class A2CEngine:
             serial = False
             for attempt in range(self._TC_ATTEMPTS + 1):
                 serial = serial or attempt == self._TC_ATTEMPTS
-                self._seg, self._tc = None, None
-                if not serial:
-                    if self._use_tc_chains():
-                        self._tc = self._pick_pieces(0, T)
-                    elif self.chain_segments > 1:
-                        self._seg = self._pick_segments(0, T)
+                self._tc = self._pick_pieces(0, T) if not serial and self._use_tc_chains() else None
                 n = self._padded(T, 1)
                 r_stream, r_pos = self._buf("r_stream", n, torch.int32), self._buf("r_pos", B, torch.int32)
                 _lib.call("icrl_build_stream", st, B, Lc, 1, 0, _p(tokcm), _p(r_stream), None, _p(r_pos), L)
@@ -975,15 +886,6 @@ class A2CEngine:
                     serial = attempt + 1 == self._TC_ATTEMPTS
                     if serial:
                         self.segment_stats["fallbacks"] += 1
-                elif self._seg is not None:
-                    Ks, _, seg_r, warm = self._seg
-                    r_stream[T:n].zero_()
-                    _lib.call("icrl_chains_fwd_fused_segmented", st, Ks, warm, None, 0, None, None, None, None, None,
-                              _p(r_stream), seg_r, _p(b["r_table"]), _p(R.rewrnn.gru.weight_hh_l0),
-                              _p(R.rewrnn.gru.bias_hh_l0[2 * H:]), _p(r_h), _p(self._seg_ws), _p(self.sync_state), L)
-                    if self._segments_ok():
-                        break
-                    serial = True
                 else:
                     _lib.call("icrl_chain_gru_fwd", st, _p(r_stream), T, _p(b["r_table"]), _p(R.rewrnn.gru.weight_hh_l0),
                               _p(R.rewrnn.gru.bias_hh_l0[2 * H:]), None, _p(r_h), None, _p(self.sync_state), None, L)

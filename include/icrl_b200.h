@@ -226,33 +226,6 @@ int icrl_chains_fwd_fused_sharded(void* stream, int shards, const int* v_stream,
 int icrl_chain_lstm_bwd_sharded(void* stream, int shards, int T, const float* W_hh, const float* stash_gates,
                                 const float* stash_c, const int* take, const float* dh_take, float* dgates,
                                 void* sync_state, int* launches);
-/* ---- chain segments (new; the reference has no equivalent).  ONE carried-state chain (the reference's semantics,
- *      models.py:133-140 / :225-231) cut into `segments` consecutive pieces of `seg` positions that advance in lockstep
- *      like the chain shards above (forward: 2, 4, 8, or 16 / 32 walked as 2 chunks of 8 / 16 per kernel step so that a
- *      chunk's exchange round trip is covered by the other chunk's arithmetic; backward: 2, 4, 8, or 16 = 8 per CTA group
- *      in one kernel step -- forward and backward may differ as long as segments * seg is the same).  Segment k >= 1 does not wait for the state of segment k-1: it starts from
- *      zero state `warm` positions early and discards those steps.  An LSTM / GRU whose gates forget contracts the
- *      difference of two states step by step, so after the warm-up the segment carries the state of the single chain
- *      up to float rounding -- which is CHECKED, not assumed: the state reached at the end of every warm-up is compared
- *      with the state the previous segment computes at the same position, and the backward recurrence (segment k starts
- *      `warm` positions late with zero dh, dc) compares the gate gradients at the joints.  The caller reads
- *      segment_ws[0..4] = {max |dh| value chain, max |dc| / max(1, |c|) value chain, max |dh| reward chain, max |d dgates| at the
- *      joints, max |dh_take|} (running maxima; zero them to re-arm) and, if they exceed its tolerance, re-runs the
- *      serial entry points on the same buffers (the array layout IS the single-chain layout).
- *      Sizes: seg = icrl_chain_segment_len(T, segments, warm) (0 = chain too short for this many segments: needs
- *      seg >= 2*warm); streams hold segments*seg + warm tokens (tail padded with token 0), take the same number of
- *      entries (tail -1), stash_h / stash_c segments*seg + warm + 1 rows, stash_gates / dgates segments*seg + warm rows.
- *      v_seg = 0 runs the reward chain only.  segment_ws: icrl_chain_segment_ws_floats() floats. */
-long long icrl_chain_segment_len(long long T, int segments, int warm);
-size_t icrl_chain_segment_ws_floats(void);
-int icrl_chains_fwd_fused_segmented(void* stream, int segments, int warm, const int* v_stream, int v_seg,
-                                    const float* v_table, const float* v_W_hh, float* v_stash_h, float* v_stash_c,
-                                    float* v_stash_gates, const int* r_stream, int r_seg, const float* r_table,
-                                    const float* r_W_hh, const float* r_b_hn, float* r_stash_h, float* segment_ws,
-                                    void* sync_state, int* launches);
-int icrl_chain_lstm_bwd_segmented(void* stream, int segments, int warm, int seg, const float* W_hh,
-                                  const float* stash_gates, const float* stash_c, const int* take, const float* dh_take,
-                                  long long take_rows, float* dgates, float* segment_ws, void* sync_state, int* launches);
 /* ---- chain pieces on tcgen05 (chain_tc.cu; the default engine).  The same ONE carried-state chain
  *      (models.py:130-135 value LSTM, :223-228 reward GRU; backward of trainers.py:479) advanced as `pieces` lockstep
  *      pieces, 128 per cluster of 8 CTAs: one kernel step is the contraction H_prev [pieces x 512] . W_hh^T on the
@@ -260,10 +233,10 @@ int icrl_chain_lstm_bwd_segmented(void* stream, int segments, int warm, int seg,
  *      update in its epilogue.  Piece k covers positions [k*seg, (k+1)*seg + warm) of the stream; pieces k >= 1 start
  *      from zero state and discard their first `warm` positions; the backward recurrence is mirrored (piece k walks
  *      (k+1)*seg + warm - 1 down to k*seg; all but the last start with dh = dc = 0 and discard `warm` steps).
- *      Array sizes are those of the chain segments above with segments = pieces (streams / take pieces*seg + warm
- *      entries padded with token 0 / -1; stash_h, stash_c one row more; row 0 is zeroed by the call); any pieces >= 2,
- *      seg >= 1 is accepted.  CHECKED, not assumed: after every launch err[] holds running maxima (zero to re-arm) of
- *      the state differences at the joints -- forward err[0] = max |dh| and err[1] = max |dc| / max(1, |c|) at the end
+ *      Array sizes: streams / take pieces*seg + warm entries (the tail past the chain padded with token 0 / -1),
+ *      stash_gates the same number of rows, stash_h / stash_c one row more (row 0 is zeroed by the call); any
+ *      pieces >= 2, seg >= 1 is accepted.  CHECKED, not assumed: after every launch err[] holds running maxima (zero
+ *      to re-arm) of the state differences at the joints -- forward err[0] = max |dh| and err[1] = max |dc| / max(1, |c|) at the end
  *      of the warm-up, err[2], err[3] the same half-way through it (the slope gives the contraction rate the caller
  *      sizes the next warm-up with); backward err[0..3] = |d(dh)|, |d(dc)| at the joints (end / half-way) relative to
  *      err[4] = max |dh_take|, err[5] = 1 when a scaled gate gradient left the fp16 range of the exchange.
@@ -309,7 +282,7 @@ int icrl_chain_tc_bwd_max_pieces(void);
 /* Experiment knob: 1 = the forward stash of the live positions leaves through TMA tensor stores, 0 (default) = per-thread
  * vector stores (measured equal: the store phase is L2-bound, not issue-bound). */
 int icrl_chain_tc_set_tma_store(int on);
-/* Debug aid: when buf != NULL (16 device int64), CTA 0 / thread 0 of the sharded / segmented chain kernels accumulates its
+/* Debug aid: when buf != NULL (16 device int64), CTA 0 / thread 0 of the sharded chain kernels accumulates its
  * cycles per phase: [0..3] value LSTM forward {exchange wait, GEMV + reduce, pointwise + publish, T}, [4..7] reward GRU
  * forward, [8..14] backward {coefficients + requests, poll wait, gate gradients + stores, barrier, contraction + reduce,
  * barrier + publish, T} (the backward runs a separately compiled, instrumented build of the kernel). */

@@ -24,9 +24,8 @@ out = {}
 e1 = A2CEngine(A, R, chain_segments=1); out["serial"] = grads(e1)
 ea = A2CEngine(A, R, chain_warmup=eng.warm["v"], chain_adapt=False); ea.warm = dict(eng.warm); out["tc_adapted"] = grads(ea)
 eb = A2CEngine(A, R, chain_warmup=1024, chain_adapt=False); out["tc_warm1024"] = grads(eb)
-ec = A2CEngine(A, R, chain_engine="simt", chain_segments=32, chain_warmup=1024); out["simt32_warm1024"] = grads(ec)
 ed = A2CEngine(A, R, chain_pieces=128, chain_warmup=1024, chain_adapt=False); out["tc_128pieces_warm1024"] = grads(ed)
-print("layouts", ea.piece_layout, eb.piece_layout, ec.segment_layout, ed.piece_layout)
+print("layouts", ea.piece_layout, eb.piece_layout, ed.piece_layout)
 print("tc errs adapted", ["%.1e" % x for x in ea.segment_stats["tc_max_err"][:14]])
 print("tc errs 1024   ", ["%.1e" % x for x in eb.segment_stats["tc_max_err"][:14]])
 names = list(out)

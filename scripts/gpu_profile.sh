@@ -1,14 +1,9 @@
 #!/bin/bash
-# ncu evidence for profiles/: launch list of the default bench workload (B=4096), then one full capture of the segmented
-# chain kernels (B=1024).  Each ncu pass runs only after the same command exited 0 without ncu.
+# ncu evidence for profiles/: launch list of the default bench workload (B=4096).  The ncu pass runs only after the same
+# command exited 0 without ncu.
 mkdir -p gpurun_out
 CMD="python bench.py --steps 1 --warmup 3 --no-e2e --no-cpu-baseline --no-serial-leg"
 $CMD > gpurun_out/prof_plain.log 2>&1 &&
 ncu --metrics gpu__time_duration.sum --clock-control none -c 2000 --csv --log-file gpurun_out/launches.csv $CMD > gpurun_out/ncu_launches.log 2>&1
 echo "launch list exit $?"
-CMD1="python bench.py --batch 1024 --steps 1 --warmup 3 --no-e2e --no-cpu-baseline --no-serial-leg"
-$CMD1 > gpurun_out/prof_plain2.log 2>&1 &&
-ncu --set full --clock-control none --import-source on -k regex:batched -s 6 -c 2 -o gpurun_out/prof_chain_segments $CMD1 > gpurun_out/ncu_chain.log 2>&1
-echo "chain capture exit $?"
-ncu -i gpurun_out/prof_chain_segments.ncu-rep --page raw --csv > gpurun_out/prof_chain_segments_raw.csv 2> /dev/null
 ls -la gpurun_out | tail -8

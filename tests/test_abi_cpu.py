@@ -129,28 +129,6 @@ def test_checkpoint_helpers_roundtrip(tmp_path):
     assert not B.policy_network.training and not B.value_network.training
 
 
-def test_chain_segment_geometry(lib):
-    """icrl_chain_segment_len: K pieces of `seg` positions plus one warm-up cover the chain, every piece is at least
-    two warm-ups long, and chains too short for that are refused (0) so that the engine uses fewer pieces or the
-    serial kernels.  Forward and backward may cut the same chain into different numbers of pieces as long as
-    pieces * seg agrees (engine: backward = every (Kf / Kb)-th forward joint)."""
-    seglen = lambda T, K, w: int(lib.call("icrl_chain_segment_len", T, K, w))
-    for T in (600, 1152, 48640, 97280, 778240):
-        for K in (2, 4, 8, 16, 32):
-            for warm in (32, 256, 512):
-                seg = seglen(T, K, warm)
-                if seg == 0:
-                    assert (T - warm + K - 1) // K < 2 * warm or T <= warm
-                    continue
-                assert seg >= 2 * warm
-                assert K * seg + warm >= T > (K * seg + warm) - K          # padding below one position per piece
-                if K >= 16:
-                    Kb = 16
-                    assert Kb * (seg * (K // Kb)) == K * seg
-    assert seglen(100, 1, 16) == 0 and seglen(16, 2, 16) == 0 and seglen(1000, 2, 0) == 0
-    assert int(lib.call("icrl_chain_segment_ws_floats")) >= 8 + 2 * 32 * 2 * 512
-
-
 def test_bench_reference_arm_json_contract():
     """`bench.py --impl reference` (the CPU arm the driver runs beside the GPU arm) prints ONE JSON line with the keys of
     the bench contract; it times oracle/ref_port on the host cores and needs no GPU."""

@@ -700,14 +700,14 @@ def test_config4_full_size_properties():
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# chain pieces: the single carried-state chain advanced as lockstep pieces with a discarded, verified warm-up.
-# Default engine = chain_tc.cu (hundreds of pieces on tcgen05); chain_engine="simt" = the CUDA-core kernels of chain.cu.
+# chain pieces: the single carried-state chain advanced as lockstep pieces on tcgen05 (chain_tc.cu) with a discarded,
+# verified warm-up.
 
-def _seg_engines(seed, segments, warm, tol=1e-5, engine="simt", **kw):
+def _seg_engines(seed, segments, warm, tol=1e-5, **kw):
     from icrl_b200.engine import A2CEngine
     A, R, w = make_nets(seed)
     return (A2CEngine(A, R, chain_segments=1),
-            A2CEngine(A, R, chain_segments=segments, chain_warmup=warm, chain_tol=tol, chain_engine=engine, **kw), A)
+            A2CEngine(A, R, chain_segments=segments, chain_warmup=warm, chain_tol=tol, **kw), A)
 
 
 @pytest.mark.parametrize("name", ["a2c_b32_l9", "curr_b24_l20_lv6", "a2c_b256_l20"])
@@ -734,7 +734,7 @@ def test_chain_pieces_equal_the_serial_chain(pieces, B, L, level, warm):
     within 2e-5 of the bucket's largest entry -- for piece counts that do not fill a cluster (7, 2), that straddle
     clusters (130, 300) and for the automatic layout."""
     seed = 131 + (pieces or 0)
-    e1, ek, A = _seg_engines(seed, 32, warm, engine="tc", chain_pieces=pieces)
+    e1, ek, A = _seg_engines(seed, 32, warm, chain_pieces=pieces)
     f, c = synth.make_inputs(seed, B, L)
     S = (L - 1) if level is None else level
     u = synth.make_uniforms(seed, S, B)
@@ -760,7 +760,7 @@ def test_chain_pieces_short_warmup_is_caught_and_rerun():
     re-run with a longer warm-up (or, after three attempts, on the serial kernels) before anything leaves the engine,
     a warning is raised, and the step comes out within the serial kernels' tolerances."""
     seed, B, L = 141, 64, 10
-    e1, ek, A = _seg_engines(seed, 32, 4, engine="tc")
+    e1, ek, A = _seg_engines(seed, 32, 4)
     f, c = synth.make_inputs(seed, B, L)
     u = synth.make_uniforms(seed, L - 1, B)
     r1 = e1.step(f, c, uniforms=u)
@@ -776,6 +776,24 @@ def test_chain_pieces_short_warmup_is_caught_and_rerun():
     with pytest.warns(UserWarning):
         assert ek.segments_verified() is False
     assert ek.segments_verified() is True
+
+
+def test_chain_pieces_fall_back_to_the_serial_kernels():
+    """A step whose joint checks fail on every tcgen05 attempt (chain_tol far below the float rounding of the joints)
+    ends on the serial kernels: one fall-back is counted, and values and rewards are those of the serial engine bit for
+    bit."""
+    seed, B, L = 141, 64, 10
+    e1, ek, A = _seg_engines(seed, 32, 64, tol=1e-12)
+    f, c = synth.make_inputs(seed, B, L)
+    u = synth.make_uniforms(seed, L - 1, B)
+    r1 = e1.step(f, c, uniforms=u)
+    v1, w1, g1 = r1["values"].clone(), r1["rewards"].clone(), e1.flat_grad.clone()
+    with pytest.warns(UserWarning, match="chain segments did not converge"):
+        rk = ek.step(f, c, uniforms=u)
+    st = ek.segment_stats
+    assert st["fallbacks"] == 1 and ek.piece_layout is None, st
+    assert torch.equal(rk["values"], v1) and torch.equal(rk["rewards"], w1)
+    assert float((ek.flat_grad - g1).abs().max() / g1.abs().max()) <= 1e-6      # atomics in the table scatter reorder sums
 
 
 def test_get_rewards_pieces_equal_the_serial_chain():
@@ -895,9 +913,9 @@ def test_pieces_survive_200_adam_steps():
     assert ev <= TOL * vscale, (ev, vscale)
     assert float((rk["rewards"] - r1["rewards"]).abs().max()) <= TOL
     # Gradients: by now the critic has learned the mean of its target, so the value-side gradients are sums that cancel
-    # (linear2.bias = sum of dL/dvalues ~ 0) and amplify any difference in the values.  The CUDA-core segment kernels
-    # agree with the serial chain to 3e-7 here, the tensor-core kernels (truncating accumulation, compensated in the mean:
-    # chain_tc.cu g_tc_bias) to ~1e-4; the policy-side gradients stay at 2e-6.  Tolerance for this regime: 3e-4 of max.
+    # (linear2.bias = sum of dL/dvalues ~ 0) and amplify any difference in the values.  The tensor-core kernels
+    # (truncating accumulation, compensated in the mean: chain_tc.cu g_tc_bias) agree with the serial chain to ~1e-4
+    # here; the policy-side gradients stay at 2e-6.  Tolerance for this regime: 3e-4 of max.
     eg = float((gk - e1.flat_grad).abs().max() / e1.flat_grad.abs().max())
     _record("pieces_200_steps", grad_rel=eg)
     assert eg <= 3e-4, eg
@@ -934,40 +952,6 @@ def test_slow_forgetting_weights_degrade_gracefully():
     for r in (rk, rk2):
         assert float((r["values"] - v1).abs().max()) <= TOL and float((r["rewards"] - w1).abs().max()) <= TOL
     assert float((ek.flat_grad - g1).abs().max() / g1.abs().max()) <= GTOL
-
-
-# ---- legacy CUDA-core segment kernels (chain_engine="simt")
-
-@pytest.mark.parametrize("segments,B,L,level", [(8, 64, 10, None), (16, 96, 14, 5), (32, 256, 20, 7)])
-def test_chain_segments_simt_equal_the_serial_chain(segments, B, L, level):
-    seed = 131 + segments
-    e1, ek, A = _seg_engines(seed, segments, 160)
-    f, c = synth.make_inputs(seed, B, L)
-    S = (L - 1) if level is None else level
-    u = synth.make_uniforms(seed, S, B)
-    r1 = e1.step(f, c, uniforms=u, level=level)
-    v1, w1, g1 = r1["values"].clone(), r1["rewards"].clone(), e1.flat_grad.clone()
-    rk = ek.step(f, c, uniforms=u, level=level)
-    assert ek.segment_layout is not None and ek.segment_layout[0] == segments, ek.segment_layout
-    assert ek.segment_stats["fallbacks"] == 0, ek.segment_stats
-    assert torch.equal(rk["tokens"], r1["tokens"])
-    ev, er = float((rk["values"] - v1).abs().max()), float((rk["rewards"] - w1).abs().max())
-    eg = float((ek.flat_grad - g1).abs().max() / g1.abs().max())
-    assert ev <= TOL and er <= TOL and eg <= GTOL, (ev, er, eg)
-
-
-def test_chain_segments_simt_fall_back_to_the_serial_kernels():
-    seed, B, L = 141, 64, 10
-    e1, ek, A = _seg_engines(seed, 8, 4)
-    f, c = synth.make_inputs(seed, B, L)
-    u = synth.make_uniforms(seed, L - 1, B)
-    r1 = e1.step(f, c, uniforms=u)
-    v1, w1, g1 = r1["values"].clone(), r1["rewards"].clone(), e1.flat_grad.clone()
-    with pytest.warns(UserWarning, match="chain segments did not converge"):
-        rk = ek.step(f, c, uniforms=u)
-    assert ek.segment_stats["fallbacks"] == 1 and ek.chain_warmup == 16
-    assert torch.equal(rk["values"], v1) and torch.equal(rk["rewards"], w1)
-    assert float((ek.flat_grad - g1).abs().max() / g1.abs().max()) <= 1e-6      # atomics in the table scatter reorder sums
 
 
 @pytest.mark.parametrize("switch", ["tma_store", "separate_forward_launches", "no_backward_overlap", "simt_policy_bptt"])
