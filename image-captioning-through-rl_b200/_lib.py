@@ -55,6 +55,10 @@ SIGNATURES = {
     "icrl_chain_tc_fwd": [P, I, I, L, I] + [P] * 10 + [LP],
     "icrl_chains_tc_fwd_fused": [P, I, L, I] + [P] * 9 + [I, L, I] + [P] * 8 + [LP],
     "icrl_chain_tc_lstm_bwd": [P, I, L, I, P, P, P, P, P, L, P, L, P, P, P, P, LP],
+    "icrl_chain_tc_lstm_fwd_from": [P, I, L, I] + [P] * 11 + [LP],
+    "icrl_lookahead_stream": [P, I, I, I, I, P, P, P, P, LP],
+    "icrl_lookahead_policy_step": [P, I, I, I, I] + [P] * 17 + [LP],
+    "icrl_lookahead_score": [P, I, I, I, P, P, P, P, P, LP],
     "icrl_chain_tc_set_profile": [P],
     "icrl_chain_tc_set_bias": [F, F],
     "icrl_chain_tc_bwd_max_pieces": [],

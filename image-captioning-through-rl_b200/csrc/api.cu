@@ -461,6 +461,67 @@ int icrl_chain_tc_lstm_bwd(void* stream, int pieces, long long seg, int warm, co
   return ICRL_OK;
 }
 
+int icrl_chain_tc_lstm_fwd_from(void* stream, int pieces, long long seg, int warm, const int* tok_stream, const float* table,
+                                const void* packed, const float* h0, const float* c0, float* stash_h, float* stash_c,
+                                float* stash_gates, void* ws, float* cp_state, float* err, int* launches) {
+  TRY(icrl_chain_tc_lstm_fwd_from_impl(S_(stream), pieces, seg, warm, tok_stream, table, packed, h0, c0, stash_h, stash_c,
+                                       stash_gates, ws, cp_state, err));
+  bump(launches, (h0 || c0) ? 3 : 2);      // the state seed, the persistent cluster kernel, the joint check
+  return ICRL_OK;
+}
+
+// ---- value-guided look-ahead decoder (trainers.py:73-105)
+int icrl_lookahead_stream(void* stream, int B, int n, int K, int k, const int* cand_tok, const int* words, int* tok_stream,
+                          int* take_pos, int* launches) {
+  ICRL_REQUIRE(B > 0 && n >= 1 && K >= 1 && k >= 1, "bad look-ahead shape");
+  ICRL_REQUIRE((long long)K * k * (n + 1) * B < (1ll << 31), "token stream longer than 2^31");
+  TRY(icrl_lookahead_stream_impl(S_(stream), B, n, K, k, cand_tok, words, tok_stream, take_pos));
+  bump(launches, 1);
+  return ICRL_OK;
+}
+
+int icrl_lookahead_policy_step(void* stream, int R, int V, int k, int first, const float* features, const float* W_cnn,
+                               const float* b_cnn, const float* table, const int* parent, const float* h_in, const float* c_in,
+                               const int* tok, const void* whh_parts, const void* wv_parts, const float* b_v, float* h_out,
+                               float* c_out, float* logits, float* top_val, int* top_idx, void* ws, int* launches) {
+  ICRL_REQUIRE(R > 0 && V > 0 && k >= 1 && k <= 16 && k <= V, "bad beam-step shape (1 <= k <= min(16, V))");
+  ICRL_REQUIRE(first ? features != nullptr : (parent && h_in && c_in), "the first step needs the features, later ones the parents");
+  cudaStream_t st = S_(stream);
+  const size_t RH = (size_t)R * H;
+  float* h_prev = reinterpret_cast<float*>(ws);
+  float* c_prev = h_prev + RH;
+  float* gpre = c_prev + RH;
+  float* gates = gpre + 4 * RH;
+  void* h_parts = gates + 4 * RH;
+  float* lg = logits ? logits : reinterpret_cast<float*>(reinterpret_cast<char*>(h_parts) + 3 * RH * 2);
+  if (first) {
+    // h0 = cnn2linear(features), c0 = 0 (models.py:75-78), as icrl_policy_rollout_fwd_tc starts
+    TRY(icrl_gemm_f32_impl(st, 0, 1, R, H, H, features, H, W_cnn, H, h_prev, H, b_cnn, 0.f, nullptr, 0, launches));
+    ICRL_CUDA(cudaMemsetAsync(c_prev, 0, RH * sizeof(float), st));
+  } else {
+    TRY(icrl_gather_rows_impl(st, R, h_in, parent, 0, h_prev));
+    TRY(icrl_gather_rows_impl(st, R, c_in, parent, 0, c_prev));
+    bump(launches, 2);
+  }
+  // one decode step of icrl_policy_rollout_fwd_tc for R rows, then the top-k of every row's logits
+  TRY(icrl_split_bf16x3_impl(st, (long long)RH, h_prev, h_parts));
+  TRY(icrl_gemm_bf16x3_impl(st, R, 4 * H, H, h_parts, whh_parts, gpre, 4 * H, nullptr));
+  TRY(icrl_lstm_pointwise_fwd(st, R, gpre, table, tok, c_prev, gates, c_out, h_out));
+  TRY(icrl_split_bf16x3_impl(st, (long long)RH, h_out, h_parts));
+  TRY(icrl_gemm_bf16x3_impl(st, R, V, H, h_parts, wv_parts, lg, V, b_v));
+  TRY(icrl_topk_rows(st, R, V, k, lg, top_val, top_idx));
+  bump(launches, 6);
+  return ICRL_OK;
+}
+
+int icrl_lookahead_score(void* stream, int B, int K, int k, const float* parent_score, const float* values, const float* top_val,
+                         float* child_score, float* means, int* launches) {
+  ICRL_REQUIRE(B > 0 && K >= 1 && k >= 1, "bad look-ahead shape");
+  TRY(icrl_lookahead_score_impl(S_(stream), B, K, k, parent_score, values, top_val, child_score, means));
+  bump(launches, 1);
+  return ICRL_OK;
+}
+
 int icrl_chain_set_profile(void* buf) { icrl_chain_set_profile_impl(reinterpret_cast<long long*>(buf)); return ICRL_OK; }
 
 size_t icrl_chain_sync_bytes(void) { return icrl_chain_sync_bytes_impl(); }

@@ -1204,6 +1204,46 @@ int icrl_chain_tc_fwd_impl(cudaStream_t st, int kind, int P, long long seg, int 
   return ICRL_OK;
 }
 
+namespace {
+// Piece 0 of an LSTM launch starts from (h0, c0) instead of zeros: what fwd_setup zeroed for it is overwritten with the
+// state itself -- the fp16 hi/lo' split of h0 in row 0 of hparts buffer 0 (the A operand of kernel step 0, split exactly as
+// the epilogue splits h for the next step), c0 in row 0 of the carried state, and stash rows 0.  A null pointer is zeros.
+__global__ void chain_tc_seed_kernel(int Ppad, const float* __restrict__ h0, const float* __restrict__ c0, __half* hparts,
+                                     float* state, float* stash_h, float* stash_c) {
+  const int u = 4 * threadIdx.x;
+  const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+  const float4 h4 = h0 ? *reinterpret_cast<const float4*>(h0 + u) : z;
+  const float4 c4 = c0 ? *reinterpret_cast<const float4*>(c0 + u) : z;
+  uint2 hi, lo;
+  split4_f16(h4, hi, lo);
+  *reinterpret_cast<uint2*>(hparts + u) = hi;
+  *reinterpret_cast<uint2*>(hparts + (size_t)Ppad * H + u) = lo;
+  *reinterpret_cast<float4*>(state + u) = c4;
+  *reinterpret_cast<float4*>(stash_h + u) = h4;
+  *reinterpret_cast<float4*>(stash_c + u) = c4;
+}
+}  // namespace
+
+int icrl_chain_tc_lstm_fwd_from_impl(cudaStream_t st, int P, long long seg, int warm, const int* stream, const float* table,
+                                     const void* packed, const float* h0, const float* c0, float* stash_h, float* stash_c,
+                                     float* stash_g, void* ws, float* cp_state, float* err) {
+  ICRL_REQUIRE(((reinterpret_cast<uintptr_t>(h0) | reinterpret_cast<uintptr_t>(c0)) & 15) == 0, "h0 / c0 must be 16-byte aligned");
+  FwdArgs a;
+  FwdMaps m;
+  int rc = fwd_setup(st, 0, P, seg, warm, stream, table, packed, nullptr, stash_h, stash_c, stash_g, ws, cp_state, err, &a, &m);
+  if (rc) return rc;
+  if (h0 || c0) {
+    chain_tc_seed_kernel<<<1, H / 4, 0, st>>>(a.Ppad, h0, c0, a.hparts, a.state, stash_h, stash_c);
+    ICRL_LAUNCH_CHECK();
+  }
+  ICRL_CUDA(cudaFuncSetAttribute(chain_tc_fwd_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdCfg<4>::SMEM));
+  chain_tc_fwd_kernel<4><<<dim3(CL * (a.Ppad / BM)), dim3(THREADS), FwdCfg<4>::SMEM, st>>>(m, a);
+  ICRL_LAUNCH_CHECK();
+  chain_tc_check_fwd_kernel<<<dim3(P - 1, 2), H, 0, st>>>(P, seg, warm, a.cp_half, cp_state, stash_h, stash_c, err);
+  ICRL_LAUNCH_CHECK();
+  return ICRL_OK;
+}
+
 // Both forward chains in one launch (chains_tc_fwd_fused_kernel): value LSTM with Pv pieces, reward GRU with Pr pieces.
 int icrl_chains_tc_fwd_fused_impl(cudaStream_t st, int Pv, long long seg_v, int warm_v, const int* v_stream,
                                   const float* v_table, const void* v_packed, float* v_stash_h, float* v_stash_c,

@@ -180,6 +180,49 @@ __global__ void build_stream_sharded_kernel(int B, int Bs, int p0, int S, int ex
   }
 }
 
+// Value chain of one beam step of the look-ahead decoder (trainers.py:87-92): for candidate c and word i (block
+// s = c*k + i, the reference's call order) the n prefix columns cand_tok[c] ([K][n][B]) and the word column
+// words[c][b][i] ([K][B][k]), rows in order.  take_pos[s*B + b] = stream position of row b of the word column.
+__global__ void lookahead_stream_kernel(int B, int n, int k, const int* __restrict__ cand_tok, const int* __restrict__ words,
+                                        int* __restrict__ stream, int* __restrict__ take_pos) {
+  const int s = blockIdx.y, c = s / k, i = s % k;
+  const long long len = (long long)(n + 1) * B;
+  const long long start = (long long)s * len;
+  for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < len; p += (long long)gridDim.x * blockDim.x) {
+    const int col = (int)(p / B), b = (int)(p % B);
+    if (col < n) {
+      stream[start + p] = cand_tok[((long long)c * n + col) * B + b];
+    } else {
+      stream[start + p] = words[((long long)c * B + b) * k + i];
+      take_pos[(long long)s * B + b] = (int)(start + p);
+    }
+  }
+}
+
+// One block per child s = c*k + i: child[s][b] = parent[c][b] - (0.6 V + 0.4 log(top)) in the reference's operation
+// order (trainers.py:92, fp32, every product and sum rounded on its own), means[s] = the batch mean of child[s].
+__global__ void lookahead_score_kernel(int B, int K, int k, const float* __restrict__ parent, const float* __restrict__ values,
+                                       const float* __restrict__ top_val, float* __restrict__ child, float* __restrict__ means) {
+  const int s = blockIdx.x, c = s / k, i = s % k, S = K * k;
+  __shared__ double red[32];
+  double acc = 0.0;
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    const float v = values[(size_t)b * S + s];
+    const float t = top_val[((size_t)c * B + b) * k + i];
+    const float x = __fsub_rn(parent[(size_t)c * B + b], __fadd_rn(__fmul_rn(0.6f, v), __fmul_rn(0.4f, logf(t))));
+    child[(size_t)s * B + b] = x;
+    acc += (double)x;
+  }
+  acc = warp_sum_d(acc);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    acc = threadIdx.x < (blockDim.x >> 5) ? red[threadIdx.x] : 0.0;
+    acc = warp_sum_d(acc);
+    if (threadIdx.x == 0) means[s] = (float)(acc / B);
+  }
+}
+
 // dst[r] = src[idx[r] + row_offset]  (rows of H floats)
 __global__ void gather_rows_kernel(long long R, const float* __restrict__ src, const int* __restrict__ idx,
                                    long long row_offset, float* __restrict__ dst) {
@@ -280,6 +323,21 @@ int icrl_build_stream_sharded_impl(cudaStream_t st, int B, int p0, int S, int ex
   const long long T = (long long)Bs * ((long long)S * (p0 + extra) + (long long)S * (S - 1) / 2);
   dim3 grid(icrl_cdiv((long long)(p0 + S + extra) * Bs, 256 * 4), S, shards);
   build_stream_sharded_kernel<<<grid, 256, 0, st>>>(B, Bs, p0, S, extra, T + 1, tokcm, stream, take, take_pos);
+  ICRL_LAUNCH_CHECK();
+  return ICRL_OK;
+}
+
+int icrl_lookahead_stream_impl(cudaStream_t st, int B, int n, int K, int k, const int* cand_tok, const int* words, int* stream,
+                               int* take_pos) {
+  dim3 grid(icrl_cdiv((long long)(n + 1) * B, 256 * 4), K * k);
+  lookahead_stream_kernel<<<grid, 256, 0, st>>>(B, n, k, cand_tok, words, stream, take_pos);
+  ICRL_LAUNCH_CHECK();
+  return ICRL_OK;
+}
+
+int icrl_lookahead_score_impl(cudaStream_t st, int B, int K, int k, const float* parent, const float* values, const float* top_val,
+                              float* child, float* means) {
+  lookahead_score_kernel<<<K * k, 256, 0, st>>>(B, K, k, parent, values, top_val, child, means);
   ICRL_LAUNCH_CHECK();
   return ICRL_OK;
 }

@@ -13,6 +13,7 @@ int icrl_softmax_sample(cudaStream_t st, int B, int V, const float* logits, int 
                         const long long* forced, int* tok_next, long long* tokens_out, float* logp_out, int S, int s, float* probs_out);
 int icrl_softmax_bwd(cudaStream_t st, int B, int S, int V, float* z, int ldl, const long long* tokens_out,
                      const float* dlogp);
+int icrl_topk_rows(cudaStream_t st, int R, int V, int k, const float* x, float* top_val, int* top_idx);
 int icrl_scatter_add_rows(cudaStream_t st, long long R, int C, const float* src, const int* idx, float* dst);
 int icrl_scatter_add_stream(cudaStream_t st, int B, int p0, int S, int extra, int C, const float* src, const int* tok_stream,
                             float* dst, unsigned* colmax);
@@ -36,6 +37,10 @@ int icrl_build_stream_impl(cudaStream_t st, int B, int p0, int S, int extra, con
                            int* take_pos);
 int icrl_gather_rows_impl(cudaStream_t st, long long R, const float* src, const int* idx, long long row_offset,
                           float* dst);
+int icrl_lookahead_stream_impl(cudaStream_t st, int B, int n, int K, int k, const int* cand_tok, const int* words, int* stream,
+                               int* take_pos);
+int icrl_lookahead_score_impl(cudaStream_t st, int B, int K, int k, const float* parent, const float* values, const float* top_val,
+                              float* child, float* means);
 int icrl_add_gate_bias_impl(cudaStream_t st, int V, int G, int fold, const float* b_ih, const float* b_hh,
                             float* table);
 
@@ -102,6 +107,9 @@ size_t icrl_chain_tc_cp_floats_impl(int pieces);
 int icrl_chain_tc_fwd_impl(cudaStream_t st, int kind, int P, long long seg, int warm, const int* stream,
                            const float* table, const void* packed, const float* b_hn, float* stash_h, float* stash_c,
                            float* stash_g, void* ws, float* cp_state, float* err);
+int icrl_chain_tc_lstm_fwd_from_impl(cudaStream_t st, int P, long long seg, int warm, const int* stream, const float* table,
+                                     const void* packed, const float* h0, const float* c0, float* stash_h, float* stash_c,
+                                     float* stash_g, void* ws, float* cp_state, float* err);
 int icrl_chain_tc_lstm_bwd_impl(cudaStream_t st, int P, long long seg, int warm, const void* packed,
                                 const float* stash_g, const float* stash_c, const int* take, const float* dh_take,
                                 long long take_rows, void* dg_pair, long long pair_rows, float* dg_inv_scale, void* ws,

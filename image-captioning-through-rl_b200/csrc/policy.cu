@@ -246,7 +246,52 @@ __global__ void wcolsum_stage2_kernel(int C, int chunks, const float* __restrict
   out[c] = acc;
 }
 
+// Order of the row top-k: larger value first, equal values by lower index; a NaN ranks above every number (torch.topk).
+__device__ __forceinline__ bool topk_before(float va, int ia, float vb, int ib) {
+  const bool na = va != va, nb = vb != vb;
+  if (na || nb) return na && (!nb || ia < ib);
+  return va > vb || (va == vb && ia < ib);
+}
+
+// One warp per row: k rounds, each the warp-wide first element (in topk_before order) that ranks after the previous pick.
+__global__ void topk_rows_kernel(int R, int V, int k, const float* __restrict__ x, float* __restrict__ top_val,
+                                 int* __restrict__ top_idx) {
+  const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (row >= R) return;
+  const float* xr = x + (size_t)row * V;
+  float pv = 0.f;
+  int pi = -1;
+  for (int r = 0; r < k; ++r) {
+    float bv = 0.f;
+    int bi = -1;
+    for (int j = lane; j < V; j += 32) {
+      const float v = xr[j];
+      if (pi >= 0 && !topk_before(pv, pi, v, j)) continue;
+      if (bi < 0 || topk_before(v, j, bv, bi)) { bv = v; bi = j; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+      const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+      if (oi >= 0 && (bi < 0 || topk_before(ov, oi, bv, bi))) { bv = ov; bi = oi; }
+    }
+    if (lane == 0) {
+      top_val[(size_t)row * k + r] = bv;
+      top_idx[(size_t)row * k + r] = bi;
+    }
+    pv = bv;
+    pi = bi;
+  }
+}
+
 }  // namespace
+
+int icrl_topk_rows(cudaStream_t st, int R, int V, int k, const float* x, float* top_val, int* top_idx) {
+  ICRL_REQUIRE(R > 0 && k >= 1 && k <= 16 && k <= V, "row top-k needs 1 <= k <= min(16, V)");
+  topk_rows_kernel<<<icrl_cdiv((long long)R * 32, 256), 256, 0, st>>>(R, V, k, x, top_val, top_idx);
+  ICRL_LAUNCH_CHECK();
+  return ICRL_OK;
+}
 
 int icrl_lstm_pointwise_fwd(cudaStream_t st, int B, const float* gpre, const float* table, const int* tok,
                             const float* c_prev, float* gates_act, float* c_out, float* h_out) {

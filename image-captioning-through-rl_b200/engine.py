@@ -822,16 +822,16 @@ class A2CEngine:
             ok_v = self._adapt_warm("v", nanmax(e[2:4]), nanmax(e[0:2]))
             if e[12] != 0.0 or any(x != 0.0 for x in e[8:12]):        # the backward recurrence ran in this step
                 ok_b = self._adapt_warm("b", nanmax(e[10:12]), nanmax(e[8:10]))
-        ok_r = self._adapt_warm("r", e[6], e[4])
+        ok_r = self._tc.get("r") is None or self._adapt_warm("r", e[6], e[4])
         ok = ok_v and ok_b and ok_r and not self._tc_force_serial
         if not ok:
             import warnings
             st["reruns"] += 1
             warnings.warn("chain segments did not converge onto the single chain within %g after the warm-up (value chain "
                           "forward |dh| %.3g |dc| %.3g, backward %.3g %.3g; reward chain |dh| %.3g%s): re-running with "
-                          "warm-ups %d / %d / %d" % (self.chain_tol, e[0], e[1], e[8], e[9], e[4],
-                                                     "; gate gradients overflowed the fp16 exchange" if self._tc_force_serial else "",
-                                                     self.warm["v"], self.warm["r"], self.warm["b"]))
+                          "warm-ups %s" % (self.chain_tol, e[0], e[1], e[8], e[9], e[4],
+                                           "; gate gradients overflowed the fp16 exchange" if self._tc_force_serial else "",
+                                           " / ".join("%d" % w for w in self.warm.values())))
         return ok, host
 
     @property
@@ -911,3 +911,161 @@ class A2CEngine:
             last = self._bufs["p_logits"][(steps - 1) * B * self.V: steps * B * self.V].view(B, self.V).clone()
             out = torch.cat((torch.from_numpy(first).to(self.device), tokens), dim=1)
         return out, last
+
+
+class LookAheadEngine(A2CEngine):
+    """The value-guided look-ahead decoder of the reference's evaluation path (GenerateCaptionsWithActorCriticLookAhead,
+    trainers.py:73-105) on the fused engine; no reward network.
+
+    Per beam step the K candidates' policy states advance by one cell on the tensor-core GEMMs (icrl_lookahead_policy_step:
+    the reference re-runs every full prefix), and the K*k value calls of the step -- known before any value is needed,
+    because the policy's top-k does not depend on them -- are ONE carried-state chain launch: tcgen05 pieces from the
+    carried (h, c) (icrl_chain_tc_lstm_fwd_from) with the joint checks, re-runs with a longer warm-up and the serial floor of
+    A2CEngine.step.  The value state starts from value_network.valrnn.hidden_cell and is written back to it (Q1)."""
+
+    def __init__(self, policy_network, value_network, chain_segments=32, chain_warmup=256, chain_tol=1e-5, chain_pieces=None,
+                 chain_adapt=True, chain_warmup_min=32):
+        self.policy, self.value, self.reward, self.a2c = policy_network, value_network, None, policy_network
+        if getattr(policy_network, "bidirectional", False) or getattr(value_network, "bidirectional", False):
+            raise NotImplementedError("the look-ahead engine is built for the unidirectional networks")
+        dev = policy_network.linear2vocab.weight.device
+        if dev.type != "cuda" or value_network.linear1.weight.device != dev:
+            raise _lib.IcrlError("the look-ahead engine needs both networks on one CUDA device (no CPU fallback)")
+        _lib.load()
+        self.device, self.V = dev, policy_network.linear2vocab.weight.shape[0]
+        self._bufs, self.launches, self.phase_events = {}, _lib.Launches(), None
+        self.chain_shards, self.chain_segments = 1, int(chain_segments)
+        self.chain_pieces = None if chain_pieces is None else int(chain_pieces)
+        self.chain_warmup, self.chain_tol = int(chain_warmup), float(chain_tol)
+        self.chain_adapt, self.chain_warmup_min = bool(chain_adapt), int(chain_warmup_min)
+        self.warm, self._clean, self._hold = {"v": self.chain_warmup}, {"v": 0}, {"v": 0}
+        self._tc = None
+        self.segment_stats = {"steps": 0, "segmented_steps": 0, "fallbacks": 0, "reruns": 0, "tc_max_err": [0.0] * 16,
+                              "warm_history": []}
+        self._seg_unverified = False
+        # per beam step: "pieces", "fallback" (pieces failed their checks, the serial kernels finished) or "serial" (too
+        # short to cut)
+        self.step_paths = []
+        with torch.cuda.device(dev):
+            self.sync_state = torch.zeros(int(_lib.call("icrl_chain_sync_bytes")), dtype=torch.uint8, device=dev)
+            # [4:20] joint-check words of the chain launch, [28:28+K*k] the children's batch means: ONE copy per beam step
+            self._stat_err = torch.zeros(28 + 16 * 16, dtype=torch.float32, device=dev)
+        self._tc_err = self._stat_err[4:20]
+
+    def pack_weights(self, reward=False):
+        """The operands of both networks, once per look_ahead call: gate tables, bf16x3 splits of the policy's W_hh and
+        W_v, the collapsed value head and the value chain's tcgen05 W_hh."""
+        st, L, V, c = self._stream, self.launches.ref, self.V, _lib.call
+        P, Vn = self.policy, self.value
+        for key, emb, lstm in (("p", P.caption_embedding, P.lstm), ("v", Vn.valrnn.caption_embedding, Vn.valrnn.lstm)):
+            c("icrl_pack_gate_table", st, V, 4 * H, 4 * H, emb.weight.shape[1], _p(emb.weight), _p(lstm.weight_ih_l0),
+              _p(lstm.bias_ih_l0), _p(lstm.bias_hh_l0), _p(self._buf(key + "_table", V * 4 * H)), L)
+        self._pack_policy_tc()
+        c("icrl_pack_value_head", st, _p(Vn.linear1.weight), _p(Vn.linear1.bias), _p(Vn.linear2.weight), _p(Vn.linear2.bias),
+          _p(self._buf("v_weff", 2 * H)), _p(self._buf("v_beff", 1)), L)
+        if self._use_tc_chains():
+            c("icrl_pack_chain_tc_weights", st, 0, _p(Vn.valrnn.lstm.weight_hh_l0),
+              _p(self._buf("v_chain_pk", int(c("icrl_chain_tc_weight_halves", 0)), torch.float16)), L)
+
+    def _value_chain(self, B, n, Kc, K, cand_tok, words, h0, c0):
+        """The value calls of one beam step as one chain from (h0, c0): values [B][Kc*K] and the chain's final (h, c) rows.
+        Pieces first; a failed joint check re-runs with the grown warm-up, then the serial kernels (A2CEngine.step)."""
+        st, L, b, Vn = self._stream, self.launches.ref, self._bufs, self.value
+        S = Kc * K
+        T = S * (n + 1) * B
+        serial, tried = False, False
+        for attempt in range(self._TC_ATTEMPTS + 1):
+            serial = serial or attempt == self._TC_ATTEMPTS
+            lay = None if serial or not self._use_tc_chains() else self._pieces_for(T, self.warm["v"])
+            self._tc = None if lay is None else {"v": (lay[0], lay[1], self.warm["v"]), "r": None}
+            npad = T if lay is None else max(T, lay[0] * lay[1] + self.warm["v"])
+            v_stream, take_pos = self._buf("la_stream", npad, torch.int32), self._buf("la_take_pos", S * B, torch.int32)
+            stash_h, stash_c = self._buf("la_stash_h", (npad + 1) * H), self._buf("la_stash_c", (npad + 1) * H)
+            _lib.call("icrl_lookahead_stream", st, B, n, Kc, K, _p(cand_tok), _p(words), _p(v_stream), _p(take_pos), L)
+            with self._phase("lookahead_value_chain"):
+              if lay is not None:
+                v_stream[T:npad].zero_()          # the last piece runs past the end of the chain
+                ws, cp = self._tc_scratch("v", lay[0])
+                _lib.call("icrl_chain_tc_lstm_fwd_from", st, lay[0], lay[1], self.warm["v"], _p(v_stream), _p(b["v_table"]),
+                          _p(b["v_chain_pk"]), _p(h0), _p(c0), _p(stash_h), _p(stash_c), None, _p(ws), _p(cp),
+                          _p(self._tc_err), L)
+              else:
+                _lib.call("icrl_chain_lstm_fwd", st, _p(v_stream), T, _p(b["v_table"]), _p(Vn.valrnn.lstm.weight_hh_l0), _p(h0),
+                          _p(c0), _p(stash_h), _p(stash_c), None, None, None, _p(self.sync_state), L)
+            take_h = self._buf("la_take_h", S * B * H)
+            _lib.call("icrl_gather_rows", st, S * B, _p(stash_h), _p(take_pos), 1, _p(take_h), L)
+            values = self._buf("la_values", B * S)
+            _lib.call("icrl_value_head_fwd", st, B, S, _p(self._la_f), _p(take_h), _p(b["v_weff"]), _p(b["v_beff"]), _p(values), L)
+            self.segment_stats["steps"] += 1
+            if lay is None:
+                break
+            tried = True
+            self.segment_stats["segmented_steps"] += 1
+            _lib.call("icrl_lookahead_score", st, B, Kc, K, _p(self._la_parent_score), _p(values), _p(self._la_top_val),
+                      _p(self._la_child), _p(self._stat_err[28:]), L)
+            ok, host = self._tc_ok()
+            if ok:
+                self.step_paths.append("pieces")
+                return stash_h[T * H:(T + 1) * H], stash_c[T * H:(T + 1) * H], host
+            serial = attempt + 1 == self._TC_ATTEMPTS
+        if tried:
+            self.segment_stats["fallbacks"] += 1
+        self.step_paths.append("fallback" if tried else "serial")
+        _lib.call("icrl_lookahead_score", st, B, Kc, K, _p(self._la_parent_score), _p(values), _p(self._la_top_val),
+                  _p(self._la_child), _p(self._stat_err[28:]), L)
+        _lib.call("icrl_chain_check", st, _p(self.sync_state))
+        return stash_h[T * H:(T + 1) * H], stash_c[T * H:(T + 1) * H], self._stat_err.tolist()
+
+    def look_ahead(self, features, first_col, beam=5, steps=16):
+        """GenerateCaptionsWithActorCriticLookAhead(most_likely=False) from the caption column `first_col` (B,): the
+        reference's list of `beam` (captions (B, steps+1) int64, score (B,1) f32) device tensors, best first."""
+        K = int(beam)
+        if not 1 <= K <= 16:
+            raise ValueError("the fused look-ahead keeps 1 to 16 candidates")
+        first = torch.as_tensor(np.asarray(first_col).reshape(-1).astype(np.int32))
+        B, V = first.numel(), self.V
+        dev, i32 = self.device, torch.int32
+        with torch.cuda.device(dev):
+            st, L = self._stream, self.launches.ref
+            P, rnn = self.policy, self.value.valrnn
+            self.pack_weights()
+            self._la_f = torch.as_tensor(features).to(dev, torch.float32).reshape(B, H).contiguous()
+            hc = rnn.hidden_cell
+            h0 = hc[0].to(dev, torch.float32).reshape(H).clone()
+            c0 = hc[1].to(dev, torch.float32).reshape(H).clone()
+            cand_tok = first.to(dev).view(1, 1, B)                  # [candidates][columns][B]
+            tok, parent = cand_tok.reshape(-1), None
+            score = torch.zeros((1, B), dtype=torch.float32, device=dev)
+            h_st = c_st = None
+            rows_b = torch.arange(B, dtype=i32, device=dev)
+            for t in range(steps):
+                Kc, n = cand_tok.shape[0], cand_tok.shape[1]
+                R, S = Kc * B, Kc * K
+                h_out, c_out = torch.empty((R, H), device=dev), torch.empty((R, H), device=dev)
+                self._la_top_val = torch.empty((R, K), dtype=torch.float32, device=dev)
+                top_idx = torch.empty((R, K), dtype=i32, device=dev)
+                ws = self._buf("la_policy_ws", (R * (46 * H + 4 * V) + 3) // 4)
+                with self._phase("lookahead_policy"):
+                    _lib.call("icrl_lookahead_policy_step", st, R, V, K, int(t == 0), _p(self._la_f), _p(P.cnn2linear.weight),
+                              _p(P.cnn2linear.bias), _p(self._bufs["p_table"]), _p(parent), _p(h_st), _p(c_st), _p(tok),
+                              _p(self._bufs["p_whh_parts"]), _p(self._bufs["p_wv_parts"]), _p(P.linear2vocab.bias), _p(h_out),
+                              _p(c_out), None, _p(self._la_top_val), _p(top_idx), _p(ws), L)
+                self._la_parent_score = score
+                self._la_child = torch.empty((S, B), dtype=torch.float32, device=dev)
+                h_fin, c_fin, host = self._value_chain(B, n, Kc, K, cand_tok, top_idx, h0, c0)
+                h0.copy_(h_fin)
+                c0.copy_(c_fin)
+                # trainers.py:93-94: a stable sort of the K*k children on their batch means, in the reference's list order
+                means = host[28:28 + S]
+                keep = sorted(range(S), key=lambda s: means[s])[:K]
+                sel = torch.tensor(keep, dtype=torch.int64).to(dev, non_blocking=True)
+                cand, word = sel // K, sel % K
+                words = top_idx.view(Kc, B, K)[cand, :, word]                          # [K][B]
+                cand_tok = torch.cat((cand_tok[cand], words.unsqueeze(1)), dim=1).contiguous()
+                score = self._la_child[sel].contiguous()
+                parent = (cand.to(i32).unsqueeze(1) * B + rows_b).reshape(-1).contiguous()
+                tok = words.reshape(-1).contiguous()
+                h_st, c_st = h_out, c_out
+            rnn.hidden_cell = (h0.view(1, 1, H), c0.view(1, 1, H))
+            caps = cand_tok.permute(0, 2, 1).to(torch.int64).contiguous()
+            return [(caps[j], score[j].view(B, 1)) for j in range(cand_tok.shape[0])]

@@ -8,7 +8,8 @@ global MT19937 stream exactly like the reference's ``np.random.choice`` calls (o
 per step, step-major), so ``np.random.seed(s)`` reproduces the reference's token ids.
 
 ``GenerateCaptionsWithActorCriticLookAhead`` / ``test_a2c_network`` (``:73-105``, ``:619-665``; SURVEY 8f row 1) run
-the reference's beam look-ahead on the drop-in modules.
+the reference's beam look-ahead on ``engine.LookAheadEngine`` (one tcgen05 value-chain launch per beam step from the
+carried value state), bidirectional networks on the drop-in modules.
 
 The supervised pretraining loops (``train_policy_network :202``, ``train_reward_network :260``,
 ``train_value_network :125``, ``VisualSemanticEmbeddingLoss :23``; SURVEY 8f row 2) run on the drop-in modules through
@@ -142,8 +143,28 @@ def GenerateCaptionsWithActorCriticLookAhead(features, captions, policy_network,
     top-k logit, a NaN where it is negative -- reproduced, the ordering key is the batch MEAN of the score), and
     keeps the `beamSize` expansions with the smallest mean.  The value network's hidden_cell is carried through
     every call and never reset inside (Q1), exactly as in the reference; callers reset it per batch
-    (trainers.py:661).  Policy and value forwards run on the CUDA kernels through the drop-in modules; top-k,
-    log and the sort are torch plumbing on (B,1,beam) tensors."""
+    (trainers.py:661).
+
+    Unidirectional networks on CUDA with beamSize <= 16 run on engine.LookAheadEngine: one policy beam step and ONE
+    value-chain launch per step (cached on the policy network, like GenerateCaptionsGreedy's engine).  Every other case
+    runs the reference's loop on the drop-in modules (_look_ahead_modules)."""
+    dev = policy_network.linear2vocab.weight.device
+    if (dev.type == "cuda" and 1 <= beamSize <= 16 and not getattr(policy_network, "bidirectional", False)
+            and not getattr(value_network, "bidirectional", False)):
+        eng = getattr(policy_network, "_icrl_lookahead", None)
+        if eng is None or eng.value is not value_network:
+            from .engine import LookAheadEngine
+            eng = LookAheadEngine(policy_network, value_network)
+            object.__setattr__(policy_network, "_icrl_lookahead", eng)
+        beam = eng.look_ahead(features, np.asarray(captions)[:, 0], beam=beamSize, steps=MAX_SEQ_LEN - 1)
+        return beam[0][0] if most_likely else beam
+    return _look_ahead_modules(features, captions, policy_network, value_network, beamSize, most_likely)
+
+
+def _look_ahead_modules(features, captions, policy_network, value_network, beamSize=5, most_likely=False):
+    """GenerateCaptionsWithActorCriticLookAhead as the reference's loop over the drop-in modules (bidirectional networks,
+    beamSize > 16, and the reference of the fused path's tests).  Policy and value forwards run on the CUDA kernels;
+    top-k, log and the sort are torch plumbing on (B,1,beam) tensors."""
     dev = policy_network.linear2vocab.weight.device
     feats = torch.as_tensor(np.asarray(features), device=dev).float().unsqueeze(0)
     start = torch.as_tensor(np.asarray(captions)[:, 0:1], device=dev).long()

@@ -264,6 +264,12 @@ int icrl_chain_tc_lstm_bwd(void* stream, int pieces, long long seg, int warm, co
                            const float* stash_gates, const float* stash_c, const int* take, const float* dh_take,
                            long long take_rows, void* dg_pairs, long long pair_rows, float* dg_inv_scale, void* ws,
                            float* cp_state, float* err, int* launches);
+/* LSTM pieces from a carried state: icrl_chain_tc_fwd(kind 0) with piece 0 starting from h0 / c0 [512] (16-byte aligned;
+ * NULL = zeros; both NULL gives icrl_chain_tc_fwd's output bit for bit).  Stash row 0 holds (h0, c0); the state after the
+ * chain's T live positions is stash row T. */
+int icrl_chain_tc_lstm_fwd_from(void* stream, int pieces, long long seg, int warm, const int* tok_stream, const float* table,
+                                const void* packed, const float* h0, const float* c0, float* stash_h, float* stash_c,
+                                float* stash_gates, void* ws, float* cp_state, float* err, int* launches);
 /*      The gate gradients of the live positions come out as the fp16 pairs the recurrence itself runs on: dg_pairs =
  *      [2][pair_rows][2048] halves (hi plane, then lo' plane; pair_rows >= pieces * seg + warm, 32-byte aligned), value =
  *      (hi + lo'/2048) * *dg_inv_scale (one power of two per launch, written to the device word dg_inv_scale), columns of
@@ -330,6 +336,28 @@ int icrl_reward_cosine_fwd(void* stream, int B, int S, const float* ve, const fl
  *      dv_sb [S][B] = dL/dvalues, dlogp [B][S] = dL/dlogp, sum_dv [1]  (all nullable). */
 int icrl_a2c_loss_fwd_bwd(void* stream, int B, int S, const float* values, const float* rewards, const float* logp,
                           float inv_denom, float* out3, float* dv_sb, float* dlogp, float* sum_dv, int* launches);
+
+/* ---- value-guided look-ahead decoder (GenerateCaptionsWithActorCriticLookAhead, trainers.py:73-105).  K candidate
+ *      caption batches of B rows and n columns each are expanded by their k best words per beam step.
+ *      Stream: cand_tok [K][n][B] int32 (each candidate's columns), words [K][B][k] int32 -> the value chain of the step,
+ *      K*k blocks of (n+1)*B positions in the reference's call order (block c*k + i = candidate c's n columns, then its
+ *      word column i), and take_pos [K*k][B] = stream position of each row of the word column (for icrl_gather_rows). */
+int icrl_lookahead_stream(void* stream, int B, int n, int K, int k, const int* cand_tok, const int* words, int* tok_stream,
+                          int* take_pos, int* launches);
+/*      Policy beam step for R rows (R = K*B): each row's (h, c) is gathered from row parent[r] of h_in / c_in [*][512]
+ *      (first != 0: the initial state cnn2linear(features [R][512]), c = 0; parent, h_in, c_in unused), one LSTM cell
+ *      consumes tok [R] (gate table `table`, W_hh as the icrl_split_bf16x3 parts whh_parts) into h_out / c_out [R][512],
+ *      logits = h_out W_v^T + b_v (wv_parts) go to `logits` [R][V] (nullable) and their top k <= 16 (descending, equal
+ *      values by lower index) to top_val [R][k] f32 / top_idx [R][k] int32.  ws: R * (46*512 + 4*V) bytes. */
+int icrl_lookahead_policy_step(void* stream, int R, int V, int k, int first, const float* features, const float* W_cnn,
+                               const float* b_cnn, const float* table, const int* parent, const float* h_in, const float* c_in,
+                               const int* tok, const void* whh_parts, const void* wv_parts, const float* b_v, float* h_out,
+                               float* c_out, float* logits, float* top_val, int* top_idx, void* ws, int* launches);
+/*      Scores: child_score [K*k][B] = parent_score [K][B] - (0.6 values + 0.4 log(top_val)) in fp32 and the reference's
+ *      operation order (values [B][K*k] of icrl_value_head_fwd with S = K*k; a negative logit gives NaN as there), and
+ *      means [K*k] = each child's batch mean (the reference's sort key). */
+int icrl_lookahead_score(void* stream, int B, int K, int k, const float* parent_score, const float* values, const float* top_val,
+                         float* child_score, float* means, int* launches);
 
 /* ---- optimizer (replaces torch.optim.Adam.step over the 18 tensors, trainers.py:378, 480; SURVEY 8f row 4): one
  *      kernel over the flat parameter / gradient buckets, torch's default Adam (betas 0.9/0.999, eps 1e-8, no weight
