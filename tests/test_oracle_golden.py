@@ -59,6 +59,58 @@ def test_ref_port_matches_reference(golden_dir, name):
     _check(res, g, 1e-7, 1e-6)          # same library calls in the same order: ~bitwise
 
 
+def _variant_case(golden_dir, name):
+    """a2c_b12_l7_bidir / a2c_b16_l8_wemb300 with the weight layout they were generated with."""
+    g, _, f, c, u, level = _load(golden_dir, name)
+    w = synth.make_weights(int(g["seed"]), wordvec_dim=int(g["wordvec_dim"]), bidirectional=name.endswith("bidir"))
+    return g, w, f, c, u, level
+
+
+@pytest.mark.parametrize("dtype,tol_val,tol_grad", [(torch.float32, 1e-7, 1e-6), (torch.float64, 2e-6, 5e-6)])
+@pytest.mark.parametrize("name", ["a2c_b12_l7_bidir", "a2c_b16_l8_wemb300"])
+def test_ref_port_variants_match_reference(golden_dir, name, dtype, tol_val, tol_grad):
+    """The bidirectional networks and the frozen 300-d word vectors, in float32 (the as-executed port: ~bitwise) and in
+    float64 (the reference the module-route kernels are checked against: tokens equal, the rest to fp32 rounding)."""
+    g, w, f, c, u, level = _variant_case(golden_dir, name)
+    nets = ref_port.Nets(w, dtype=dtype, bidirectional=name.endswith("bidir"))
+    res = ref_port.a2c_minibatch(nets, f, c, u, level=level)
+    _check(res, g, tol_val, tol_grad)
+    assert nets.v_state[0].dtype == dtype and nets.v_state[0].shape == (1 + nets.bidirectional, 1, 512)
+    if name.endswith("wemb300"):
+        assert nets.p_rnn.weight_ih_l0.shape == (2048, 300) and not nets.p_emb.weight.requires_grad
+        assert len(res["grads"]) == 16
+
+
+@pytest.mark.parametrize("dtype,tol_val,tol_grad", [(torch.float32, 1e-7, 1e-6), (torch.float64, 2e-6, 5e-6)])
+def test_ref_port_pretraining_losses_match_reference(golden_dir, dtype, tol_val, tol_grad):
+    """The three supervised pretraining losses (weighted cross-entropy, VisualSemanticEmbeddingLoss, MSE on the greedy
+    captions' rewards) and all 27 gradients, against one minibatch of each of the reference's loops."""
+    g = np.load(os.path.join(golden_dir, "pretrain_b12.npz"))
+    seed, B = int(g["seed"]), int(g["B"])
+    w = synth.make_weights(seed)
+    f, c = synth.make_inputs(seed, B, 17)
+    nets = ref_port.Nets(w, dtype=dtype)
+    k = int(g["value_prefix_len"])
+    runs = {"policy": lambda: ref_port.policy_xent_loss(nets, f, c),
+            "reward": lambda: ref_port.reward_vse_loss(nets, f, c),
+            "value": lambda: ref_port.value_mse_loss(nets, f, c, k)}
+    ngrads = 0
+    for key, fn in runs.items():
+        res, grads = ref_port.network_grads(nets, key, fn)
+        ref_loss = float(g[key + "_loss"])
+        loss = float(res[0].detach())
+        assert abs(loss - ref_loss) <= tol_val * max(1.0, abs(ref_loss)), (key, loss, ref_loss)
+        for name, grad in grads.items():
+            flat = grad.numpy().reshape(-1)
+            ref = g["%s/gsamp/%s" % (key, name)]
+            scale = max(float(np.abs(ref).max()), 1e-12)
+            assert np.abs(flat[grad_sample_index(flat.size)] - ref).max() <= tol_grad * scale, (key, name)
+            nrm, ref_n = float(np.sqrt((flat.astype(np.float64) ** 2).sum())), float(g["%s/gnorm/%s" % (key, name)])
+            assert abs(nrm - ref_n) <= 1e-5 * max(ref_n, 1e-12), (key, name)
+            ngrads += 1
+    assert ngrads == 27
+
+
 @pytest.mark.parametrize("name", A2C_CASES)
 @pytest.mark.parametrize("lib", [False, True])
 def test_single_pass_matches_reference(golden_dir, name, lib):
