@@ -719,4 +719,32 @@ int icrl_a2c_loss_fwd_bwd(void* stream, int B, int S, const float* values, const
   return ICRL_OK;
 }
 
+// ---- entropy bonus (new; the reference's loss has none)
+int icrl_policy_entropy(void* stream, int B, int S, int V, const float* logits, int ldl, float* entropy, int* launches) {
+  ICRL_REQUIRE(B > 0 && S > 0 && V > 0 && ldl >= V, "bad entropy shape (B, S, V > 0, ldl >= V)");
+  ICRL_REQUIRE(logits && entropy, "the entropy pass needs the logits and the output");
+  TRY(icrl_policy_entropy_impl(S_(stream), B, S, V, logits, ldl, entropy));
+  bump(launches, 1);
+  return ICRL_OK;
+}
+
+int icrl_a2c_loss_entropy_fwd_bwd(void* stream, int B, int S, const float* values, const float* rewards, const float* logp,
+                                  const float* entropy, float entropy_coef, float inv_denom, float* out4, float* dv_sb,
+                                  float* dlogp, float* sum_dv, int* launches) {
+  ICRL_REQUIRE(entropy && out4, "the entropy loss needs the entropy and four output words");
+  TRY(icrl_a2c_loss_impl(S_(stream), B, S, values, rewards, logp, inv_denom, out4, dv_sb, dlogp, sum_dv, entropy,
+                         entropy_coef));
+  bump(launches, 1);
+  return ICRL_OK;
+}
+
+int icrl_softmax_entropy_bwd(void* stream, int B, int S, int V, float* z, int ldz, const long long* tokens_out,
+                             const float* dlogp, const float* entropy, float scale, int* launches) {
+  ICRL_REQUIRE(B > 0 && S > 0 && V > 0 && ldz >= V, "bad logits shape (B, S, V > 0, ldz >= V)");
+  ICRL_REQUIRE(z && tokens_out && dlogp && entropy, "the softmax backward needs z, the tokens, dL/dlogp and the entropy");
+  TRY(icrl_softmax_bwd(S_(stream), B, S, V, z, ldz, tokens_out, dlogp, entropy, scale));
+  bump(launches, 1);
+  return ICRL_OK;
+}
+
 }  // extern "C"

@@ -4,7 +4,8 @@
 //                w_eff = W2 W1 (1024), b_eff = W2 b1 + b2; the gradients of W1, b1, W2, b2 are
 //                reconstructed exactly from g = sum dv * [f, h] and sum dv (rank-1 structure).
 //   reward       trainers.py:117-120 : cos(visual_embed(f), semantic_embed(h)), F.normalize eps 1e-12.
-//   loss         trainers.py:471-475 : adv = values - rewards; mean(-logp*adv) + 0.5*mean(adv^2).
+//   loss         trainers.py:471-475 : adv = values - rewards; mean(-logp*adv) + 0.5*mean(adv^2)
+//                (optionally - entropy_coef * mean(policy entropy): the entropy bonus, off by default).
 #include "common.cuh"
 
 namespace {
@@ -100,11 +101,14 @@ __global__ void reward_cosine_kernel(int B, int S, const float* __restrict__ ve,
 // = 1/(B_global*S); for a data-parallel shard these are partial sums to be all-reduced).
 //   dL/dvalues = (adv - logp) * inv_denom   (written [S][B] for the chain backward)
 //   dL/dlogp   = -adv * inv_denom           (written [B][S])
+// entropy != NULL ([B][S], the policy's entropy per sampled step): the entropy bonus -entropy_coef * mean(H) is added
+// to out[0] and out[3] = mean entropy (scaled by inv_denom like the others); the gradient seeds do not change.
 __global__ void a2c_loss_kernel(int B, int S, const float* __restrict__ values, const float* __restrict__ rewards,
                                 const float* __restrict__ logp, float inv_denom, float* __restrict__ out,
-                                float* __restrict__ dv_sb, float* __restrict__ dlogp, float* __restrict__ sum_dv) {
-  __shared__ double red[4][32];
-  double l = 0.0, r = 0.0, a = 0.0, d = 0.0;
+                                float* __restrict__ dv_sb, float* __restrict__ dlogp, float* __restrict__ sum_dv,
+                                const float* __restrict__ entropy, float entropy_coef) {
+  __shared__ double red[5][32];
+  double l = 0.0, r = 0.0, a = 0.0, d = 0.0, e = 0.0;
   const int n = B * S;
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
     const int b = i / S, s = i % S;
@@ -117,18 +121,25 @@ __global__ void a2c_loss_kernel(int B, int S, const float* __restrict__ values, 
     d += (double)dv;
     if (dv_sb) dv_sb[(size_t)s * B + b] = dv;
     if (dlogp) dlogp[i] = -adv * inv_denom;
+    if (entropy) e += (double)entropy[i];
   }
-  l = warp_sum_d(l); r = warp_sum_d(r); a = warp_sum_d(a); d = warp_sum_d(d);
+  l = warp_sum_d(l); r = warp_sum_d(r); a = warp_sum_d(a); d = warp_sum_d(d); e = warp_sum_d(e);
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (lane == 0) { red[0][w] = l; red[1][w] = r; red[2][w] = a; red[3][w] = d; }
+  if (lane == 0) { red[0][w] = l; red[1][w] = r; red[2][w] = a; red[3][w] = d; red[4][w] = e; }
   __syncthreads();
   if (w == 0) {
     const int nw = blockDim.x >> 5;
     l = lane < nw ? red[0][lane] : 0.0; r = lane < nw ? red[1][lane] : 0.0;
     a = lane < nw ? red[2][lane] : 0.0; d = lane < nw ? red[3][lane] : 0.0;
-    l = warp_sum_d(l); r = warp_sum_d(r); a = warp_sum_d(a); d = warp_sum_d(d);
+    e = lane < nw ? red[4][lane] : 0.0;
+    l = warp_sum_d(l); r = warp_sum_d(r); a = warp_sum_d(a); d = warp_sum_d(d); e = warp_sum_d(e);
     if (lane == 0) {
-      out[0] = (float)(l * (double)inv_denom);
+      if (entropy) {
+        out[0] = (float)((l - (double)entropy_coef * e) * (double)inv_denom);
+        out[3] = (float)(e * (double)inv_denom);
+      } else {
+        out[0] = (float)(l * (double)inv_denom);
+      }
       out[1] = (float)(r * (double)inv_denom);
       out[2] = (float)(a * (double)inv_denom);
       if (sum_dv) sum_dv[0] = (float)d;
@@ -303,8 +314,10 @@ int icrl_reward_cosine_impl(cudaStream_t st, int B, int S, const float* ve, cons
 }
 
 int icrl_a2c_loss_impl(cudaStream_t st, int B, int S, const float* values, const float* rewards, const float* logp,
-                       float inv_denom, float* out3, float* dv_sb, float* dlogp, float* sum_dv) {
-  a2c_loss_kernel<<<1, 1024, 0, st>>>(B, S, values, rewards, logp, inv_denom, out3, dv_sb, dlogp, sum_dv);
+                       float inv_denom, float* out3, float* dv_sb, float* dlogp, float* sum_dv, const float* entropy,
+                       float entropy_coef) {
+  a2c_loss_kernel<<<1, 1024, 0, st>>>(B, S, values, rewards, logp, inv_denom, out3, dv_sb, dlogp, sum_dv, entropy,
+                                      entropy_coef);
   ICRL_LAUNCH_CHECK();
   return ICRL_OK;
 }

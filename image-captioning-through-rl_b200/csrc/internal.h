@@ -11,8 +11,10 @@ int icrl_lstm_pointwise_bwd(cudaStream_t st, int B, const float* dh_rec, const f
                             const float* gates_act, const float* c_prev, const float* c_cur, float* dgpre);
 int icrl_softmax_sample(cudaStream_t st, int B, int V, const float* logits, int ldl, const double* uniforms, int greedy,
                         const long long* forced, int* tok_next, long long* tokens_out, float* logp_out, int S, int s, float* probs_out);
+// entropy (nullable, [B][S]): add the entropy bonus's term scale * p (log p + H) to dL/dlogits
 int icrl_softmax_bwd(cudaStream_t st, int B, int S, int V, float* z, int ldl, const long long* tokens_out,
-                     const float* dlogp);
+                     const float* dlogp, const float* entropy = nullptr, float scale = 0.f);
+int icrl_policy_entropy_impl(cudaStream_t st, int B, int S, int V, const float* logits, int ldl, float* entropy);
 int icrl_topk_rows(cudaStream_t st, int R, int V, int k, const float* x, float* top_val, int* top_idx);
 int icrl_scatter_add_rows(cudaStream_t st, long long R, int C, const float* src, const int* idx, float* dst);
 int icrl_scatter_add_stream(cudaStream_t st, int B, int p0, int S, int extra, int C, const float* src, const int* tok_stream,
@@ -32,7 +34,8 @@ int icrl_value_head_grads_impl(cudaStream_t st, const float* g, const float* sdv
                                const float* W2, float* dW1, float* db1, float* dW2, float* db2);
 int icrl_reward_cosine_impl(cudaStream_t st, int B, int S, const float* ve, const float* se, float* rewards);
 int icrl_a2c_loss_impl(cudaStream_t st, int B, int S, const float* values, const float* rewards, const float* logp,
-                       float inv_denom, float* out3, float* dv_sb, float* dlogp, float* sum_dv);
+                       float inv_denom, float* out3, float* dv_sb, float* dlogp, float* sum_dv,
+                       const float* entropy = nullptr, float entropy_coef = 0.f);
 int icrl_build_stream_impl(cudaStream_t st, int B, int p0, int S, int extra, const int* tokcm, int* stream, int* take,
                            int* take_pos);
 int icrl_gather_rows_impl(cudaStream_t st, long long R, const float* src, const int* idx, long long row_offset,

@@ -119,8 +119,11 @@ __global__ void softmax_sample_kernel(int B, int V, const float* __restrict__ lo
 }
 
 // In place: row r = s*B + b of z (logits) becomes dL/dlogits = dlogp[b][s] * (onehot(a) - softmax(z)).
+// entropy != NULL (entropy [B][S] of policy_entropy_kernel) adds the entropy bonus's term scale * p (log p + H), with
+// log p = (z - max) - log(sum) so that it stays finite where p underflows to zero.
 __global__ void softmax_bwd_kernel(int B, int S, int V, float* __restrict__ z, int ldl,
-                                   const long long* __restrict__ tokens_out, const float* __restrict__ dlogp) {
+                                   const long long* __restrict__ tokens_out, const float* __restrict__ dlogp,
+                                   const float* __restrict__ entropy, float scale) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= B * S) return;
   const int s = warp / B, b = warp % B;
@@ -130,13 +133,45 @@ __global__ void softmax_bwd_kernel(int B, int S, int V, float* __restrict__ z, i
   mx = warp_max(mx);
   float sum = 0.f;
   for (int v = lane; v < V; v += 32) sum += expf(x[v] - mx);
-  const float inv = 1.0f / warp_sum(sum);
+  const float tot = warp_sum(sum);
+  const float inv = 1.0f / tot;
   const float d = dlogp[(size_t)b * S + s];
   const int a = (int)tokens_out[(size_t)b * S + s];
+  if (entropy) {
+    const float h = entropy[(size_t)b * S + s], lsum = logf(tot);
+    for (int v = lane; v < V; v += 32) {
+      const float p = expf(x[v] - mx) * inv;
+      x[v] = d * ((v == a ? 1.f : 0.f) - p) + scale * p * ((x[v] - mx) - lsum + h);
+    }
+    return;
+  }
   for (int v = lane; v < V; v += 32) {
     const float p = expf(x[v] - mx) * inv;
     x[v] = d * ((v == a ? 1.f : 0.f) - p);
   }
+}
+
+// One warp per row r = s*B + b of the logits stash (row stride ldl, the V real columns only): entropy[b][s] =
+// -sum p log p = log(sum) - sum e (z - max) / sum with e = exp(z - max), the max / exp / sum of softmax_bwd_kernel.
+// A column whose e underflows to zero adds nothing (also for z = -inf).
+__global__ void policy_entropy_kernel(int B, int S, int V, const float* __restrict__ logits, int ldl,
+                                      float* __restrict__ entropy) {
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (warp >= B * S) return;
+  const int s = warp / B, b = warp % B;
+  const float* x = logits + (size_t)warp * ldl;
+  float mx = -INFINITY;
+  for (int v = lane; v < V; v += 32) mx = fmaxf(mx, x[v]);
+  mx = warp_max(mx);
+  float sum = 0.f, t = 0.f;
+  for (int v = lane; v < V; v += 32) {
+    const float y = x[v] - mx, e = expf(y);
+    sum += e;
+    if (e > 0.f) t = fmaf(e, y, t);
+  }
+  const float tot = warp_sum(sum);
+  t = warp_sum(t);
+  if (lane == 0) entropy[(size_t)b * S + s] = logf(tot) - t / tot;
 }
 
 // The same with 16-byte vector reductions (red.global.add.v4.f32, sm_90+): a quarter of the instructions and of the L2
@@ -318,8 +353,15 @@ int icrl_softmax_sample(cudaStream_t st, int B, int V, const float* logits, int 
 }
 
 int icrl_softmax_bwd(cudaStream_t st, int B, int S, int V, float* z, int ldl, const long long* tokens_out,
-                     const float* dlogp) {
-  softmax_bwd_kernel<<<icrl_cdiv((long long)B * S * 32, 128), 128, 0, st>>>(B, S, V, z, ldl, tokens_out, dlogp);
+                     const float* dlogp, const float* entropy, float scale) {
+  softmax_bwd_kernel<<<icrl_cdiv((long long)B * S * 32, 128), 128, 0, st>>>(B, S, V, z, ldl, tokens_out, dlogp, entropy,
+                                                                           scale);
+  ICRL_LAUNCH_CHECK();
+  return ICRL_OK;
+}
+
+int icrl_policy_entropy_impl(cudaStream_t st, int B, int S, int V, const float* logits, int ldl, float* entropy) {
+  policy_entropy_kernel<<<icrl_cdiv((long long)B * S * 32, 128), 128, 0, st>>>(B, S, V, logits, ldl, entropy);
   ICRL_LAUNCH_CHECK();
   return ICRL_OK;
 }

@@ -33,9 +33,10 @@ def _p(t):
 
 
 class StepResult(dict):
-    """Device tensors of one minibatch; ``loss`` / ``mean_reward`` / ``mean_adv`` sync lazily."""
+    """Device tensors of one minibatch; ``loss`` / ``mean_reward`` / ``mean_adv`` (and ``mean_entropy`` when the engine
+    has an entropy bonus) sync lazily."""
 
-    host_stats = None       # (loss, mean reward, mean advantage) when the step's check already brought them to the host
+    host_stats = None       # (loss, mean reward, mean advantage[, mean entropy]) when the step's check brought them over
 
     def _stat(self, i):
         if self.host_stats is not None:
@@ -53,6 +54,13 @@ class StepResult(dict):
     @property
     def mean_adv(self):
         return self._stat(2)
+
+    @property
+    def mean_entropy(self):
+        """Mean policy entropy of the sampled steps; only steps of an engine with entropy_coef != 0 track it."""
+        if len(self["stats"]) < 4:
+            raise AttributeError("the step ran without an entropy bonus (entropy_coef = 0): no entropy was computed")
+        return self._stat(3)
 
 
 class Prepared:
@@ -79,10 +87,16 @@ def plan_rollout(captions, level=None):
 
 class A2CEngine:
     DECODE_MODES = ("fused", "tc", "simt")
+    entropy_coef = 0.0            # engines that skip __init__ (look-ahead, greedy decode) have no entropy bonus
 
     def __init__(self, a2c_network, reward_network, use_tc=None, decode="fused", chain_shards=1, wgrad="tc",
                  chain_segments=32, chain_warmup=256, chain_tol=1e-5, chain_engine="tc",
-                 chain_pieces=None, chain_adapt=True, chain_warmup_min=32, policy_bptt="tc", chain_fuse_fwd=True, overlap_backward=True):
+                 chain_pieces=None, chain_adapt=True, chain_warmup_min=32, policy_bptt="tc", chain_fuse_fwd=True, overlap_backward=True,
+                 entropy_coef=0.0):
+        # entropy_coef: weight of the entropy bonus, loss = reference loss - entropy_coef * mean policy entropy over the
+        # sampled steps (the A3C regulariser; positive values favour exploration).  0 is the reference's loss, computed
+        # by exactly the kernels it always was.
+        self.entropy_coef = float(entropy_coef)
         self.policy = a2c_network.policy_network
         self.value = a2c_network.value_network
         self.reward = reward_network
@@ -173,8 +187,9 @@ class A2CEngine:
         self._seg_unverified = False
         with torch.cuda.device(dev):
             self.sync_state = torch.zeros(int(_lib.call("icrl_chain_sync_bytes")), dtype=torch.uint8, device=dev)
-            # [0:3] loss, mean reward, mean advantage; [4:20] joint-check words of the tc chain launches (value forward
-            # 4..7, reward forward 8..11, value backward 12..17): read together in ONE device-to-host copy per step
+            # [0:3] loss, mean reward, mean advantage; [3] mean entropy (entropy bonus only); [4:20] joint-check words of
+            # the tc chain launches (value forward 4..7, reward forward 8..11, value backward 12..17): read together in ONE
+            # device-to-host copy per step
             # [20:28] words of the policy's tcgen05 BPTT ([24] max |dL/dh|, [25] fp16-exchange overflow flag)
             self._stat_err = torch.zeros(28, dtype=torch.float32, device=dev)
         self._tc_err = self._stat_err[4:20]
@@ -559,8 +574,9 @@ class A2CEngine:
         _lib.call("icrl_reward_cosine_fwd", st, B, S, _p(ve), _p(se), _p(rewards), L)
         return values, rewards
 
-    def _backward(self, f, tokcm, tokens, B, p0, S, Tv):
-        """Backward of the minibatch.  The policy's backward depends only on dL/dlogp; the value network's only on
+    def _backward(self, f, tokcm, tokens, B, p0, S, Tv, ent=None):
+        """Backward of the minibatch.  The policy's backward depends only on dL/dlogp (and the entropy bonus, `ent` =
+        (entropy [B][S], entropy_coef * inv_denom) or None); the value network's only on
         dL/dvalues: with overlap_backward the policy side runs on a second stream (own workspaces) while the main stream
         walks the value chain backwards -- the chain kernels occupy 120 of the 148 SMs (clusters of 8 cannot span GPCs),
         the policy's contractions fill the rest and whatever the chain kernel leaves in time."""
@@ -582,7 +598,7 @@ class A2CEngine:
                               gemm_ws_floats * 4, 2, self.launches.ref)
                     h_packed = torch.cuda.Event()
                     h_packed.record(self._side_stream)
-                self._backward_policy(f, tokcm, tokens, B, p0, S, "_p")
+                self._backward_policy(f, tokcm, tokens, B, p0, S, "_p", ent)
                 join = torch.cuda.Event()
                 join.record(self._side_stream)
             if h_packed is not None:
@@ -592,7 +608,7 @@ class A2CEngine:
         else:
             self._backward_value(f, B, p0, S, Tv, launch_only_chain=True)
             self._backward_value(f, B, p0, S, Tv, launch_only_chain=False)
-            self._backward_policy(f, tokcm, tokens, B, p0, S, "")
+            self._backward_policy(f, tokcm, tokens, B, p0, S, "", ent)
 
     def _bwd_workspaces(self, B, S, Tv, tag):
         """(colsum_ws, gemm_ws, gemm_ws_floats, dtable) of the value side (tag "") or the policy side on its own stream."""
@@ -660,7 +676,7 @@ class A2CEngine:
             _lib.call("icrl_chain_lstm_bwd", st, Tv, _p(Vn.valrnn.lstm.weight_hh_l0), _p(b["v_stash_g"]), _p(b["v_stash_c"]),
                   _p(b["v_take"]), _p(dh_take), _p(dgates), _p(self.sync_state), None, None, None, None, L)
 
-    def _backward_policy(self, f, tokcm, tokens, B, p0, S, tag):
+    def _backward_policy(self, f, tokcm, tokens, B, p0, S, tag, ent=None):
         # policy BPTT.  icrl_policy_rollout_bwd turns the logits into dL/dlogits IN PLACE; a step whose chains are re-run
         # (longer warm-up, serial fall-back) runs this backward again with slightly different dL/dlogp, so it works on a
         # copy and the rollout's logits stay intact.
@@ -680,8 +696,13 @@ class A2CEngine:
             self._dz_ld = ldz
         with self._phase("policy_bwd"):
           dz[:SB * ldz].view(SB, ldz)[:, :V].copy_(b["p_logits"][:SB * V].view(SB, V))
+          dlogp = b["dlogp"]
+          if ent is not None:
+            # dL/dlogits with the entropy bonus's term, in place; the rollout backward then starts from it (dlogp = NULL)
+            _lib.call("icrl_softmax_entropy_bwd", st, B, S, V, _p(dz), ldz, _p(tokens), _p(dlogp), _p(ent[0]), ent[1], L)
+            dlogp = None
           args = [st, B, V, p0, S, P.caption_embedding.weight.shape[1], _p(f), _p(P.caption_embedding.weight), _p(pl.weight_ih_l0),
-                  _p(pl.weight_hh_l0), _p(P.linear2vocab.weight), _p(tokcm), _p(tokens), _p(b["dlogp"]), _p(b["p_Hs"]),
+                  _p(pl.weight_hh_l0), _p(P.linear2vocab.weight), _p(tokcm), _p(tokens), _p(dlogp), _p(b["p_Hs"]),
                   _p(b["p_Cs"]), _p(b["p_Gs"]), _p(dz), _p(self._buf("p_dHv", SB * H)),
                   _p(self._buf("p_DG", n_cell * B * 4 * H)), _p(self._buf("p_dh", 2 * B * H)), _p(self._buf("p_dc", B * H)),
                   _p(dtable), _p(colsum_ws), _p(gemm_ws), gemm_ws_floats * 4, _p(g(P.caption_embedding.weight, True)),
@@ -725,14 +746,26 @@ class A2CEngine:
             dlogp = self._buf("dlogp", S * B)
             sum_dv = self._buf("sum_dv", 1)
             inv = 1.0 / float((global_rows or B) * S)
+            ent = None
+            if self.entropy_coef:
+                # the entropy of every sampled step's softmax, from the logits stash; a chain re-run leaves it as it is
+                entropy = self._buf("p_entropy", S * B)
+                with self._phase("policy_entropy"):
+                    _lib.call("icrl_policy_entropy", self._stream, B, S, self.V, _p(self._bufs["p_logits"]), self.V, _p(entropy),
+                              self.launches.ref)
+                ent = (entropy, self.entropy_coef * inv)
 
             def run_chains(serial):
                 Tv, Tr = self._streams(tokcm, B, p0, S, serial=serial)
                 values, rewards = self._chains_forward(f, B, S, Tv, Tr, backward)
-                _lib.call("icrl_a2c_loss_fwd_bwd", self._stream, B, S, _p(values), _p(rewards), _p(logp), inv, _p(self._stat_err),
-                          _p(dv_sb), _p(dlogp), _p(sum_dv), self.launches.ref)
+                if ent is None:
+                    _lib.call("icrl_a2c_loss_fwd_bwd", self._stream, B, S, _p(values), _p(rewards), _p(logp), inv, _p(self._stat_err),
+                              _p(dv_sb), _p(dlogp), _p(sum_dv), self.launches.ref)
+                else:             # _stat_err[3] = mean entropy, brought over with the joint-check words
+                    _lib.call("icrl_a2c_loss_entropy_fwd_bwd", self._stream, B, S, _p(values), _p(rewards), _p(logp), _p(ent[0]),
+                              self.entropy_coef, inv, _p(self._stat_err), _p(dv_sb), _p(dlogp), _p(sum_dv), self.launches.ref)
                 if backward:
-                    self._backward(f, tokcm, tokens, B, p0, S, Tv)
+                    self._backward(f, tokcm, tokens, B, p0, S, Tv, ent)
                 self.segment_stats["steps"] += 1
                 return Tv, Tr, values, rewards
 
@@ -756,13 +789,14 @@ class A2CEngine:
                 serial = self._tc_force_serial or attempt + 1 == self._TC_ATTEMPTS
                 if serial:
                     self.segment_stats["fallbacks"] += 1
-            stats = self._stat_err[:3].clone()
+            n_stats = 3 if ent is None else 4
+            stats = self._stat_err[:n_stats].clone()
             if check and self._tc is None:
                 _lib.call("icrl_chain_check", self._stream, _p(self.sync_state))
         res = StepResult(tokens=tokens, logp=logp, values=values, rewards=rewards, stats=stats, p0=p0, S=S, B=B,
                          Tv=Tv, Tr=Tr)
         if host is not None:
-            res.host_stats = host[:3]
+            res.host_stats = host[:n_stats]
         return res
 
     _TC_ATTEMPTS = 3

@@ -40,11 +40,13 @@ except Exception:               # pragma: no cover
             pass
 
 
-def _engine_for(a2c_network, reward_network):
+def _engine_for(a2c_network, reward_network, entropy_coef=0.0):
     eng = getattr(a2c_network, "_icrl_engine", None)
     if eng is None or eng.reward is not reward_network:
-        eng = A2CEngine(a2c_network, reward_network)
+        eng = A2CEngine(a2c_network, reward_network, entropy_coef=entropy_coef)
         object.__setattr__(a2c_network, "_icrl_engine", eng)
+    # the cached engine is kept (its flat gradient bucket is the one FlatAdam steps); only the coefficient follows the call
+    eng.entropy_coef = float(entropy_coef)
     return eng
 
 
@@ -366,14 +368,15 @@ def train_value_network(train_data, network_paths, plot_dir, bidirectional, epoc
 
 
 class _ModuleRouteResult:
-    def __init__(self, loss, mean_reward, mean_adv):
-        self.loss, self.mean_reward, self.mean_adv = loss, mean_reward, mean_adv
+    def __init__(self, loss, mean_reward, mean_adv, mean_entropy=None):
+        self.loss, self.mean_reward, self.mean_adv, self.mean_entropy = loss, mean_reward, mean_adv, mean_entropy
 
 
-def _module_route_step(a2c_network, reward_network, features, captions, level):
+def _module_route_step(a2c_network, reward_network, features, captions, level, entropy_coef=0.0):
     """One minibatch through the modules' autograd instead of the fused engine (used for the bidirectional variant):
     the reference's loop body, trainers.py:428-479 / 544-593.  Leaves the gradients in .grad; returns None when the
-    curriculum level does not fit (trainers.py:550)."""
+    curriculum level does not fit (trainers.py:550).  entropy_coef != 0 subtracts entropy_coef times the mean entropy
+    of the sampled steps' softmax from the loss (A2CEngine's entropy bonus); autograd carries it into the policy."""
     from .engine import plan_rollout
     p0, S = plan_rollout(captions, level)
     if p0 < 1:
@@ -381,9 +384,12 @@ def _module_route_step(a2c_network, reward_network, features, captions, level):
     dev = a2c_network.policy_network.linear2vocab.weight.device
     feats = torch.as_tensor(np.asarray(features), device=dev).float()
     caps_in = torch.as_tensor(np.asarray(captions)[:, :p0], device=dev).long()
-    values, rewards, log_probs = [], [], []
+    values, rewards, log_probs, entropies = [], [], [], []
     for _ in range(S):
         value, logits = a2c_network(feats, caps_in)
+        if entropy_coef:
+            z = logits[:, 0, :]
+            entropies.append(-(F.softmax(z, dim=1) * F.log_softmax(z, dim=1)).sum(dim=1))
         probs = F.softmax(logits, dim=2)
         dist = probs.detach().cpu().numpy()[:, 0]
         acts = [np.random.choice(probs.shape[-1], p=dist[i]) for i in range(dist.shape[0])]     # trainers.py:447-450
@@ -397,10 +403,15 @@ def _module_route_step(a2c_network, reward_network, features, captions, level):
     log_probs = torch.stack(log_probs, dim=1).squeeze()
     advantage = values - rewards
     loss = (-log_probs * advantage).mean() + 0.5 * advantage.pow(2).mean()
+    mean_entropy = None
+    if entropy_coef:
+        mean_entropy = torch.stack(entropies, dim=1).mean()
+        loss = loss - entropy_coef * mean_entropy
+        mean_entropy = float(mean_entropy.detach())
     for p in a2c_network.parameters():
         p.grad = None
     loss.backward()
-    return _ModuleRouteResult(float(loss), float(rewards.mean()), float(advantage.mean()))
+    return _ModuleRouteResult(float(loss), float(rewards.mean()), float(advantage.mean()), mean_entropy)
 
 
 def get_coco_minibatches_device(data, eng, batch_size=100, split="train"):
@@ -421,13 +432,14 @@ def get_coco_minibatches_device(data, eng, batch_size=100, split="train"):
         yield data["%s_captions" % split][mask], eng.gather_rows(feats, idxs), data["%s_urls" % split][idxs]
 
 
-def _run_minibatches(train_data, a2c_network, reward_network, optimizer, writer, batch_size, epoch, level, tag, best):
+def _run_minibatches(train_data, a2c_network, reward_network, optimizer, writer, batch_size, epoch, level, tag, best,
+                     entropy_coef=0.0):
     bidir = getattr(a2c_network.policy_network, "bidirectional", False)
-    eng = None if bidir else _engine_for(a2c_network, reward_network)
+    eng = None if bidir else _engine_for(a2c_network, reward_network, entropy_coef)
     batches = get_coco_minibatches(train_data, batch_size=batch_size) if bidir else \
         get_coco_minibatches_device(train_data, eng, batch_size=batch_size)
     for minibatch_id, (captions, features, _) in enumerate(batches):
-        res = (_module_route_step(a2c_network, reward_network, features, captions, level) if bidir
+        res = (_module_route_step(a2c_network, reward_network, features, captions, level, entropy_coef) if bidir
                else eng.step(features, captions, level=level))
         if res is not None:                           # curriculum: prefix shorter than 1 => skipped (trainers.py:550)
             optimizer.step()                          # gradients already sit in .grad (flat bucket)
@@ -437,6 +449,8 @@ def _run_minibatches(train_data, a2c_network, reward_network, optimizer, writer,
             writer.add_scalar(tag + "loss", loss, n)
             writer.add_scalar(tag + "mean-rewards", res.mean_reward, n)
             writer.add_scalar(tag + "mean-advantage", res.mean_adv, n)
+            if entropy_coef:
+                writer.add_scalar(tag + "mean-entropy", res.mean_entropy, n)
         # trainers.py:495-496 / :611-612 -- the engine always starts its chains from zero state;
         # the module-level carried state is reset too so mixed use stays consistent
         reward_network.rewrnn.init_hidden()
@@ -444,36 +458,39 @@ def _run_minibatches(train_data, a2c_network, reward_network, optimizer, writer,
     return best
 
 
-def a2c_training(train_data, a2c_network, reward_network, optimizer, plot_dir, save_paths, batch_size, epochs):
-    """trainers.py:402-500."""
+def a2c_training(train_data, a2c_network, reward_network, optimizer, plot_dir, save_paths, batch_size, epochs,
+                 entropy_coef=0.0):
+    """trainers.py:402-500.  entropy_coef: weight of the entropy bonus (A2CEngine); 0 is the reference's loss."""
     writer = SummaryWriter(log_dir=os.path.join(plot_dir, "runs"))
     best = float("inf")
     for epoch in range(epochs):
         best = _run_minibatches(train_data, a2c_network, reward_network, optimizer, writer, batch_size, epoch, None,
-                                "A2C Network-episodic-", best)
+                                "A2C Network-episodic-", best, entropy_coef)
         save_a2c_model(a2c_network, save_paths)
     return a2c_network
 
 
 def a2c_curriculum_training(train_data, a2c_network, reward_network, optimizer, plot_dir, save_paths, batch_size,
-                            epochs, curriculum):
+                            epochs, curriculum, entropy_coef=0.0):
     """trainers.py:503-616: for each level, rollouts start from the ground-truth prefix
-    captions[:, :caplen-level] and sample `level` tokens."""
+    captions[:, :caplen-level] and sample `level` tokens (the entropy bonus, when set, over those `level` steps)."""
     writer = SummaryWriter(log_dir=os.path.join(plot_dir, "runs"))
     for level in curriculum:
         best = float("inf")
         for epoch in range(epochs):
             best = _run_minibatches(train_data, a2c_network, reward_network, optimizer, writer, batch_size, epoch,
-                                    level, "A2C Curriculum Level-%s-" % level, best)
+                                    level, "A2C Curriculum Level-%s-" % level, best, entropy_coef)
             save_a2c_model(a2c_network, save_paths)
     return a2c_network
 
 
 def train_a2c_network(train_data, save_paths, network_paths, plot_dir, bidirectional, epochs, batch_size,
-                      retrain_all=False, curriculum=None):
+                      retrain_all=False, curriculum=None, entropy_coef=0.0):
     """trainers.py:312-399: build the three networks, load the pretrained state dicts
     (``torch.load(path, map_location=device)`` + ``load_state_dict(strict=False)``), freeze the
-    reward network, wrap, Adam(lr=1e-4), dispatch."""
+    reward network, wrap, Adam(lr=1e-4), dispatch.  entropy_coef > 0 adds the entropy bonus
+    ``- entropy_coef * mean policy entropy`` to the A2C loss and logs ``<tag>mean-entropy``; the default 0 is the
+    reference's loss."""
     w2i, emb = train_data["word_to_idx"], train_data.get("embeddings")
     trainers_ = {"reward_network": train_reward_network, "policy_network": train_policy_network,
                  "value_network": train_value_network}
@@ -497,15 +514,16 @@ def train_a2c_network(train_data, save_paths, network_paths, plot_dir, bidirecti
         # fused route: the same Adam(lr=1e-4) as ONE kernel over the flat gradient bucket the engine fills (optim.FlatAdam;
         # torch's update operation by operation, <= 2e-7 from torch.optim.Adam over 3 steps)
         from .optim import FlatAdam
-        optimizer = FlatAdam(_engine_for(a2c_network, reward_network), lr=0.0001)
+        optimizer = FlatAdam(_engine_for(a2c_network, reward_network, entropy_coef), lr=0.0001)
     paths = [save_paths["model_path"], network_paths["a2c_network"]]
     if curriculum is None:
-        a2c_network = a2c_training(train_data, a2c_network, reward_network, optimizer, plot_dir, paths, batch_size, epochs)
+        a2c_network = a2c_training(train_data, a2c_network, reward_network, optimizer, plot_dir, paths, batch_size, epochs,
+                                   entropy_coef)
     else:
         if 16 not in curriculum:
             curriculum.append(16)                    # trainers.py:389-390
         a2c_network = a2c_curriculum_training(train_data, a2c_network, reward_network, optimizer, plot_dir, paths,
-                                              batch_size, epochs, curriculum)
+                                              batch_size, epochs, curriculum, entropy_coef)
     with open(save_paths["results_path"], "a") as fh:
         fh.write("\n" + "-" * 10 + " network " + "-" * 10 + "\n" + str(a2c_network) + "\n" + "-" * 10 + " network "
                  + "-" * 10 + "\n")

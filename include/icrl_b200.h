@@ -337,6 +337,27 @@ int icrl_reward_cosine_fwd(void* stream, int B, int S, const float* ve, const fl
 int icrl_a2c_loss_fwd_bwd(void* stream, int B, int S, const float* values, const float* rewards, const float* logp,
                           float inv_denom, float* out3, float* dv_sb, float* dlogp, float* sum_dv, int* launches);
 
+/* ---- entropy bonus (new; the reference's loss, trainers.py:471-475, has none): the A3C regulariser
+ *      loss = reference loss - entropy_coef * mean_{b,s} H[b][s],  H = -sum_j p_j log p_j of the softmax the rollout
+ *      sampled step s of row b from.  Off (no call) reproduces the reference.
+ *      Policy entropy over the logits stash of the rollout (icrl_policy_rollout_fwd*: logits [S][B][ldl], the V real
+ *      columns summed): entropy [B][S] (the layout of logp), same max / exp / sum arithmetic as the softmax backward.
+ *      One warp per row; reads S*B*V*4 bytes once. */
+int icrl_policy_entropy(void* stream, int B, int S, int V, const float* logits, int ldl, float* entropy, int* launches);
+/*      icrl_a2c_loss_fwd_bwd with the entropy bonus: out4 = {loss - entropy_coef * mean entropy, mean reward,
+ *      mean advantage, mean entropy} (partial sums scaled by inv_denom); dv_sb, dlogp, sum_dv bit-identical to
+ *      icrl_a2c_loss_fwd_bwd's (the bonus does not depend on values, rewards or log-probs). */
+int icrl_a2c_loss_entropy_fwd_bwd(void* stream, int B, int S, const float* values, const float* rewards, const float* logp,
+                                  const float* entropy, float entropy_coef, float inv_denom, float* out4, float* dv_sb,
+                                  float* dlogp, float* sum_dv, int* launches);
+/*      Step 1 of icrl_policy_rollout_bwd[_tc] with the bonus (logits backward of trainers.py:458 plus the entropy term):
+ *      z [S][B][ldz] (the logits) becomes, in place,
+ *        dL/dz = dlogp[b][s] (onehot(a) - p) + scale * p (log p + H[b][s]),  scale = entropy_coef * inv_denom.
+ *      Columns >= V are not touched (the zero padding of ldz = icrl_vocab_pad() stays zero).  Then call
+ *      icrl_policy_rollout_bwd[_tc] with dlogp = NULL. */
+int icrl_softmax_entropy_bwd(void* stream, int B, int S, int V, float* z, int ldz, const long long* tokens_out,
+                             const float* dlogp, const float* entropy, float scale, int* launches);
+
 /* ---- value-guided look-ahead decoder (GenerateCaptionsWithActorCriticLookAhead, trainers.py:73-105).  K candidate
  *      caption batches of B rows and n columns each are expanded by their k best words per beam step.
  *      Stream: cand_tok [K][n][B] int32 (each candidate's columns), words [K][B][k] int32 -> the value chain of the step,
