@@ -85,6 +85,7 @@ SIGNATURES = {
     "icrl_policy_entropy": [P, I, I, I, P, I, P, LP],
     "icrl_a2c_loss_entropy_fwd_bwd": [P, I, I, P, P, P, P, F, F, P, P, P, P, LP],
     "icrl_softmax_entropy_bwd": [P, I, I, I, P, I, P, P, P, F, LP],
+    "icrl_policy_xent_fwd_bwd": [P, I, I, I, P, P, P, P, P, I, P, P, LP],
 }
 _RESTYPES = {"icrl_last_error": c_char_p, "icrl_wgrad_tc_ws_bytes": c_size_t, "icrl_decode_weight_halves": c_size_t, "icrl_colsum_ws_floats": c_size_t, "icrl_stream_len": c_longlong,
              "icrl_chain_sync_bytes": c_size_t, "icrl_chain_tc_weight_halves": c_size_t, "icrl_chain_tc_ws_bytes": c_size_t, "icrl_chain_tc_cp_floats": c_size_t,

@@ -747,4 +747,16 @@ int icrl_softmax_entropy_bwd(void* stream, int B, int S, int V, float* z, int ld
   return ICRL_OK;
 }
 
+// ---- policy pretraining loss (trainers.py:202-257)
+int icrl_policy_xent_fwd_bwd(void* stream, int B, int S, int V, const float* logits, const long long* targets,
+                             const int* n_rows, const double* w_rows, float* dz, int ldz, float* ce, float* loss,
+                             int* launches) {
+  ICRL_REQUIRE(B > 0 && S > 0 && V > 0 && ldz >= V, "bad logits shape (B, S, V > 0, ldz >= V)");
+  ICRL_REQUIRE(logits && targets && n_rows && w_rows && dz && ce && loss, "null argument");
+  ICRL_REQUIRE(dz != logits, "dL/dlogits is written out of place: the logits stay intact for a re-run");
+  TRY(icrl_policy_xent_impl(S_(stream), B, S, V, logits, targets, n_rows, w_rows, dz, ldz, ce, loss));
+  bump(launches, 2);
+  return ICRL_OK;
+}
+
 }  // extern "C"

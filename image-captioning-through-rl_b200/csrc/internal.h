@@ -15,6 +15,8 @@ int icrl_softmax_sample(cudaStream_t st, int B, int V, const float* logits, int 
 int icrl_softmax_bwd(cudaStream_t st, int B, int S, int V, float* z, int ldl, const long long* tokens_out,
                      const float* dlogp, const float* entropy = nullptr, float scale = 0.f);
 int icrl_policy_entropy_impl(cudaStream_t st, int B, int S, int V, const float* logits, int ldl, float* entropy);
+int icrl_policy_xent_impl(cudaStream_t st, int B, int S, int V, const float* logits, const long long* targets,
+                          const int* n_rows, const double* w_rows, float* dz, int ldz, float* ce, float* loss);
 int icrl_topk_rows(cudaStream_t st, int R, int V, int k, const float* x, float* top_val, int* top_idx);
 int icrl_scatter_add_rows(cudaStream_t st, long long R, int C, const float* src, const int* idx, float* dst);
 int icrl_scatter_add_stream(cudaStream_t st, int B, int p0, int S, int extra, int C, const float* src, const int* tok_stream,

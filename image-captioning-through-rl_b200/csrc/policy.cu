@@ -174,6 +174,55 @@ __global__ void policy_entropy_kernel(int B, int S, int V, const float* __restri
   if (lane == 0) entropy[(size_t)b * S + s] = logf(tot) - t / tot;
 }
 
+// Weighted cross entropy of the policy's supervised pretraining (trainers.py:202-257).  One warp per row r = s*B + b of
+// the teacher-forced logits stash z [S][B][V]: for s < n[b], with p = softmax(z) (the max / exp / sum of
+// softmax_bwd_kernel), ce[r] = log(sum exp(z - max)) - (z[t] - max) -- finite where p[t] underflows, unlike log(p[t]) --
+// and dz[r][v] = w[b] (p[v] - [v == t]), t = target[b][s]; rows with s >= n[b] get ce = 0 and dz = 0.  Columns V..ldz-1
+// of dz are written zero.  z is read only, so the backward can be re-run from it.
+__global__ void policy_xent_kernel(int B, int S, int V, const float* __restrict__ z, const long long* __restrict__ target,
+                                   const int* __restrict__ n_rows, const double* __restrict__ w_rows, float* __restrict__ dz,
+                                   int ldz, float* __restrict__ ce) {
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (warp >= B * S) return;
+  const int s = warp / B, b = warp % B;
+  float* d = dz + (size_t)warp * ldz;
+  if (s >= n_rows[b]) {
+    for (int v = lane; v < ldz; v += 32) d[v] = 0.f;
+    if (lane == 0) ce[warp] = 0.f;
+    return;
+  }
+  const float* x = z + (size_t)warp * V;
+  float mx = -INFINITY;
+  for (int v = lane; v < V; v += 32) mx = fmaxf(mx, x[v]);
+  mx = warp_max(mx);
+  float sum = 0.f;
+  for (int v = lane; v < V; v += 32) sum += expf(x[v] - mx);
+  const float tot = warp_sum(sum);
+  const float inv = 1.0f / tot;
+  const int t = (int)target[(size_t)b * S + s];
+  const float w = (float)w_rows[b];
+  for (int v = lane; v < V; v += 32) d[v] = w * (expf(x[v] - mx) * inv - (v == t ? 1.f : 0.f));
+  for (int v = V + lane; v < ldz; v += 32) d[v] = 0.f;
+  if (lane == 0) ce[warp] = logf(tot) - (x[t] - mx);
+}
+
+// Single block: loss = sum_r w[r % B] ce[r] in double, in a fixed order (no atomics), as a2c_loss_kernel sums.
+__global__ void xent_loss_kernel(int B, int n, const float* __restrict__ ce, const double* __restrict__ w_rows,
+                                 float* __restrict__ loss) {
+  __shared__ double red[32];
+  double l = 0.0;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) l += w_rows[i % B] * (double)ce[i];
+  l = warp_sum_d(l);
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (lane == 0) red[w] = l;
+  __syncthreads();
+  if (w == 0) {
+    l = lane < (int)(blockDim.x >> 5) ? red[lane] : 0.0;
+    l = warp_sum_d(l);
+    if (lane == 0) loss[0] = (float)l;
+  }
+}
+
 // The same with 16-byte vector reductions (red.global.add.v4.f32, sm_90+): a quarter of the instructions and of the L2
 // atomic transactions of the scalar form (1.6 G atomics per step at B = 4096: 3.9 ms, 6.5 % of the step).  C % 4 == 0.
 __global__ void scatter_add_rows_v4_kernel(long long R, int C4, const float4* __restrict__ src, const int* __restrict__ idx,
@@ -362,6 +411,16 @@ int icrl_softmax_bwd(cudaStream_t st, int B, int S, int V, float* z, int ldl, co
 
 int icrl_policy_entropy_impl(cudaStream_t st, int B, int S, int V, const float* logits, int ldl, float* entropy) {
   policy_entropy_kernel<<<icrl_cdiv((long long)B * S * 32, 128), 128, 0, st>>>(B, S, V, logits, ldl, entropy);
+  ICRL_LAUNCH_CHECK();
+  return ICRL_OK;
+}
+
+int icrl_policy_xent_impl(cudaStream_t st, int B, int S, int V, const float* logits, const long long* targets,
+                          const int* n_rows, const double* w_rows, float* dz, int ldz, float* ce, float* loss) {
+  policy_xent_kernel<<<icrl_cdiv((long long)B * S * 32, 128), 128, 0, st>>>(B, S, V, logits, targets, n_rows, w_rows, dz, ldz,
+                                                                           ce);
+  ICRL_LAUNCH_CHECK();
+  xent_loss_kernel<<<1, 1024, 0, st>>>(B, B * S, ce, w_rows, loss);
   ICRL_LAUNCH_CHECK();
   return ICRL_OK;
 }

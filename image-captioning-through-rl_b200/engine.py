@@ -85,6 +85,26 @@ def plan_rollout(captions, level=None):
     return caplen - int(level), int(level)
 
 
+def plan_xent(captions):
+    """Row plan of the policy's cross-entropy pretraining (trainers.py:202-257), as the reference derives it: caplen_b =
+    column of the FIRST <END> of row b + 1; the row counts its first n_b = min(caplen_b, L-1) teacher-forced positions
+    (the last counted one predicts the token after <END>) with weight w_b = caplen_b / (B * n_b) -- the reference's
+    (caplen/B) * mean, with the unclamped caplen.  Returns (n [B] int, w [B] float64, S = max n_b): positions at or past
+    every row's n_b add nothing, so the decode runs S steps only.  Raises ValueError for a row without <END> (the
+    reference fails there with an IndexError)."""
+    caps = np.asarray(captions)
+    if caps.ndim != 2 or caps.shape[0] < 1 or caps.shape[1] < 2:
+        raise ValueError("captions must be (B, L) with B >= 1 and L >= 2, got %s" % (caps.shape,))
+    B, L = caps.shape
+    end = caps == END_TOKEN
+    missing = np.nonzero(~end.any(axis=1))[0]
+    if missing.size:
+        raise ValueError("caption row %d has no <END> (=2) token (the reference's loop raises IndexError there)" % missing[0])
+    caplen = end.argmax(axis=1) + 1
+    n = np.minimum(caplen, L - 1)
+    return n, caplen / (float(B) * n), int(n.max())
+
+
 class A2CEngine:
     DECODE_MODES = ("fused", "tc", "simt")
     entropy_coef = 0.0            # engines that skip __init__ (look-ahead, greedy decode) have no entropy bonus
@@ -203,7 +223,7 @@ class A2CEngine:
         return list(self.a2c.parameters())
 
     def _check_params(self):
-        for p in list(self.a2c.parameters()) + list(self.reward.parameters()):
+        for p in list(self.a2c.parameters()) + (list(self.reward.parameters()) if self.reward is not None else []):
             if p.dtype != torch.float32 or not p.is_contiguous() or p.device != self.device:
                 raise _lib.IcrlError("parameters must be contiguous float32 on %s" % self.device)
 
@@ -676,10 +696,12 @@ class A2CEngine:
             _lib.call("icrl_chain_lstm_bwd", st, Tv, _p(Vn.valrnn.lstm.weight_hh_l0), _p(b["v_stash_g"]), _p(b["v_stash_c"]),
                   _p(b["v_take"]), _p(dh_take), _p(dgates), _p(self.sync_state), None, None, None, None, L)
 
-    def _backward_policy(self, f, tokcm, tokens, B, p0, S, tag, ent=None):
+    def _backward_policy(self, f, tokcm, tokens, B, p0, S, tag, ent=None, seed=None, bptt=None):
         # policy BPTT.  icrl_policy_rollout_bwd turns the logits into dL/dlogits IN PLACE; a step whose chains are re-run
         # (longer warm-up, serial fall-back) runs this backward again with slightly different dL/dlogp, so it works on a
-        # copy and the rollout's logits stay intact.
+        # copy and the rollout's logits stay intact.  seed(dz, ldz), when given, writes dL/dlogits into the [S*B][ldz]
+        # buffer itself (padding columns included) and the backward starts from it (dlogp = NULL); bptt overrides
+        # policy_bptt for this call.
         st, L, b, V = self._stream, self.launches.ref, self._bufs, self.V
         P = self.policy
         SB = S * B
@@ -688,15 +710,19 @@ class A2CEngine:
         g = self._g
         colsum_ws, gemm_ws, gemm_ws_floats, dtable = self._bwd_workspaces(B, S, 0, tag)
         pl = P.lstm
-        tc = self.policy_bptt == "tc"
+        tc = (bptt or self.policy_bptt) == "tc"
         ldz = int(_lib.call("icrl_vocab_pad")) if tc and V <= 1024 else V      # padded rows: vocabulary contractions on tcgen05
         dz = self._bufs.get("p_dlogits")
         if dz is None or dz.numel() < SB * ldz or self._dz_ld != ldz:
             dz = self._bufs["p_dlogits"] = torch.zeros(SB * ldz, dtype=torch.float32, device=self.device)   # padding stays zero
             self._dz_ld = ldz
         with self._phase("policy_bwd"):
-          dz[:SB * ldz].view(SB, ldz)[:, :V].copy_(b["p_logits"][:SB * V].view(SB, V))
-          dlogp = b["dlogp"]
+          if seed is not None:
+            seed(dz, ldz)
+            dlogp = None
+          else:
+            dz[:SB * ldz].view(SB, ldz)[:, :V].copy_(b["p_logits"][:SB * V].view(SB, V))
+            dlogp = b["dlogp"]
           if ent is not None:
             # dL/dlogits with the entropy bonus's term, in place; the rollout backward then starts from it (dlogp = NULL)
             _lib.call("icrl_softmax_entropy_bwd", st, B, S, V, _p(dz), ldz, _p(tokens), _p(dlogp), _p(ent[0]), ent[1], L)
@@ -708,7 +734,7 @@ class A2CEngine:
                   _p(dtable), _p(colsum_ws), _p(gemm_ws), gemm_ws_floats * 4, _p(g(P.caption_embedding.weight, True)),
                   _p(g(P.cnn2linear.weight)), _p(g(P.cnn2linear.bias)), _p(g(pl.weight_ih_l0)), _p(g(pl.weight_hh_l0)),
                   _p(g(pl.bias_ih_l0)), _p(g(pl.bias_hh_l0)), _p(g(P.linear2vocab.weight)), _p(g(P.linear2vocab.bias))]
-          if self.policy_bptt == "tc":
+          if tc:
             # the n_cell serial cell-backward steps as ONE launch of the tcgen05 chain-backward kernel (rows = MMA rows)
             ws = self._buf("p_bptt_ws", (int(_lib.call("icrl_policy_bwd_tc_ws_bytes", B, S, n_cell)) + 3) // 4)
             _lib.call("icrl_policy_rollout_bwd_tc", *args, _p(b["p_chain_pk"]), _p(ws), _p(self._stat_err[20:]), ldz, L)
@@ -945,6 +971,94 @@ class A2CEngine:
             last = self._bufs["p_logits"][(steps - 1) * B * self.V: steps * B * self.V].view(B, self.V).clone()
             out = torch.cat((torch.from_numpy(first).to(self.device), tokens), dim=1)
         return out, last
+
+
+class PolicyOnlyEngine(A2CEngine):
+    """A2CEngine restricted to the policy (greedy decode needs no value / reward network)."""
+
+    def __init__(self, policy_network):
+        self.policy, self.value, self.reward, self.a2c = policy_network, None, None, policy_network
+        dev = policy_network.linear2vocab.weight.device
+        if dev.type != "cuda":
+            raise _lib.IcrlError("the policy engine needs the policy on a CUDA device (no CPU fallback)")
+        _lib.load()
+        self.device, self.V = dev, policy_network.linear2vocab.weight.shape[0]
+        self._bufs, self.launches, self.phase_events = {}, _lib.Launches(), None
+        self.decode, self.use_tc = ("fused" if self.V <= 1024 and self.V % 4 == 0 else "simt"), False
+
+    def pack_weights(self, reward=False):
+        P = self.policy
+        _lib.call("icrl_pack_gate_table", self._stream, self.V, 4 * H, 4 * H, P.caption_embedding.weight.shape[1], _p(P.caption_embedding.weight),
+                  _p(P.lstm.weight_ih_l0), _p(P.lstm.bias_ih_l0), _p(P.lstm.bias_hh_l0),
+                  _p(self._buf("p_table", self.V * 4 * H)), self.launches.ref)
+        if self.decode == "fused":
+            n = int(_lib.call("icrl_decode_weight_halves"))
+            _lib.call("icrl_pack_decode_weights", self._stream, self.V, _p(P.lstm.weight_hh_l0), _p(P.linear2vocab.weight),
+                      _p(self._buf("p_decode_pk", n, torch.float16)), self.launches.ref)
+
+
+class PolicyPretrainEngine(PolicyOnlyEngine):
+    """Cross-entropy pretraining of the unidirectional policy (train_policy_network, trainers.py:202-257) on the fused
+    engine: per minibatch the teacher-forced decode of A2CEngine (the persistent tcgen05 kernel with forced tokens; the
+    per-step kernels where A2CEngine takes them), the fused masked cross entropy (icrl_policy_xent_fwd_bwd) and the
+    policy backward of A2CEngine started from its dL/dlogits.  Gradients land in the flat bucket over
+    policy.parameters() that the parameters' .grad alias, so optim.FlatAdam(engine) steps them.
+
+    policy_bptt: "tc" runs the serial cell-backward steps on the tcgen05 chain-backward kernel; when its fp16 exchange
+    overflows, the minibatch's backward is re-run on the fp32 kernels ("simt", which can also be chosen outright)."""
+
+    def __init__(self, policy_network, policy_bptt="tc"):
+        super().__init__(policy_network)
+        if getattr(policy_network, "bidirectional", False):
+            raise NotImplementedError("the fused pretraining engine is built for the unidirectional policy; bidirectional=True "
+                                      "runs on the module (autograd) route")
+        if policy_bptt not in ("tc", "simt"):
+            raise ValueError("policy_bptt must be 'tc' or 'simt'")
+        self.policy_bptt, self.wgrad, self._n_cell_max, self._dz_ld = policy_bptt, "tc", 1, None
+        self.bptt_reruns = 0          # minibatches whose backward fell back to the fp32 kernels
+        with torch.cuda.device(self.device):
+            # [0] the loss; [20:28] words of the policy's tcgen05 BPTT ([25] fp16-exchange overflow flag): ONE copy per step
+            self._stat_err = torch.zeros(28, dtype=torch.float32, device=self.device)
+        self._check_params()
+        self._bind_flat_grads()
+
+    def pack_weights(self, reward=False):
+        super().pack_weights()
+        if self.policy_bptt == "tc":
+            n = int(_lib.call("icrl_chain_tc_weight_halves", 0))
+            _lib.call("icrl_pack_chain_tc_weights", self._stream, 0, _p(self.policy.lstm.weight_hh_l0),
+                      _p(self._buf("p_chain_pk", n, torch.float16)), self.launches.ref)
+
+    def xent_step(self, features, captions):
+        """One minibatch of train_policy_network: features (B,512) f32 (host or device), captions (B,L) int (host).
+        Leaves the gradients of the reference's loss in the parameters' .grad (flat bucket) and returns the loss (one
+        device-to-host copy, which also brings the BPTT's overflow flag)."""
+        caps = captions.cpu().numpy() if isinstance(captions, torch.Tensor) else np.asarray(captions)
+        n, w, S = plan_xent(caps)
+        if caps.min() < 0 or caps.max() >= self.V:
+            raise ValueError("caption tokens must lie in [0, %d)" % self.V)
+        B, V = caps.shape[0], self.V
+        with torch.cuda.device(self.device):
+            self._attach_grads()
+            self.pack_weights()
+            prep = self.prepare(features, caps, plan=(1, S))
+            f, tokcm, _, fo, _ = self._stage_inputs(prep, caps[:, 1:1 + S])
+            tokens, _ = self._policy_forward(f, tokcm, None, fo, B, 1, S, False)
+            n_rows = torch.from_numpy(n.astype(np.int32)).to(self.device, non_blocking=True)
+            w_rows = torch.from_numpy(w.astype(np.float64)).to(self.device, non_blocking=True)
+            ce = self._buf("p_xent_ce", S * B)
+
+            def seed(dz, ldz):
+                _lib.call("icrl_policy_xent_fwd_bwd", self._stream, B, S, V, _p(self._bufs["p_logits"]), _p(fo), _p(n_rows),
+                          _p(w_rows), _p(dz), ldz, _p(ce), _p(self._stat_err), self.launches.ref)
+
+            self._backward_policy(f, tokcm, tokens, B, 1, S, "_p", seed=seed)
+            host = self._stat_err[:26].tolist()
+            if self.policy_bptt == "tc" and host[25] != 0.0:
+                # the gate gradients overflowed the tcgen05 BPTT's fp16 exchange: the same backward on the fp32 kernels
+                self.bptt_reruns += 1
+                self._backward_policy(f, tokcm, tokens, B, 1, S, "_p", seed=seed, bptt="simt")
+        return host[0]
 
 
 class LookAheadEngine(A2CEngine):

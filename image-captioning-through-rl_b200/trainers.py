@@ -12,10 +12,12 @@ the reference's beam look-ahead on ``engine.LookAheadEngine`` (one tcgen05 value
 carried value state), bidirectional networks on the drop-in modules.
 
 The supervised pretraining loops (``train_policy_network :202``, ``train_reward_network :260``,
-``train_value_network :125``, ``VisualSemanticEmbeddingLoss :23``; SURVEY 8f row 2) run on the drop-in modules through
-their autograd wrappers: the recurrent forwards / backwards are the CUDA kernels, the loss arithmetic on the module
-outputs (cross entropy, MSE, hinge) is torch host code exactly as in the reference.  As in the reference, a missing
-pretrained file makes ``train_a2c_network`` pretrain that network.
+``train_value_network :125``, ``VisualSemanticEmbeddingLoss :23``; SURVEY 8f row 2): ``train_policy_network`` with a
+unidirectional policy runs on ``engine.PolicyPretrainEngine`` (teacher-forced fused decode, fused masked cross entropy
+and tcgen05 BPTT in one ``xent_step`` per minibatch, ``optim.FlatAdam``).  The bidirectional policy and the reward and
+value loops run on the drop-in modules through their autograd wrappers: the recurrent forwards / backwards are the CUDA
+kernels, the loss arithmetic on the module outputs (cross entropy, MSE, hinge) is torch host code exactly as in the
+reference.  As in the reference, a missing pretrained file makes ``train_a2c_network`` pretrain that network.
 """
 import math
 import os
@@ -25,7 +27,7 @@ import numpy as np
 import torch
 import torch.optim as optim
 
-from .engine import A2CEngine
+from .engine import A2CEngine, PolicyOnlyEngine, PolicyPretrainEngine
 from .models import *          # noqa: F401,F403  (torch, nn, F, np, device, MAX_SEQ_LEN, classes)
 from .models import AdvantageActorCriticNetwork, PolicyNetwork, RewardNetwork, ValueNetwork, device, MAX_SEQ_LEN
 
@@ -129,7 +131,7 @@ def GenerateCaptionsGreedy(features, captions, policy_network):
         return gen
     eng = getattr(policy_network, "_icrl_greedy", None)
     if eng is None:
-        eng = _PolicyOnlyEngine(policy_network)
+        eng = PolicyOnlyEngine(policy_network)
         object.__setattr__(policy_network, "_icrl_greedy", eng)
     tokens, _ = eng.greedy_decode(np.asarray(features, dtype=np.float32), np.asarray(captions)[:, 0], MAX_SEQ_LEN - 1)
     return tokens
@@ -229,34 +231,6 @@ def test_a2c_network(a2c_network, test_data, image_caption_data, data_size, vali
             a2c_network.value_network.valrnn.init_hidden()
 
 
-class _PolicyOnlyEngine(A2CEngine):
-    """A2CEngine restricted to the policy (greedy decode needs no value / reward network)."""
-
-    def __init__(self, policy_network):
-        self.policy, self.value, self.reward, self.a2c = policy_network, None, None, policy_network
-        dev = policy_network.linear2vocab.weight.device
-        if dev.type != "cuda":
-            from . import _lib
-            raise _lib.IcrlError("GenerateCaptionsGreedy needs the policy on a CUDA device (no CPU fallback)")
-        from . import _lib
-        _lib.load()
-        self.device, self.V = dev, policy_network.linear2vocab.weight.shape[0]
-        self._bufs, self.launches, self.phase_events = {}, _lib.Launches(), None
-        self.decode, self.use_tc = ("fused" if self.V <= 1024 and self.V % 4 == 0 else "simt"), False
-
-    def pack_weights(self, reward=False):
-        from . import _lib
-        from .engine import _p, H
-        P = self.policy
-        _lib.call("icrl_pack_gate_table", self._stream, self.V, 4 * H, 4 * H, P.caption_embedding.weight.shape[1], _p(P.caption_embedding.weight),
-                  _p(P.lstm.weight_ih_l0), _p(P.lstm.bias_ih_l0), _p(P.lstm.bias_hh_l0),
-                  _p(self._buf("p_table", self.V * 4 * H)), self.launches.ref)
-        if self.decode == "fused":
-            n = int(_lib.call("icrl_decode_weight_halves"))
-            _lib.call("icrl_pack_decode_weights", self._stream, self.V, _p(P.lstm.weight_hh_l0), _p(P.linear2vocab.weight),
-                      _p(self._buf("p_decode_pk", n, torch.float16)), self.launches.ref)
-
-
 def VisualSemanticEmbeddingLoss(visuals, semantics):
     """Bidirectional hinge ranking loss of the reward pretraining (trainers.py:23-54), beta = 0.2:
     sum(relu(S - diag(S)[:,None] + (beta/N)(1 - I))) / N for S = V S^T and for its transpose."""
@@ -278,12 +252,37 @@ def _minibatches(train_data, batch_size):
 
 def train_policy_network(train_data, network_paths, plot_dir, bidirectional, epochs=100, batch_size=512):
     """Cross-entropy pretraining of the policy (trainers.py:202-257): teacher-forced logits of captions[:, :-1]
-    against captions[:, 1:], each row weighted by caplen/B and averaged over its first caplen positions."""
+    against captions[:, 1:], each row weighted by caplen/B and averaged over its first caplen positions.
+
+    The unidirectional policy runs on engine.PolicyPretrainEngine: features resident in HBM (get_coco_minibatches_device,
+    the same torch.randperm draw), one xent_step per minibatch (teacher-forced fused decode, fused cross entropy, policy
+    BPTT) and Adam(lr=1e-3) as optim.FlatAdam.  The bidirectional policy runs the reference's loop on the drop-in modules
+    (_train_policy_modules)."""
     policy_network = PolicyNetwork(train_data["word_to_idx"], pretrained_embeddings=train_data.get("embeddings"),
                                    bidirectional=bidirectional).to(device)
+    writer = SummaryWriter(log_dir=os.path.join(plot_dir, "runs"))
+    if bidirectional:
+        return _train_policy_modules(policy_network, train_data, network_paths, writer, epochs, batch_size)
+    from .optim import FlatAdam
+    eng = PolicyPretrainEngine(policy_network)
+    optimizer = FlatAdam(eng, lr=0.001)
+    best = float("inf")
+    for epoch in range(epochs):
+        for minibatch_id, (captions, features, _) in enumerate(get_coco_minibatches_device(train_data, eng, batch_size)):
+            loss = eng.xent_step(features, captions)
+            if loss < best:
+                best = loss           # saved before the step: the checkpoint holds the parameters that gave this loss
+                torch.save(policy_network.state_dict(), network_paths["policy_network"])
+            writer.add_scalar("Policy Network-loss", loss, global_minibatch_number(epoch, minibatch_id, batch_size))
+            optimizer.step()
+    return policy_network
+
+
+def _train_policy_modules(policy_network, train_data, network_paths, writer, epochs, batch_size):
+    """train_policy_network as the reference's loop over the drop-in modules (bidirectional policy, and the reference of
+    the fused route's tests): autograd through the policy's CUDA forward / backward, one CrossEntropyLoss per row."""
     criterion = nn.CrossEntropyLoss().to(device)
     optimizer = optim.Adam(policy_network.parameters(), lr=0.001)
-    writer = SummaryWriter(log_dir=os.path.join(plot_dir, "runs"))
     best = float("inf")
     for epoch in range(epochs):
         for minibatch_id, (captions, features, _) in enumerate(_minibatches(train_data, batch_size)):

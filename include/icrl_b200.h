@@ -358,6 +358,20 @@ int icrl_a2c_loss_entropy_fwd_bwd(void* stream, int B, int S, const float* value
 int icrl_softmax_entropy_bwd(void* stream, int B, int S, int V, float* z, int ldz, const long long* tokens_out,
                              const float* dlogp, const float* entropy, float scale, int* launches);
 
+/* ---- policy pretraining loss (train_policy_network, trainers.py:202-257): teacher-forced logits [S][B][V] of
+ *      icrl_policy_rollout_fwd* with forced tokens, targets [B][S] int64 (the forced tokens, captions[:, 1:1+S]).
+ *      Row b counts its first n_rows[b] <= S positions with weight w_rows[b] (f64; the reference's
+ *      caplen_b / (B * n_b)):
+ *        loss[0] = sum_b w_b sum_{s < n_b} CE(z[s][b], t[b][s]),  CE = log(sum exp(z - max)) - (z_t - max),
+ *      summed in double in a fixed order; ce [S*B] f32 holds the per-row CE terms (zero past n_b).
+ *      dz [S*B][ldz] (out of place; the logits are not modified):
+ *        dz[s*B+b][v] = w_b (softmax(z)[v] - [v == t]) for s < n_b, 0 for s >= n_b and for the columns V..ldz-1.
+ *      Then call icrl_policy_rollout_bwd_tc with dlogp = NULL, logits = dz and this ldz (or icrl_policy_rollout_bwd with
+ *      ldz = V). */
+int icrl_policy_xent_fwd_bwd(void* stream, int B, int S, int V, const float* logits, const long long* targets,
+                             const int* n_rows, const double* w_rows, float* dz, int ldz, float* ce, float* loss,
+                             int* launches);
+
 /* ---- value-guided look-ahead decoder (GenerateCaptionsWithActorCriticLookAhead, trainers.py:73-105).  K candidate
  *      caption batches of B rows and n columns each are expanded by their k best words per beam step.
  *      Stream: cand_tok [K][n][B] int32 (each candidate's columns), words [K][B][k] int32 -> the value chain of the step,
